@@ -2,7 +2,7 @@
 """bench.py -- images/sec of the ViT forward (BASELINE.json `metric`: ViT-B/16 224, batch 256 per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dtype bf16|fp16]
-                    [--config c2|c3|c4|c5] [--batch B | --global-batch G]
+                    [--config c2|c3|c4|c5] [--batch B | --global-batch G] [--dump-outputs DIR]
 
 One "step" = one forward of the per-GPU batch.  N > 1 is launched by torchrun (one rank per GPU); images
 are independent, so the batch is sharded and the only collective is the in-place NCCL all-gather of the
@@ -17,6 +17,10 @@ pinned HOST buffers (H2D + forward + gather + D2H inside the timed region); `roo
 family against the measured bf16 peak; `cpu_baseline` = the torch-CPU restatement of the reference timed on
 this box's cores.  `--impl reference` times that CPU restatement alone (JAX/Flax cannot be installed here:
 the reference itself is not runnable, see DESIGN.md / BASELINE.md).
+
+`--dump-outputs DIR` writes the logits of the last timed step of every timed operand format as
+DIR/logits_<dtype>.npy (float32), so that two builds run with the same arguments, and therefore on the same
+seeded weights and images, can be compared output for output.
 """
 from __future__ import annotations
 
@@ -37,6 +41,7 @@ sys.path.insert(0, str(ROOT))
 
 METRIC = "images/sec ViT-B/16 224 bf16 fwd at 1/2/4/8 B200; % tensor-pipe peak"
 NOMINAL_BF16_TFLOPS = 2250.0
+DUMP_BYTES = 64 << 20          # --dump-outputs: at most this much in all
 # BASELINE.json configs[1..4]: model, image size, (default batch, is it the GLOBAL batch = strong scaling)
 CONFIGS = {
     "c2": (dict(image_size=224, patch_size=16, num_classes=1000, dim=768, depth=12, heads=12, mlp_dim=3072), 256, False,
@@ -137,6 +142,20 @@ class ClockSampler:
                 "power_w_max": max(power) if power else None, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each [rows, classes] tensor as out_dir/<name>.npy in float32.  A tensor larger than its share of
+    DUMP_BYTES is cut to a fixed sample of its rows (seed 0, ascending row order): the same rows in every run."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // max(1, len(arrays))
+    for name, a in arrays.items():
+        rows, row_bytes = a.shape[0], a[0].numel() * 4
+        if rows * row_bytes > budget:
+            keep = np.sort(np.random.default_rng(0).choice(rows, size=budget // row_bytes, replace=False))
+            a = a[torch.as_tensor(keep, device=a.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.to("cpu", torch.float32).numpy())
+
+
 def workload_config(args, world: int) -> dict:
     cfg, batch, strong, label, src = CONFIGS[args.config]
     if args.global_batch:
@@ -180,12 +199,12 @@ def cpu_reference(cfg: dict, steps: int, warmup: int, sample_images: int) -> dic
         vit_torch.vit_forward(pt, img, **cfg)
     t0 = time.perf_counter()
     for _ in range(steps):
-        vit_torch.vit_forward(pt, img, **cfg)
+        logits = vit_torch.vit_forward(pt, img, **cfg)
     dt = (time.perf_counter() - t0) / max(1, steps)
     return {"value": sample_images / dt, "unit": "images/s", "cores": cores, "kind": "port",
             "sample": f"{sample_images} images/step of the workload in fp32, {steps} steps after {warmup} warm-up, "
                       f"torch {torch.__version__} CPU restatement of vit_flax/vit.py (JAX/Flax not installable)",
-            "ms_per_step": dt * 1e3}
+            "ms_per_step": dt * 1e3, "logits": logits}
 
 
 def run_reference(args) -> None:
@@ -194,21 +213,20 @@ def run_reference(args) -> None:
         return
     world = max(1, args.gpus)
     wl = workload_config(args, world)
-    # every step is a bounded sample (args.cpu_images images, ~0.75 s on 24 cores); the CPU work is capped so
-    # that the whole run stays within a couple of minutes whatever K the caller passes -- the line reports the
-    # caller's K / W (the arm's protocol) and says how many sample steps were actually timed
-    timed, warm = max(1, min(args.steps, 30)), max(1, min(args.warmup, 3))
-    cb = cpu_reference(wl["cfg"], timed, warm, args.cpu_images)
+    # every step is a bounded sample of the workload: args.cpu_images images (~0.75 s on 24 cores)
+    cb = cpu_reference(wl["cfg"], args.steps, args.warmup, args.cpu_images)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits_fp32": cb["logits"]})
     cfg_block = config_block(wl, world, args.dtype)        # identical to our arm's `config`
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "images/s",
-        "n_gpus": args.gpus, "steps": args.steps, "warmup": max(3, args.warmup), "ms_per_step": cb["ms_per_step"],
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": cb["ms_per_step"],
         "higher_is_better": True, "scaling": "strong" if wl["strong"] else "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic", "config": cfg_block,
         "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")},
         "e2e": {"value": cb["value"], "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
-        "reference_sample": (f"{args.cpu_images} images per CPU step, {timed} timed steps after {warm} warm-up "
+        "reference_sample": (f"{args.cpu_images} images per CPU step, {args.steps} timed steps after {args.warmup} warm-up "
                              "(CPU port of the reference on the host cores; rank 0 only)"),
     }
     print(json.dumps(line), flush=True)
@@ -331,6 +349,8 @@ def run_b200(args) -> None:
                     counts = new
                     make_images()
         runs[dt] = timed_forward(engines[dt], args.steps, args.warmup, sample_clocks=(dt == args.dtype))
+    if args.dump_outputs and rank == 0:         # the gathered [global_batch, classes] logits of the last timed step
+        dump_outputs(args.dump_outputs, {f"logits_{dt}": runs[dt]["logits"] for dt in formats})
     images, start, stop = state["images"], state["start"], state["stop"]
     B_local = stop - start
     eng, main = engines[args.dtype], runs[args.dtype]
@@ -577,7 +597,12 @@ def main():
                          "to a faster GPU costs it a ninth wave (profiles/r02_scaling.md)")
     ap.add_argument("--quick", action="store_true", help="headline format only, no e2e / train / CPU legs, parity on 8 images "
                                                           "(the strong-scaling runs of profiles/r02_scaling.md)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logits of the last timed step as DIR/logits_<dtype>.npy (float32, at most 64 MB in "
+                         "all: a seeded sample of the rows when larger)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

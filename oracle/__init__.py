@@ -7,12 +7,12 @@ CPU baseline, never as a fallback for the CUDA path.
 
 PARITY: pinned to a run of the reference's OWN SOURCE, not to a run of its libraries.  jax / jaxlib / flax are
 absent and not installable here and the reference ships no tests, golden vectors or fixtures (SURVEY.md section 8c), so
-``/root/reference/vit_flax/vit.py`` and ``simple_vit.py`` are executed UNMODIFIED over ``oracle/flax_shim`` -- a numpy
+the reference's ``vit_flax/vit.py`` and ``simple_vit.py`` are executed UNMODIFIED over ``oracle/flax_shim`` -- a numpy
 restatement of the jax / flax.linen API subset they call (third-party dependency, flax 0.5.0 / jax 0.3.13 per the
 reference README; the shim's README lists every restated definition).  ``tests/golden/make_reference_golden.py`` stores
 what the reference computes (logits on three configs, the dropped forward, ``init`` leaf names / shapes, the printed
 output of its demo blocks) as ``tests/golden/ref_*.npz``; ``tests/test_reference_run.py`` holds both oracles and the
-CUDA path to those vectors, and re-runs the reference live wherever /root/reference exists.  So every line written IN
+CUDA path to those vectors, and re-runs the reference live wherever VIT_FLAX_REFERENCE names it.  So every line written IN
 the reference is pinned; what stays restated-not-run is the inside of nn.Dense / nn.LayerNorm / nn.gelu / nn.softmax /
 nn.Dropout and Flax's auto-naming, cross-checked by two independent restatements (numpy float64 in ``vit_numpy.py``,
 torch-CPU float32 in ``vit_torch.py``), an einops check of the patchify order, the known answers the reference documents

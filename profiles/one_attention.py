@@ -1,5 +1,6 @@
 import sys, ctypes as C, torch
-sys.path.insert(0,'/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from vit_flax_b200 import _lib
 lib=_lib.load()
 b,T,h=map(int,sys.argv[1:4])

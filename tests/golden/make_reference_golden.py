@@ -1,6 +1,7 @@
-"""Run the REFERENCE ITSELF and store what it computes:  python tests/golden/make_reference_golden.py
+"""Run the REFERENCE ITSELF and store what it computes:
+    VIT_FLAX_REFERENCE=<checkout of conceptofmind/vit-flax>/vit_flax python tests/golden/make_reference_golden.py
 
-Imports /root/reference/vit_flax/vit.py and simple_vit.py UNMODIFIED (importlib, straight from where they lie) with
+Imports $VIT_FLAX_REFERENCE/vit.py and simple_vit.py UNMODIFIED (importlib, straight from where they lie) with
 oracle/flax_shim on sys.path in place of the absent jax / flax (oracle/flax_shim/README.md says exactly what that shim
 restates), runs their `init` / `apply` and their `__main__` demo blocks, and writes
 
@@ -9,8 +10,8 @@ restates), runs their `init` / `apply` and their `__main__` demo blocks, and wri
                                      the leaf names and shapes of `ViT.init`, the demo block's printed lines
     tests/golden/ref_simple_vit.npz  the same for simple_vit.py: init names / shapes, inputs, parameters and logits
 
-Only this container has /root/reference; the fixtures travel (tests/test_reference_run.py compares the oracle, and on
-the GPU box the CUDA path, with them; when /root/reference is present that test also re-runs the reference live).
+The reference is not part of this repository; the fixtures are (tests/test_reference_run.py compares the oracle, and on
+a GPU the CUDA path, with them; when VIT_FLAX_REFERENCE names the reference's sources that test also re-runs it live).
 What the vectors pin: every line of the reference's own files.  What they do not: the numerics inside jax / flax
 (restated by the shim in float64) and JAX's random stream (parameters and images come from this repository's seeded
 numpy generators; dropout masks from oracle/philox.py, plugged in as `jax.random.bernoulli`).
@@ -20,6 +21,7 @@ from __future__ import annotations
 import contextlib
 import importlib.util
 import io
+import os
 import runpy
 import sys
 from pathlib import Path
@@ -28,7 +30,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parents[2]
 HERE = Path(__file__).resolve().parent
-REFERENCE = Path("/root/reference/vit_flax")
+REFERENCE = Path(os.environ["VIT_FLAX_REFERENCE"]) if os.environ.get("VIT_FLAX_REFERENCE") else None
 SHIM = ROOT / "oracle" / "flax_shim"
 
 TINY = dict(image_size=32, patch_size=8, num_classes=8, dim=64, depth=2, heads=2, mlp_dim=128)
@@ -39,7 +41,7 @@ DROP_KEY = 0x1234_5678_9ABC_DEF0
 
 
 def reference_available() -> bool:
-    return (REFERENCE / "vit.py").is_file() and (REFERENCE / "simple_vit.py").is_file()
+    return REFERENCE is not None and (REFERENCE / "vit.py").is_file() and (REFERENCE / "simple_vit.py").is_file()
 
 
 @contextlib.contextmanager
@@ -93,7 +95,7 @@ def run_demo(stem):
 
 
 def generate():
-    """-> (dict for ref_vit.npz, dict for ref_simple_vit.npz).  Needs /root/reference."""
+    """-> (dict for ref_vit.npz, dict for ref_simple_vit.npz).  Needs the reference (VIT_FLAX_REFERENCE)."""
     sys.path.insert(0, str(ROOT))
     sys.path.insert(0, str(ROOT / "tests"))
     from _util import load_golden
@@ -165,7 +167,8 @@ def generate():
 
 def main():
     if not reference_available():
-        raise SystemExit("/root/reference is not here: the fixtures can only be regenerated where the reference lies")
+        raise SystemExit("set VIT_FLAX_REFERENCE to the vit_flax/ directory of a conceptofmind/vit-flax checkout: "
+                         "the fixtures can only be regenerated from the reference's own files")
     vit_out, simple_out = generate()
     np.savez_compressed(HERE / "ref_vit.npz", **vit_out)
     np.savez_compressed(HERE / "ref_simple_vit.npz", **simple_out)

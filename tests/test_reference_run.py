@@ -1,9 +1,9 @@
 """The oracle (and on a GPU the CUDA path) against OUTPUTS OF THE REFERENCE ITSELF.
 
 tests/golden/ref_vit.npz and ref_simple_vit.npz were written by tests/golden/make_reference_golden.py, which executes
-/root/reference/vit_flax/vit.py and simple_vit.py unmodified over oracle/flax_shim (a numpy restatement of the jax /
-flax API they use; its README states what that pins and what it does not).  Where /root/reference is present (the build
-container) the reference is also re-run live and compared with the committed fixtures.
+the reference's vit_flax/vit.py and simple_vit.py unmodified over oracle/flax_shim (a numpy restatement of the jax /
+flax API they use; its README states what that pins and what it does not).  Where VIT_FLAX_REFERENCE names the
+reference's vit_flax/ directory, the reference is also re-run live and compared with the committed fixtures.
 """
 import importlib.util
 import sys
@@ -124,7 +124,8 @@ def test_simple_vit_oracle_reproduces_the_reference_run(ref_simple):
     assert np.abs(y - ref_simple["logits"]).max() < 1e-10
 
 
-@pytest.mark.skipif(not mrg.reference_available(), reason="/root/reference exists only in the build container")
+@pytest.mark.skipif(not mrg.reference_available(),
+                    reason="needs the reference's sources: set VIT_FLAX_REFERENCE to a vit-flax checkout's vit_flax/ directory")
 def test_fixtures_are_what_the_reference_computes_today(ref_vit, ref_simple):
     vit_out, simple_out = mrg.generate()
     for want, got in ((ref_vit, vit_out), (ref_simple, simple_out)):
