@@ -162,6 +162,18 @@ int vitb200_train_forward(vitb200_model* m, void* stream, const float* images_de
  * 16-bit intermediates: with fp16 operands scale dlogits up (and the gradients down) yourself
  * when its entries are below ~1e-4 (loss scaling); gradients are linear in dlogits.             */
 int vitb200_backward(vitb200_model* m, void* stream, const float* dlogits_dev, int batch);
+/* What a backward differentiates with respect to (jax.vjp(v.apply, params, x) takes both): */
+#define VITB200_GRAD_PARAMS 1   /* one fp32 gradient per parameter leaf (vitb200_get_grad & co.)  */
+#define VITB200_GRAD_IMAGES 2   /* the gradient of the images given to train_forward            */
+/* wrt: a non-zero OR of the two flags.  dimages_dev: required iff VITB200_GRAD_IMAGES; fp32, the layout of the images
+ * given to train_forward ([B,H,W,C], or [B,C,H,W] for VITB200_FLAG_NCHW models), fully overwritten.  Image gradients are
+ * the same bits with or without VITB200_GRAD_PARAMS.  Without it the weight-gradient GEMMs are skipped (saliency /
+ * adversarial loops want dimages only) and vitb200_get_grad, vitb200_grad_device and vitb200_grads_buffer return
+ * VITB200_ERR_INVALID until a backward with VITB200_GRAD_PARAMS runs.  The first image-gradient backward allocates a
+ * [max_batch * T, round_up(ph*pw*C, 64)] fp32 scratch (patch-feature gradients) kept with the model.
+ * vitb200_backward(m, s, dl, b) == vitb200_backward_ex(m, s, dl, b, VITB200_GRAD_PARAMS, NULL).                    */
+int vitb200_backward_ex(vitb200_model* m, void* stream, const float* dlogits_dev, int batch,
+                        int wrt, float* dimages_dev);
 /* gradient of one leaf (flax path, same shape as the parameter) -> host; synchronises the stream */
 int vitb200_get_grad(vitb200_model* m, void* stream, const char* path, float* host_out);
 /* all leaf gradients as ONE contiguous fp32 buffer (leaves 256-byte aligned, padding zero): the unit of
@@ -284,6 +296,11 @@ int vitb200_patchify(void* stream, const float* images, void* patches, int batch
 int vitb200_patchify_tokens(void* stream, const float* images, void* patches, int batch,
                             int H, int W, int C, int ph, int pw, int Kpad, int out_dtype,
                             int nchw, int cls_slot);
+/* adjoint of vitb200_patchify_tokens with fp32 patches (the last step of an image-gradient backward):
+ * patches [batch*(Np+cls_slot), Kpad] fp32 -> images fp32 in the layout `nchw` selects.  A pure permutation: every
+ * pixel is written once; the pad columns and the class-token slot rows are not read. */
+int vitb200_unpatchify(void* stream, const float* patches, float* images, int batch, int H, int W,
+                       int C, int ph, int pw, int Kpad, int nchw, int cls_slot);
 /* cls rows (vit.py:151-153): x[b*T + 0, :] = cls + pos[0] */
 int vitb200_cls_rows(void* stream, const float* cls, const float* pos, float* x,
                      int batch, int T, int dim);

@@ -22,6 +22,7 @@ CATEGORIES = ["patchify", "gemm_patch", "cls_rows", "layernorm", "gemm_qkv", "at
               "gemm_ff1", "gemm_ff2", "pool_ln", "gemm_head"]
 EPI_STORE_16, EPI_BIAS_GELU_16, EPI_BIAS_RESID_F32, EPI_BIAS_F32, EPI_PATCH_F32, EPI_TOKENS_F32, EPI_BIAS_16, EPI_BIAS_PRE_GELU_16 = range(8)
 EPI_RESID_LN, EPI_TOKENS_LN, EPI_LN_STORE_16, EPI_LN_GELU_16 = range(8, 12)
+GRAD_PARAMS, GRAD_IMAGES = 1, 2
 
 
 class Config(C.Structure):
@@ -67,6 +68,7 @@ SIGNATURES = {
     "vitb200_debug_tokens": (_i, [_vp, _vp, _fp, _i]),
     "vitb200_train_forward": (_i, [_vp, _vp, _fp, _i, _fp]),
     "vitb200_backward": (_i, [_vp, _vp, _fp, _i]),
+    "vitb200_backward_ex": (_i, [_vp, _vp, _fp, _i, _i, _fp]),
     "vitb200_get_grad": (_i, [_vp, _vp, C.c_char_p, _fp]),
     "vitb200_grads_buffer": (_i, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
     "vitb200_grad_device": (_i, [_vp, C.c_char_p, C.POINTER(C.c_void_p)]),
@@ -86,6 +88,7 @@ SIGNATURES = {
     "vitb200_attention_f32": (_i, [_vp, _fp, _fp, _i, _i, _i]),
     "vitb200_patchify": (_i, [_vp, _fp, _vp, _i, _i, _i, _i, _i, _i, _i, _i]),
     "vitb200_patchify_tokens": (_i, [_vp, _fp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i]),
+    "vitb200_unpatchify": (_i, [_vp, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _i]),
     "vitb200_cls_rows": (_i, [_vp, _fp, _fp, _fp, _i, _i, _i]),
     "vitb200_pool_layernorm": (_i, [_vp, _fp, _fp, _fp, _vp, _i, _i, _i, _i, _i]),
     "vitb200_pack_weight": (_i, [_vp, _fp, _vp, _i, _i, _i, _i]),

@@ -180,7 +180,9 @@ struct vitb200_model {
     std::vector<TrainLayer> layers;
     DevBuf<float> dx, pooled_ln, dpl, zeros, grads, attn_ws;
     DevBuf<uint16_t> dy16, dhid16, dxn16, do16, dqkv16, tA, tB;
+    DevBuf<float> dpatches;               // [rows, K0pad] patch-feature gradient (first image-gradient backward)
     std::vector<size_t> grad_off;         // per leaf: element offset into grads
+    bool grads_valid = true;              // false after a backward that did not compute parameter gradients
   };
   std::unique_ptr<TrainState> train;
 
@@ -1046,6 +1048,14 @@ int ensure_train(vitb200_model* m, cudaStream_t st) {
   };
   for (auto& L : m->layers)
     if ((rc = make_wf(L.qkv)) || (rc = make_wf(L.out)) || (rc = make_wf(L.ff1)) || (rc = make_wf(L.ff2))) return rc;
+  {  // the patch Dense's copy (image gradients: dpatches = dY W^T) has K0pad rows, the ones past K0 zero, so that its
+     // output rows have the K0pad pitch of the patch matrix (an fp32 pitch of K0 = 147 floats is no legal TMA stride)
+    DenseW& d = m->patch;
+    const size_t n = size_t(m->K0pad) * d.N;
+    VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.wf), n * sizeof(uint16_t)));
+    VB_CUDA(cudaMemsetAsync(d.wf, 0, n * sizeof(uint16_t), st));
+    if ((rc = launch_cast16(st, m->leaves[d.leaf_kernel].dev, d.wf, int64_t(d.K) * d.N, m->dt))) return rc;
+  }
   m->train = std::move(ts);
   return 0;
 }
@@ -1113,28 +1123,33 @@ int vitb200_train_forward(vitb200_model* m, void* stream, const float* images, i
   return 0;
 }
 
-int vitb200_backward(vitb200_model* m, void* stream, const float* dlogits, int batch) {
-  if (!m || !dlogits) return fail(VITB200_ERR_INVALID, "backward: null argument");
-  if (m->train && m->train->fwd_batch == 0 && m->train->stale)
-    return fail(VITB200_ERR_INVALID, "backward: a forward ran on this handle since train_forward and overwrote its workspace; "
-                                     "call train_forward again");
-  if (!m->train || m->train->fwd_batch == 0) return fail(VITB200_ERR_INVALID, "backward: call train_forward first");
-  if (batch != m->train->fwd_batch) return fail(VITB200_ERR_INVALID, "backward: batch differs from the last train_forward");
-  if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "backward: parameters changed since train_forward");
-  DeviceGuard guard(m->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+namespace {
+
+// One backward schedule for every choice of what to differentiate with respect to.  The chain that carries the
+// token-stream cotangent dx from the logits to the images is the same kernels with the same arguments in the same order
+// whatever `wrt` is, so image gradients do not depend on whether parameter gradients are computed.  Without
+// VITB200_GRAD_PARAMS the weight-gradient GEMMs (4 per layer + the patch kernel's), the head's weight and bias gradients
+// and the token-embedding gradients are not launched; the column sums fused into the dx chain's own kernels still land in
+// the gradient buffer, which then reads as invalid (vitb200_get_grad & co. refuse).
+int backward_impl(vitb200_model* m, cudaStream_t st, const float* dlogits, int batch, int wrt, float* dimages) {
   auto& ts = *m->train;
   const auto& c = m->cfg;
   const int D = c.dim, I = m->inner, T = m->T, H = c.mlp_dim, R = batch * T, dt = m->dt;
+  const bool params = (wrt & VITB200_GRAD_PARAMS) != 0, images = (wrt & VITB200_GRAD_IMAGES) != 0;
   int rc;
+  if (images && ts.dpatches.n == 0) {   // first image-gradient backward: parameter-only callers never pay for it
+    if ((rc = ts.dpatches.alloc(size_t(c.max_batch) * T * m->K0pad))) return rc;
+  }
+  ts.grads_valid = params;
   // the nn.Dropout masks of the forward are pure functions of (key, site, element): replayed, never stored
   const uint64_t cur_key = m->dropout_key;
   m->dropout_key = ts.fwd_key;
   struct KeyRestore { vitb200_model* m; uint64_t k; ~KeyRestore() { m->dropout_key = k; } } restore{m, cur_key};
   VB_CUDA(cudaMemsetAsync(ts.grads.p, 0, ts.grads.n * sizeof(float), st));
   // head: logits = LN(pool(x)) Wh + bh   (vit.py:159-165)
-  if ((rc = launch_head_bwd(st, ts.pooled_ln.p, dlogits, leaf_ptr(m, m->head.leaf_kernel), grad_ptr(m, m->head.leaf_kernel),
-                            grad_ptr(m, m->head.leaf_bias), ts.dpl.p, batch, D, c.num_classes))) return rc;
+  if ((rc = launch_head_bwd(st, ts.pooled_ln.p, dlogits, leaf_ptr(m, m->head.leaf_kernel),
+                            params ? grad_ptr(m, m->head.leaf_kernel) : nullptr, params ? grad_ptr(m, m->head.leaf_bias) : nullptr,
+                            ts.dpl.p, batch, D, c.num_classes))) return rc;
   if ((rc = launch_pool_ln_bwd(st, ts.xs[2 * size_t(c.depth)].p, ts.dpl.p, leaf_ptr(m, m->leaf_head_scale), ts.dx.p,
                                grad_ptr(m, m->leaf_head_scale), grad_ptr(m, m->leaf_head_bias), batch, T, D, c.pool, m->eps))) return rc;
   // dy16 = cast(dx) (+ the replayed mask of the Dropout behind FF Dense_1) and its column sums = that bias gradient;
@@ -1146,21 +1161,21 @@ int vitb200_backward(vitb200_model* m, void* stream, const float* dlogits, int b
     auto& S = ts.layers[l];
     // ---- x2 = x1 + Dense_1(gelu(Dense_0(LN2(x1))))   (vit.py:39,47-53) ----
     if ((rc = gemm16(m, st, ts.dy16.p, R, D, L.ff2.wf, D, H, ts.dhid16.p, R, VITB200_EPI_STORE_16, nullptr))) return rc;
-    if ((rc = wgrad(m, st, S.hid, H, ts.dy16.p, D, R, grad_ptr(m, L.ff2.leaf_kernel), H))) return rc;
+    if (params && (rc = wgrad(m, st, S.hid, H, ts.dy16.p, D, R, grad_ptr(m, L.ff2.leaf_kernel), H))) return rc;
     if ((rc = launch_gelu_bwd_colsum(st, S.pre.p, ts.dhid16.p, ts.dhid16.p, grad_ptr(m, L.ff1.leaf_bias), R, H, dt,
                                      m->drop(c.dropout, 2 + 3 * l)))) return rc;
     if ((rc = gemm16(m, st, ts.dhid16.p, R, H, L.ff1.wf, H, D, ts.dxn16.p, R, VITB200_EPI_STORE_16, nullptr))) return rc;
-    if ((rc = wgrad(m, st, S.xn2.p, D, ts.dhid16.p, H, R, grad_ptr(m, L.ff1.leaf_kernel), D))) return rc;
+    if (params && (rc = wgrad(m, st, S.xn2.p, D, ts.dhid16.p, H, R, grad_ptr(m, L.ff1.leaf_kernel), D))) return rc;
     // LayerNorm adjoint; its dx is the cotangent of to_out's output: 16-bit copy + to_out bias gradient ride along
     if ((rc = launch_ln_bwd(st, ts.dxn16.p, ts.xs[2 * l + 1].p, leaf_ptr(m, L.ln2_scale), ts.dx.p, grad_ptr(m, L.ln2_scale),
                             grad_ptr(m, L.ln2_bias), R, D, dt, m->eps, 1, ts.dy16.p, grad_ptr(m, L.out.leaf_bias),
                             m->drop(c.dropout, 1 + 3 * l)))) return rc;
     // ---- x1 = x0 + to_out(attention(to_qkv(LN1(x0))))   (vit.py:39,62-87) ----
     if ((rc = gemm16(m, st, ts.dy16.p, R, D, L.out.wf, D, I, ts.do16.p, R, VITB200_EPI_STORE_16, nullptr))) return rc;
-    if ((rc = wgrad(m, st, S.o.p, I, ts.dy16.p, D, R, grad_ptr(m, L.out.leaf_kernel), I))) return rc;
+    if (params && (rc = wgrad(m, st, S.o.p, I, ts.dy16.p, D, R, grad_ptr(m, L.out.leaf_kernel), I))) return rc;
     if ((rc = launch_attention_bwd(st, S.qkv.p, S.o.p, ts.do16.p, ts.dqkv16.p, batch, T, c.heads, dt, ts.attn_ws.p, S.lse.p))) return rc;
     if ((rc = gemm16(m, st, ts.dqkv16.p, R, 3 * I, L.qkv.wf, 3 * I, D, ts.dxn16.p, R, VITB200_EPI_STORE_16, nullptr))) return rc;
-    if ((rc = wgrad(m, st, S.xn1.p, D, ts.dqkv16.p, 3 * I, R, grad_ptr(m, L.qkv.leaf_kernel), D))) return rc;
+    if (params && (rc = wgrad(m, st, S.xn1.p, D, ts.dqkv16.p, 3 * I, R, grad_ptr(m, L.qkv.leaf_kernel), D))) return rc;
     // its dx is the cotangent of the previous layer's FF Dense_1 output (layer 0: of the token embedding, handled below)
     if (l > 0) {
       if ((rc = launch_ln_bwd(st, ts.dxn16.p, ts.xs[2 * l].p, leaf_ptr(m, L.ln1_scale), ts.dx.p, grad_ptr(m, L.ln1_scale),
@@ -1173,17 +1188,54 @@ int vitb200_backward(vitb200_model* m, void* stream, const float* dlogits, int b
   }
   // ---- tokens = Dropout(concat(cls, patches W + b) + pos)   (vit.py:147-155) ----
   if ((rc = launch_mask_inplace(st, ts.dx.p, int64_t(R) * D, m->drop(c.emb_dropout, 0)))) return rc;
-  if ((rc = launch_token_grads(st, ts.dx.p, grad_ptr(m, m->leaf_pos), grad_ptr(m, m->leaf_cls), grad_ptr(m, m->patch.leaf_bias),
-                               batch, T, D, m->cls_off))) return rc;
+  if (params && (rc = launch_token_grads(st, ts.dx.p, grad_ptr(m, m->leaf_pos), grad_ptr(m, m->leaf_cls),
+                                         grad_ptr(m, m->patch.leaf_bias), batch, T, D, m->cls_off))) return rc;
   if ((rc = launch_cast16(st, ts.dx.p, ts.dy16.p, int64_t(R) * D, dt))) return rc;
   // the class-token slot rows of the patch matrix are zero, so their dx rows add nothing to dW
-  if ((rc = wgrad(m, st, m->patches_h.p, m->K0pad, ts.dy16.p, D, R, grad_ptr(m, m->patch.leaf_kernel), m->K0))) return rc;
+  if (params && (rc = wgrad(m, st, m->patches_h.p, m->K0pad, ts.dy16.p, D, R, grad_ptr(m, m->patch.leaf_kernel), m->K0))) return rc;
+  if (images) {
+    // ---- patches = patchify(images)   (vit.py:146) ----
+    // dpatches [R, K0pad] = dY W^T; the class-token slot rows come out as rows nobody reads, the pad columns as zeros
+    if ((rc = gemm16(m, st, ts.dy16.p, R, D, m->patch.wf, D, m->K0pad, ts.dpatches.p, R, VITB200_EPI_BIAS_F32, ts.zeros.p))) return rc;
+    if ((rc = launch_unpatchify(st, ts.dpatches.p, dimages, batch, c.image_h, c.image_w, c.channels, c.patch_h, c.patch_w,
+                                m->K0pad, m->nchw, m->cls_off))) return rc;
+  }
   return 0;
+}
+
+int grads_ready(const vitb200_model* m, const char* who) {
+  if (!m->train->grads_valid)
+    return fail(VITB200_ERR_INVALID, std::string(who) + ": the last backward did not compute parameter gradients "
+                                     "(run one with VITB200_GRAD_PARAMS)");
+  return 0;
+}
+
+}  // namespace
+
+int vitb200_backward_ex(vitb200_model* m, void* stream, const float* dlogits, int batch, int wrt, float* dimages) {
+  if (!m || !dlogits) return fail(VITB200_ERR_INVALID, "backward: null argument");
+  if (wrt == 0 || (wrt & ~(VITB200_GRAD_PARAMS | VITB200_GRAD_IMAGES)) != 0)
+    return fail(VITB200_ERR_INVALID, "backward: wrt must be a non-zero OR of VITB200_GRAD_PARAMS and VITB200_GRAD_IMAGES");
+  if ((wrt & VITB200_GRAD_IMAGES) && !dimages)
+    return fail(VITB200_ERR_INVALID, "backward: VITB200_GRAD_IMAGES needs an image-gradient buffer");
+  if (m->train && m->train->fwd_batch == 0 && m->train->stale)
+    return fail(VITB200_ERR_INVALID, "backward: a forward ran on this handle since train_forward and overwrote its workspace; "
+                                     "call train_forward again");
+  if (!m->train || m->train->fwd_batch == 0) return fail(VITB200_ERR_INVALID, "backward: call train_forward first");
+  if (batch != m->train->fwd_batch) return fail(VITB200_ERR_INVALID, "backward: batch differs from the last train_forward");
+  if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "backward: parameters changed since train_forward");
+  DeviceGuard guard(m->device);
+  return backward_impl(m, static_cast<cudaStream_t>(stream), dlogits, batch, wrt, dimages);
+}
+
+int vitb200_backward(vitb200_model* m, void* stream, const float* dlogits, int batch) {
+  return vitb200_backward_ex(m, stream, dlogits, batch, VITB200_GRAD_PARAMS, nullptr);
 }
 
 int vitb200_get_grad(vitb200_model* m, void* stream, const char* path, float* host_out) {
   if (!m || !path || !host_out) return fail(VITB200_ERR_INVALID, "get_grad: null argument");
   if (!m->train) return fail(VITB200_ERR_INVALID, "get_grad: no backward pass has run");
+  if (int rc = grads_ready(m, "get_grad")) return rc;
   auto it = m->index.find(path);
   if (it == m->index.end()) return fail(VITB200_ERR_INVALID, std::string("get_grad: unknown parameter path '") + path + "'");
   DeviceGuard guard(m->device);
@@ -1197,6 +1249,7 @@ int vitb200_get_grad(vitb200_model* m, void* stream, const char* path, float* ho
 int vitb200_grads_buffer(vitb200_model* m, float** dev_out, int64_t* count) {
   if (!m || !dev_out || !count) return fail(VITB200_ERR_INVALID, "grads_buffer: null argument");
   if (!m->train) return fail(VITB200_ERR_INVALID, "grads_buffer: no train_forward has run");
+  if (int rc = grads_ready(m, "grads_buffer")) return rc;
   *dev_out = m->train->grads.p;
   *count = int64_t(m->train->grads.n);
   return 0;
@@ -1205,6 +1258,7 @@ int vitb200_grads_buffer(vitb200_model* m, float** dev_out, int64_t* count) {
 int vitb200_grad_device(vitb200_model* m, const char* path, float** dev_out) {
   if (!m || !path || !dev_out) return fail(VITB200_ERR_INVALID, "grad_device: null argument");
   if (!m->train) return fail(VITB200_ERR_INVALID, "grad_device: no backward pass has run");
+  if (int rc = grads_ready(m, "grad_device")) return rc;
   auto it = m->index.find(path);
   if (it == m->index.end()) return fail(VITB200_ERR_INVALID, std::string("grad_device: unknown parameter path '") + path + "'");
   *dev_out = grad_ptr(m, it->second);
@@ -1392,6 +1446,14 @@ int vitb200_patchify_tokens(void* stream, const float* images, void* patches, in
     return fail(VITB200_ERR_INVALID, "patchify: nchw and cls_slot are 0 or 1");
   return launch_patchify(static_cast<cudaStream_t>(stream), images, patches, batch, H, W, C, ph, pw, Kpad, out_dtype,
                          nchw, cls_slot);
+}
+
+int vitb200_unpatchify(void* stream, const float* patches, float* images, int batch, int H, int W, int C, int ph, int pw,
+                       int Kpad, int nchw, int cls_slot) {
+  if (!patches || !images) return fail(VITB200_ERR_INVALID, "unpatchify: null pointer");
+  if ((nchw != 0 && nchw != 1) || (cls_slot != 0 && cls_slot != 1))
+    return fail(VITB200_ERR_INVALID, "unpatchify: nchw and cls_slot are 0 or 1");
+  return launch_unpatchify(static_cast<cudaStream_t>(stream), patches, images, batch, H, W, C, ph, pw, Kpad, nchw, cls_slot);
 }
 
 int vitb200_cls_rows(void* stream, const float* cls, const float* pos, float* x, int batch, int T, int dim) {

@@ -615,13 +615,16 @@ int launch_pool_ln_bwd(cudaStream_t st, const float* x, float* dpl, const float*
 int launch_head_bwd(cudaStream_t st, const float* pl, const float* dl, const float* W, float* dW, float* dbias,
                     float* dpl, int batch, int dim, int classes) {
   if (batch <= 0 || dim <= 0 || classes <= 0) return fail(VITB200_ERR_INVALID, "head_bwd: empty problem");
-  head_wgrad_kernel<<<dim3(unsigned((classes + 255) / 256), unsigned(dim)), 256, 0, st>>>(pl, dl, dW, batch, dim, classes);
-  VB_LAUNCH_CHECK("head_wgrad_kernel");
+  if (dW) {   // null: no parameter gradients wanted (image-only backward)
+    head_wgrad_kernel<<<dim3(unsigned((classes + 255) / 256), unsigned(dim)), 256, 0, st>>>(pl, dl, dW, batch, dim, classes);
+    VB_LAUNCH_CHECK("head_wgrad_kernel");
+  }
   head_dgrad_kernel<<<unsigned((int64_t(batch) * dim * 32 + 255) / 256), 256, 0, st>>>(dl, W, dpl, batch, dim, classes);
   VB_LAUNCH_CHECK("head_dgrad_kernel");
-  // dbias[c] += sum_b dl[b, c]  (classes may be odd: one column per thread)
-  pos_grad_kernel<<<dim3(unsigned((classes + 255) / 256), 1), 256, 0, st>>>(dl, dbias, batch, 1, classes);
-  VB_LAUNCH_CHECK("pos_grad_kernel(head bias)");
+  if (dbias) {   // dbias[c] += sum_b dl[b, c]  (classes may be odd: one column per thread)
+    pos_grad_kernel<<<dim3(unsigned((classes + 255) / 256), 1), 256, 0, st>>>(dl, dbias, batch, 1, classes);
+    VB_LAUNCH_CHECK("pos_grad_kernel(head bias)");
+  }
   return 0;
 }
 

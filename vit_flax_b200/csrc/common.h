@@ -142,6 +142,10 @@ int launch_attention_f32(cudaStream_t stream, const float* qkv, float* out, int 
                          int heads);
 int launch_patchify(cudaStream_t stream, const float* images, void* patches, int batch, int H,
                     int W, int C, int ph, int pw, int Kpad, int out_dtype, int nchw = 0, int tok_off = 0);
+// adjoint of launch_patchify for fp32 patches: images (NHWC, or NCHW) <- patches [batch*(Np+tok_off), Kpad]; every
+// pixel written once, the pad columns and the class-token slot rows never read
+int launch_unpatchify(cudaStream_t stream, const float* patches, float* images, int batch, int H, int W, int C,
+                      int ph, int pw, int Kpad, int nchw = 0, int tok_off = 0);
 int launch_cls_rows(cudaStream_t stream, const float* cls, const float* pos, float* x, int batch,
                     int T, int dim, const Dropout& drop = Dropout());
 int launch_pool_layernorm(cudaStream_t stream, const float* x, const float* scale,
@@ -181,6 +185,7 @@ int launch_ln_bwd(cudaStream_t stream, const void* dy, const float* x, const flo
 // dpl: in = gradient wrt LayerNorm(pooled), out = gradient wrt pooled (overwritten)
 int launch_pool_ln_bwd(cudaStream_t stream, const float* x, float* dpl, const float* gamma, float* dx,
                        float* dgamma, float* dbeta, int batch, int T, int dim, int pool_mean, float eps);
+// dW / dbias null: only dpl (the image-only backward)
 int launch_head_bwd(cudaStream_t stream, const float* pl, const float* dl, const float* W, float* dW,
                     float* dbias, float* dpl, int batch, int dim, int classes);
 int launch_token_grads(cudaStream_t stream, const float* dx, float* dpos, float* dcls, float* dbias, int batch,

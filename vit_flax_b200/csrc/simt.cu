@@ -1,6 +1,7 @@
 // simt.cu -- the CUDA-core kernels of the path:
 //   K2  LayerNorm (warp-shuffle, vectorised; fp32 in, 16-bit or fp32 out)    vit.py:31,163
 //   K1a patchify + fp32->16-bit cast (im2col folded into the mandatory cast) vit.py:146
+//       and its adjoint, unpatchify (fp32 patch-feature gradient -> image gradient)
 //   K1b cls rows (fp32 mode; the tensor-core path writes them in the patch GEMM) vit.py:151-153
 //   K5a pool (cls / mean) + head LayerNorm                                   vit.py:159-163
 //   K7  weight pack (fp32 [K,N] -> 16-bit [N,Kpad])
@@ -297,6 +298,70 @@ patchify_row4_kernel(const float* __restrict__ img, void* __restrict__ out, int 
           if constexpr (kDT != DT_F32) reinterpret_cast<uint32_t*>(out)[o >> 1] = 0u;
           else reinterpret_cast<float2*>(out)[o >> 1] = make_float2(0.f, 0.f);
         }
+      }
+    }
+  }
+}
+
+// ------------------------------------------------------ unpatchify (adjoint of K1a)
+// img[b, y, x, c] (or img[b, c, y, x]) = patches[row(b, patch of (y, x)), f(y, x, c)] -- the transpose of the patchify
+// permutation, fp32 in and out.  Patches do not overlap, so every pixel is written exactly once (no accumulation); the
+// pad columns K0..Kpad and the class-token slot rows (tok_off = 1) are never read.
+__global__ void __launch_bounds__(256)
+unpatchify_kernel(const float* __restrict__ patches, float* __restrict__ img, int batch, int H, int W, int C,
+                  int ph, int pw, int Kpad, int nchw, int tok_off) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int gw = W / pw, gh = H / ph;
+  const int64_t total = int64_t(batch) * H * W * C;
+  for (int64_t i = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; i < total; i += int64_t(gridDim.x) * blockDim.x) {
+    int64_t r = i;
+    int b, y, x, c;
+    if (nchw) {
+      x = int(r % W); r /= W;
+      y = int(r % H); r /= H;
+      c = int(r % C); b = int(r / C);
+    } else {
+      c = int(r % C); r /= C;
+      x = int(r % W); r /= W;
+      y = int(r % H); b = int(r / H);
+    }
+    const int hh = y / ph, p1 = y - hh * ph, ww = x / pw, p2 = x - ww * pw;
+    const int64_t row = (int64_t(b) * gh + hh) * gw + ww + (int64_t(b) + 1) * tok_off;
+    img[i] = __ldcs(patches + row * Kpad + (p1 * pw + p2) * C + c);
+  }
+}
+
+// NHWC fast path (pw*C and Kpad multiples of 4, 16-byte aligned buffers), the mirror of patchify_row4_kernel: a block
+// walks IMAGE ROWS (b, y); each float4 of the row is one 16-byte piece of a pw*C patch-row segment, read from the patch
+// matrix and stored coalesced into the image row.
+__global__ void __launch_bounds__(256)
+unpatchify_row4_kernel(const float* __restrict__ patches, float* __restrict__ img, int rows, int H, int W, int C,
+                       int ph, int pw, int Kpad, int tok_off) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int gw = W / pw, gh = H / ph;
+  const int seg4 = (pw * C) >> 2;          // float4 per patch-row segment
+  const int n4 = (W * C) >> 2;             // float4 per image row
+  constexpr int U = 4;                      // image rows in flight per thread (memory-level parallelism)
+  for (int r0 = blockIdx.x; r0 < rows; r0 += U * gridDim.x) {   // image row index b*H + y
+    for (int t = threadIdx.x; t < n4; t += blockDim.x) {
+      const int ww = t / seg4, rem4 = t - ww * seg4;
+      float4 v[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int r = r0 + u * gridDim.x;
+        if (r < rows) {
+          const int b = r / H, y = r - b * H;
+          const int hh = y / ph, p1 = y - hh * ph;
+          const int64_t o = ((int64_t(b) * gh + hh) * gw + ww + (b + 1) * tok_off) * Kpad + p1 * (seg4 << 2) + (rem4 << 2);
+          v[u] = __ldcs(reinterpret_cast<const float4*>(patches + o));
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int r = r0 + u * gridDim.x;
+        if (r < rows) reinterpret_cast<float4*>(img + int64_t(r) * W * C)[t] = v[u];
       }
     }
   }
@@ -606,6 +671,30 @@ int launch_patchify(cudaStream_t st, const float* images, void* patches, int bat
   const int grid = int(std::min<int64_t>((total + 255) / 256, int64_t(sm_count()) * 16));
   VB_DT_DISPATCH(out_dtype, (launch_kernel(patchify_kernel<kDT>, dim3(grid), dim3(256), 0, st, 1, images, patches, batch, H, W, C, ph, pw, Kpad, nchw, tok_off)));
   VB_LAUNCH_CHECK("patchify_kernel");
+  return 0;
+}
+
+int launch_unpatchify(cudaStream_t st, const float* patches, float* images, int batch, int H, int W, int C, int ph,
+                      int pw, int Kpad, int nchw, int tok_off) {
+  if (batch <= 0 || H <= 0 || W <= 0 || C <= 0 || ph <= 0 || pw <= 0)
+    return fail(VITB200_ERR_INVALID, "unpatchify: empty problem");
+  if (H % ph != 0 || W % pw != 0)
+    return fail(VITB200_ERR_INVALID, "unpatchify: image not divisible by patch (vit.py:133-134)");
+  if (Kpad < ph * pw * C) return fail(VITB200_ERR_INVALID, "unpatchify: Kpad must be >= ph*pw*C");
+  if (!nchw && ((pw * C) & 3) == 0 && (Kpad & 3) == 0 && (reinterpret_cast<uintptr_t>(images) & 15) == 0 &&
+      (reinterpret_cast<uintptr_t>(patches) & 15) == 0 && int64_t(batch) * H < (int64_t(1) << 31)) {
+    const int n4 = (W * C) >> 2;
+    const int threads = n4 >= 256 ? 256 : ((n4 + 31) / 32) * 32;
+    VB_CUDA(launch_kernel(unpatchify_row4_kernel, dim3(unsigned(std::min<int64_t>(int64_t(batch) * H, int64_t(sm_count()) * 8))),
+                          dim3(threads), 0, st, 1, patches, images, batch * H, H, W, C, ph, pw, Kpad, tok_off));
+    VB_LAUNCH_CHECK("unpatchify_row4_kernel");
+    return 0;
+  }
+  const int64_t total = int64_t(batch) * H * W * C;
+  const int grid = int(std::min<int64_t>((total + 255) / 256, int64_t(sm_count()) * 16));
+  VB_CUDA(launch_kernel(unpatchify_kernel, dim3(grid), dim3(256), 0, st, 1, patches, images, batch, H, W, C, ph, pw, Kpad,
+                        nchw, tok_off));
+  VB_LAUNCH_CHECK("unpatchify_kernel");
   return 0;
 }
 

@@ -15,6 +15,10 @@ from . import _lib
 from .params import flatten_params, geometry, leaf_to_numpy
 
 
+# Engine.backward(wrt=...) -> the VITB200_GRAD_* flags of vitb200_backward_ex
+_WRT = {"params": _lib.GRAD_PARAMS, "input": _lib.GRAD_IMAGES, "both": _lib.GRAD_PARAMS | _lib.GRAD_IMAGES}
+
+
 def _stream_ptr(torch, device) -> C.c_void_p:
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
@@ -131,12 +135,19 @@ class Engine:
                                                   images.data_ptr(), b, out.data_ptr()))
         return out
 
-    def backward(self, dlogits, epoch: Optional[int] = None) -> None:
+    def backward(self, dlogits, epoch: Optional[int] = None, *, wrt: str = "params", dimages=None):
         """Cotangent of the logits of the last ``train_forward`` (fp32 CUDA tensor [B, classes]) ->
         one fp32 gradient per parameter leaf, read with ``grads()`` / ``grad_tensor(path)``.
         ``epoch``: the value of ``self.epoch`` right after the ``train_forward`` this cotangent belongs
-        to; a mismatch means another forward / reload ran on this engine since and is an error."""
+        to; a mismatch means another forward / reload ran on this engine since and is an error.
+        ``wrt``: ``"params"`` (the leaf gradients), ``"input"`` (the gradient of the images only: the weight-gradient
+        GEMMs are skipped, and ``grads()`` & co. raise until a backward with parameters runs) or ``"both"``.  With
+        the images in ``wrt`` the image gradient is written to ``dimages`` (a contiguous float32 CUDA tensor of the
+        images' shape and layout; allocated when None) and returned; otherwise None is returned."""
         torch = self._torch
+        flags = _WRT.get(wrt)
+        if flags is None:
+            raise ValueError(f"wrt must be one of {sorted(_WRT)}, got {wrt!r}")
         if self.handle is None:
             raise RuntimeError("backward: this engine was closed (a larger batch re-created it); run vjp again")
         if epoch is not None and epoch != self.epoch:
@@ -145,8 +156,18 @@ class Engine:
         if dlogits.dtype != torch.float32 or not dlogits.is_cuda or not dlogits.is_contiguous() or dlogits.dim() != 2 \
                 or dlogits.shape[1] != self.num_classes:
             raise ValueError(f"backward expects a contiguous float32 CUDA tensor [B, {self.num_classes}]")
-        _lib.check(self.lib.vitb200_backward(self.handle, _stream_ptr(torch, dlogits.device),
-                                             dlogits.data_ptr(), int(dlogits.shape[0])))
+        b = int(dlogits.shape[0])
+        ptr = None
+        if flags & _lib.GRAD_IMAGES:
+            if dimages is None:
+                dimages = torch.empty((b, *self.image_shape), dtype=torch.float32, device=dlogits.device)
+            if dimages.dtype != torch.float32 or not dimages.is_cuda or not dimages.is_contiguous() \
+                    or tuple(dimages.shape) != (b, *self.image_shape):
+                raise ValueError(f"dimages must be a contiguous float32 CUDA tensor of shape {(b, *self.image_shape)}")
+            ptr = dimages.data_ptr()
+        _lib.check(self.lib.vitb200_backward_ex(self.handle, _stream_ptr(torch, dlogits.device),
+                                                dlogits.data_ptr(), b, flags, ptr))
+        return dimages if flags & _lib.GRAD_IMAGES else None
 
     def grad_tensor(self, path: str):
         """The gradient of one leaf as a CUDA tensor viewing the library's buffer (overwritten by the

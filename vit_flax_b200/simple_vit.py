@@ -34,7 +34,7 @@ from typing import Any, Dict, Optional, Tuple, Union
 import numpy as np
 
 from .params import _lecun_normal as lecun_normal, geometry, leaf_to_numpy
-from .vit import _current_device, _seed_from_key
+from .vit import _current_device, _parse_wrt, _seed_from_key, _unscale_images
 
 
 def posemb_sincos_2d(h: int, w: int, dim: int, temperature: float = 10000.0) -> np.ndarray:
@@ -199,10 +199,13 @@ class SimpleViT:
             return {"params": {"Dense_0": patch, "Transformer_0": t, "Sequential_0": {"layers_0": norm, "layers_1": head}}}
         return {"params": {"LayerNorm_0": norm, "Dense_0": head, "Dense_1": patch, "Transformer_0": t}}
 
-    def vjp(self, variables: Any, img: Any, *, precision: Optional[str] = None, device: Optional[int] = None,
-            max_batch: Optional[int] = None):
+    def vjp(self, variables: Any, img: Any, *, wrt: str = "params", precision: Optional[str] = None,
+            device: Optional[int] = None, max_batch: Optional[int] = None):
         """``jax.vjp(lambda p: v.apply(p, img), variables)`` (ours; simple_vit.py never differentiates):
-        ``(logits, vjp_fn)``, ``vjp_fn(dlogits)`` -> ``{'params': tree}`` of float32 gradients in SimpleViT's names."""
+        ``(logits, vjp_fn)``, ``vjp_fn(dlogits)`` -> ``{'params': tree}`` of float32 gradients in SimpleViT's names.
+        ``wrt="input"`` gives the float32 image gradient in the NCHW layout of ``img`` instead, ``wrt="both"``
+        ``({'params': tree}, dimg)`` (``ViT.vjp``)."""
+        want_params, want_input = _parse_wrt(wrt)
         import torch
         is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
         eng = self._engine(variables, img, precision, device, max_batch)
@@ -220,8 +223,13 @@ class SimpleViT:
                 raise ValueError(f"vjp_fn expects a cotangent of shape ({batch}, {self.num_classes})")
             peak = float(d.abs().max())
             scale = 1.0 if peak == 0.0 or not np.isfinite(peak) else float(2.0 ** -np.round(np.log2(peak)))
-            eng.backward(d * scale if scale != 1.0 else d, epoch=epoch)
-            return self._grads_tree({k: g / np.float32(scale) for k, g in eng.grads().items()}, layout)
+            dx = eng.backward(d * scale if scale != 1.0 else d, epoch=epoch, wrt=wrt)
+            out = []
+            if want_params:
+                out.append(self._grads_tree({k: g / np.float32(scale) for k, g in eng.grads().items()}, layout))
+            if want_input:
+                out.append(_unscale_images(dx, scale, is_cuda))
+            return out[0] if len(out) == 1 else tuple(out)
 
         return (logits if is_cuda else logits.cpu().numpy()), vjp_fn
 

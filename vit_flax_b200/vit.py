@@ -133,7 +133,7 @@ class ViT:
             return eng.forward(xin)
         return eng.forward_host(np.asarray(x, dtype=np.float32))
 
-    def vjp(self, variables: Any, x: Any, rngs: Any = None, *, precision: Optional[str] = None,
+    def vjp(self, variables: Any, x: Any, rngs: Any = None, *, wrt: str = "params", precision: Optional[str] = None,
             device: Optional[int] = None, max_batch: Optional[int] = None):
         """``jax.vjp(lambda p: v.apply(p, x), variables)`` (ours: nothing in the reference trains).
 
@@ -142,7 +142,13 @@ class ViT:
         in -> CUDA logits out (gradients always come back as numpy).  With fp16 operands the
         cotangent is scaled to unit magnitude on the way in and the gradients back on the way out
         (loss scaling: the map is linear).  With dropout rates > 0 pass ``rngs={'dropout': key}``: the
-        forward drops with that key's masks and ``vjp_fn`` differentiates that same dropped forward."""
+        forward drops with that key's masks and ``vjp_fn`` differentiates that same dropped forward.
+
+        ``wrt`` picks what ``vjp_fn`` differentiates with respect to: ``"params"`` (the default, above),
+        ``"input"`` -- ``dx``, the float32 gradient of the images with the shape of ``x`` (saliency maps,
+        FGSM / PGD); the weight-gradient GEMMs are skipped -- or ``"both"`` -- ``({'params': tree}, dx)``, the
+        order of ``jax.vjp(v.apply, variables, x)``.  ``dx`` is a CUDA tensor when ``x`` is one, numpy otherwise."""
+        want_params, want_input = _parse_wrt(wrt)
         from .runtime import get_engine
         import torch
         key = self._dropout_key(rngs)          # rates > 0 need rngs={'dropout': key}, like apply
@@ -167,9 +173,14 @@ class ViT:
                 raise ValueError(f"vjp_fn expects a cotangent of shape ({batch}, {self.num_classes})")
             peak = float(d.abs().max())
             scale = 1.0 if peak == 0.0 or not np.isfinite(peak) else float(2.0 ** -np.round(np.log2(peak)))
-            eng.backward(d * scale if scale != 1.0 else d, epoch=epoch)
-            from .checkpoint import _unflatten
-            return {"params": _unflatten({k: g / np.float32(scale) for k, g in eng.grads().items()})}
+            dx = eng.backward(d * scale if scale != 1.0 else d, epoch=epoch, wrt=wrt)
+            out = []
+            if want_params:
+                from .checkpoint import _unflatten
+                out.append({"params": _unflatten({k: g / np.float32(scale) for k, g in eng.grads().items()})})
+            if want_input:
+                out.append(_unscale_images(dx, scale, is_torch_cuda))
+            return out[0] if len(out) == 1 else tuple(out)
 
         return (logits if is_torch_cuda else logits.cpu().numpy()), vjp_fn
 
@@ -202,6 +213,21 @@ class ViT:
 
     def __call__(self, *a, **k):  # flax modules are called through init/apply
         raise TypeError("call ViT through .init(rngs, x) / .apply(variables, x), like the flax module")
+
+
+def _parse_wrt(wrt: str) -> Tuple[bool, bool]:
+    """``vjp(wrt=...)`` -> (parameter gradients?, image gradient?); checked before any device work."""
+    choices = {"params": (True, False), "input": (False, True), "both": (True, True)}
+    if wrt not in choices:
+        raise ValueError(f"wrt must be one of 'params', 'input' or 'both', got {wrt!r}")
+    return choices[wrt]
+
+
+def _unscale_images(dx, scale: float, as_cuda: bool):
+    """Undo the power-of-two cotangent scaling on an image gradient (exact) and hand it out like the logits."""
+    if scale != 1.0:
+        dx.div_(scale)
+    return dx if as_cuda else dx.cpu().numpy()
 
 
 def _current_device() -> int:
