@@ -182,6 +182,46 @@ int vitb200_grads_buffer(vitb200_model* m, float** dev_out, int64_t* count);
 /* device pointer of the same gradient (valid until the model is destroyed; overwritten by backward) */
 int vitb200_grad_device(vitb200_model* m, const char* path, float** dev_out);
 
+/* ---- on-device training step: AdamW on the fp32 leaves, then the 16-bit copies re-derived in place ----------------
+ * Semantics of optax.apply_if_finite(optax.chain(optax.clip_by_global_norm(max_grad_norm), optax.adamw(...))) with the
+ * gradient g = grads_buffer * grad_scale * clip, t = count + 1:
+ *   mu = b1 mu + (1 - b1) g;  nu = b2 nu + (1 - b2) g^2;  p -= lr ((mu / (1 - b1^t)) / (sqrt(nu / (1 - b2^t)) + eps) + wd p)
+ * (the weight-decay term only on DECAY leaves).  clip = max_grad_norm / max(norm, max_grad_norm), or 1 when
+ * max_grad_norm is 0; norm = the global norm of g over the TRAINABLE leaves.  When any such gradient is not finite the
+ * step is skipped: parameters, mu, nu and count stay bit for bit as they were and `skipped` reads 1.             */
+typedef struct vitb200_adamw {
+  float lr, b1, b2, eps, weight_decay;
+  float max_grad_norm;   /* 0 = no clipping (optax.clip_by_global_norm)                         */
+  float grad_scale;      /* multiplies the gradient buffer: 1 / (loss scale * data-parallel world) */
+  int32_t reserved[4];
+} vitb200_adamw;
+#define VITB200_LEAF_TRAINABLE 1   /* the leaf is updated (a frozen leaf is never read or written by the step) */
+#define VITB200_LEAF_DECAY     2   /* the weight-decay term applies (optax.adamw's mask)                      */
+/* num_params entries in param_info order; default: every leaf TRAINABLE | DECAY (optax.adamw without a mask) */
+int vitb200_set_leaf_flags(vitb200_model* m, const uint8_t* flags);
+/* Asynchronous (no host synchronisation): the gradient norm, the update and the re-derivation of every packed 16-bit
+ * weight copy (transposed packs, Flax-layout copies, LayerNorm folds) from the new fp32 leaves INTO THE SAME BUFFERS,
+ * so the captured small-batch forward graphs stay valid.  Needs a vitb200_backward_ex with VITB200_GRAD_PARAMS since
+ * the last step (else VITB200_ERR_INVALID); afterwards a backward whose train_forward ran before the step is refused.
+ * mu / nu (fp32, the layout of vitb200_grads_buffer) and the fold scratch are allocated by the first step.
+ * vitb200_set_param / vitb200_finalize_params do not touch mu, nu or count.  fp32 models: VITB200_ERR_UNSUPPORTED. */
+int vitb200_adamw_step(vitb200_model* m, void* stream, const vitb200_adamw* h);
+/* count, skipped and grad_norm (the norm of the last step, NaN when it was skipped); synchronises the stream */
+int vitb200_optim_status(vitb200_model* m, void* stream, int32_t* count, int32_t* skipped, float* grad_norm);
+/* device pointers of mu, nu ([n] fp32 each; leaf i at element offset sum_{j<i} round_up(numel_j, 64), padding zero) and
+ * of count (int32), for checkpoints and resumption; allocates them (zero) if no step has run yet, and then waits for the
+ * zeroing to finish, so the caller may write into them from any stream */
+int vitb200_optim_state(vitb200_model* m, float** mu_dev, float** nu_dev, int32_t** count_dev, int64_t* n);
+/* one fp32 parameter leaf (flax path) -> host; synchronises the stream */
+int vitb200_get_param(vitb200_model* m, void* stream, const char* path, float* host_out);
+/* optax.softmax_cross_entropy(logits, optax.smooth_labels(one_hot(labels), label_smoothing)).mean() and its gradient
+ * in one pass: logits [batch, classes] fp32, labels [batch] int32 (all DEVICE pointers) -> *loss_dev (fp32, reduced in
+ * a fixed order) and dlogits_dev = dscale * d loss / d logits.  A label outside [0, classes) makes the loss and its row
+ * of dlogits NaN (a following vitb200_adamw_step then skips).  All four buffers must be on one device; the kernels run
+ * there whatever device is current, and `stream` must belong to it.                                                */
+int vitb200_softmax_xent(void* stream, const float* logits, const int32_t* labels, int batch, int classes,
+                         float label_smoothing, float dscale, float* loss_dev, float* dlogits_dev);
+
 /* ---- per-kernel entry points (unit parity tests, ncu) -------------------
  * All pointers are DEVICE pointers.                                         */
 

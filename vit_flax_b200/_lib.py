@@ -23,6 +23,7 @@ CATEGORIES = ["patchify", "gemm_patch", "cls_rows", "layernorm", "gemm_qkv", "at
 EPI_STORE_16, EPI_BIAS_GELU_16, EPI_BIAS_RESID_F32, EPI_BIAS_F32, EPI_PATCH_F32, EPI_TOKENS_F32, EPI_BIAS_16, EPI_BIAS_PRE_GELU_16 = range(8)
 EPI_RESID_LN, EPI_TOKENS_LN, EPI_LN_STORE_16, EPI_LN_GELU_16 = range(8, 12)
 GRAD_PARAMS, GRAD_IMAGES = 1, 2
+LEAF_TRAINABLE, LEAF_DECAY = 1, 2
 
 
 class Config(C.Structure):
@@ -35,6 +36,12 @@ class Config(C.Structure):
         ("max_batch", C.c_int32), ("dropout", C.c_float), ("emb_dropout", C.c_float),
         ("flags", C.c_int32), ("ln_eps", C.c_float), ("reserved", C.c_int32 * 1),
     ]
+
+
+class AdamW(C.Structure):
+    _fields_ = [("lr", C.c_float), ("b1", C.c_float), ("b2", C.c_float), ("eps", C.c_float),
+                ("weight_decay", C.c_float), ("max_grad_norm", C.c_float), ("grad_scale", C.c_float),
+                ("reserved", C.c_int32 * 4)]
 
 
 class VitB200Error(RuntimeError):
@@ -72,6 +79,12 @@ SIGNATURES = {
     "vitb200_get_grad": (_i, [_vp, _vp, C.c_char_p, _fp]),
     "vitb200_grads_buffer": (_i, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
     "vitb200_grad_device": (_i, [_vp, C.c_char_p, C.POINTER(C.c_void_p)]),
+    "vitb200_set_leaf_flags": (_i, [_vp, C.POINTER(C.c_uint8)]),
+    "vitb200_adamw_step": (_i, [_vp, _vp, C.POINTER(AdamW)]),
+    "vitb200_optim_status": (_i, [_vp, _vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_float)]),
+    "vitb200_optim_state": (_i, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
+    "vitb200_get_param": (_i, [_vp, _vp, C.c_char_p, _fp]),
+    "vitb200_softmax_xent": (_i, [_vp, _fp, _fp, _i, _i, C.c_float, C.c_float, _fp, _fp]),
     "vitb200_gemm_tc_wgrad": (_i, [_vp, _vp, _vp, _fp, _i, _i, _i, _i, _i]),
     "vitb200_attention_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
     "vitb200_layernorm_bwd": (_i, [_vp, _vp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i, C.c_float, _i]),

@@ -2,6 +2,7 @@
 // (the Flax pytree of vit.py, looked up by path), weight packing, the forward
 // schedule of ViT.__call__ (vit.py:127-167) and the per-kernel entry points.
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <map>
 #include <memory>
@@ -109,6 +110,9 @@ struct vitb200_model {
   CUtensorMap patch_tm_i2c{};
   std::map<std::pair<const float*, int>, CUtensorMap> img_maps;   // im2col maps by (images pointer, batch)
   uint64_t dropout_key = 0;   // 'dropout' rng stream (vitb200_set_dropout_key)
+  uint64_t weights_version = 0;   // bumped by every vitb200_adamw_step: a backward must follow a forward on the same weights
+  std::vector<uint8_t> leaf_flags;   // VITB200_LEAF_* per leaf (vitb200_set_leaf_flags)
+  bool opt_table_dirty = true;       // the AdamW chunk table must be rebuilt from leaf_flags
 
   // the Dropout instance `site` of this model (rate 0 => off)
   Dropout drop(float rate, uint32_t site) const {
@@ -183,6 +187,15 @@ struct vitb200_model {
     DevBuf<float> dpatches;               // [rows, K0pad] patch-feature gradient (first image-gradient backward)
     std::vector<size_t> grad_off;         // per leaf: element offset into grads
     bool grads_valid = true;              // false after a backward that did not compute parameter gradients
+    bool grads_fresh = false;             // grads hold a parameter backward no optimiser step has consumed yet
+    uint64_t fwd_version = 0;             // weights_version of the last train_forward
+    // AdamW (allocated by the first step or vitb200_optim_state): moments in the layout of grads, the chunk table of the
+    // trainable leaves, the norm partials, the device-side status, the LayerNorm-fold scratch of the weight refresh
+    DevBuf<float> mu, nu, fold_scratch;
+    DevBuf<double> partial;
+    DevBuf<OptChunk> chunks;
+    std::vector<OptChunk> chunks_host;
+    DevBuf<OptStatus> status;
   };
   std::unique_ptr<TrainState> train;
 
@@ -326,13 +339,21 @@ int get_act_maps(vitb200_model* m, int batch, const ActMaps** out) {
   return 0;
 }
 
+// the 16-bit copies of one Dense kernel re-derived from its fp32 leaf, into the buffers they already have
+int repack_dense(vitb200_model* m, DenseW& d, cudaStream_t st) {
+  if (d.leaf_kernel < 0) return 0;
+  int rc = launch_pack_weight(st, m->leaves[d.leaf_kernel].dev, d.wt, d.K, d.N, d.Kpad, m->dt);
+  if (rc) return rc;
+  if (d.wf && (rc = launch_cast16(st, m->leaves[d.leaf_kernel].dev, d.wf, int64_t(d.K) * d.N, m->dt))) return rc;
+  return 0;
+}
+
 int pack_dense(vitb200_model* m, DenseW& d, cudaStream_t st) {
   if (d.leaf_kernel < 0) return 0;
   if (d.wt == nullptr)
     VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.wt), size_t(d.N) * d.Kpad * sizeof(uint16_t)));
-  int rc = launch_pack_weight(st, m->leaves[d.leaf_kernel].dev, d.wt, d.K, d.N, d.Kpad, m->dt);
+  int rc = repack_dense(m, d, st);
   if (rc) return rc;
-  if (d.wf && (rc = launch_cast16(st, m->leaves[d.leaf_kernel].dev, d.wf, int64_t(d.K) * d.N, m->dt))) return rc;
   if ((rc = make_tmap_2d(&d.tm, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN, m->dt))) return rc;
   if ((rc = make_tmap_2d(&d.tm2, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN / 2, m->dt))) return rc;
   return make_tmap_2d(&d.tm4, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN / 4, m->dt);
@@ -340,15 +361,22 @@ int pack_dense(vitb200_model* m, DenseW& d, cudaStream_t st) {
 
 inline const float* leaf_ptr(const vitb200_model* m, int idx) { return idx >= 0 ? m->leaves[idx].dev : nullptr; }
 
+// launch_fold_layernorm's K * N scratch for the largest folded Dense (to_qkv or FeedForward Dense_0)
+inline size_t fold_scratch_floats(const vitb200_model* m) { return size_t(m->cfg.dim) * std::max(3 * m->inner, m->cfg.mlp_dim); }
+
 // The Dense that follows a PreNorm, with that LayerNorm folded in (gemm_tc.cu header)
+int refold_dense(vitb200_model* m, DenseW& d, int ln_scale, int ln_bias, float* scratch, cudaStream_t st) {
+  return launch_fold_layernorm(st, m->leaves[d.leaf_kernel].dev, leaf_ptr(m, ln_scale), leaf_ptr(m, ln_bias),
+                               leaf_ptr(m, d.leaf_bias), d.wt_ln, d.ln_c, d.ln_d, d.K, d.N, d.Kpad, m->dt, scratch);
+}
+
 int fold_dense(vitb200_model* m, DenseW& d, int ln_scale, int ln_bias, float* scratch, cudaStream_t st) {
   if (d.wt_ln == nullptr) {
     VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.wt_ln), size_t(d.N) * d.Kpad * sizeof(uint16_t)));
     VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.ln_c), size_t(d.N) * sizeof(float)));
     VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.ln_d), size_t(d.N) * sizeof(float)));
   }
-  int rc = launch_fold_layernorm(st, m->leaves[d.leaf_kernel].dev, leaf_ptr(m, ln_scale), leaf_ptr(m, ln_bias),
-                                 leaf_ptr(m, d.leaf_bias), d.wt_ln, d.ln_c, d.ln_d, d.K, d.N, d.Kpad, m->dt, scratch);
+  int rc = refold_dense(m, d, ln_scale, ln_bias, scratch, st);
   if (rc) return rc;
   if ((rc = make_tmap_2d(&d.tm_ln, d.wt_ln, d.N, d.Kpad, d.Kpad, GEMM_BN, m->dt))) return rc;
   if ((rc = make_tmap_2d(&d.tm2_ln, d.wt_ln, d.N, d.Kpad, d.Kpad, GEMM_BN / 2, m->dt))) return rc;
@@ -666,6 +694,7 @@ int vitb200_create(const vitb200_config* cfg, int device, vitb200_model** out) {
   if (!m->tc && m->K0pad != m->K0)
     return fail(VITB200_ERR_UNSUPPORTED, "create: fp32 mode needs an even patch feature count");
   build_registry(m.get());
+  m->leaf_flags.assign(m->leaves.size(), VITB200_LEAF_TRAINABLE | VITB200_LEAF_DECAY);
   int rc = alloc_workspace(m.get());
   if (rc) return rc;
   *out = m.release();
@@ -738,7 +767,7 @@ int vitb200_finalize_params(vitb200_model* m, void* stream) {
     }
     if (m->fold) {
       DevBuf<float> scratch;
-      if ((rc = scratch.alloc(size_t(m->cfg.dim) * std::max(3 * m->inner, m->cfg.mlp_dim)))) return rc;
+      if ((rc = scratch.alloc(fold_scratch_floats(m)))) return rc;
       for (auto& L : m->layers) {
         if ((rc = fold_dense(m, L.qkv, L.ln1_scale, L.ln1_bias, scratch.p, st))) return rc;
         if ((rc = fold_dense(m, L.ff1, L.ln2_scale, L.ln2_bias, scratch.p, st))) return rc;
@@ -1120,6 +1149,7 @@ int vitb200_train_forward(vitb200_model* m, void* stream, const float* images, i
   }
   ts.fwd_batch = batch;
   ts.fwd_key = m->dropout_key;
+  ts.fwd_version = m->weights_version;
   return 0;
 }
 
@@ -1141,6 +1171,7 @@ int backward_impl(vitb200_model* m, cudaStream_t st, const float* dlogits, int b
     if ((rc = ts.dpatches.alloc(size_t(c.max_batch) * T * m->K0pad))) return rc;
   }
   ts.grads_valid = params;
+  ts.grads_fresh = params;
   // the nn.Dropout masks of the forward are pure functions of (key, site, element): replayed, never stored
   const uint64_t cur_key = m->dropout_key;
   m->dropout_key = ts.fwd_key;
@@ -1223,6 +1254,8 @@ int vitb200_backward_ex(vitb200_model* m, void* stream, const float* dlogits, in
                                      "call train_forward again");
   if (!m->train || m->train->fwd_batch == 0) return fail(VITB200_ERR_INVALID, "backward: call train_forward first");
   if (batch != m->train->fwd_batch) return fail(VITB200_ERR_INVALID, "backward: batch differs from the last train_forward");
+  if (m->train->fwd_version != m->weights_version)
+    return fail(VITB200_ERR_INVALID, "backward: an optimiser step changed the weights since train_forward; call train_forward again");
   if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "backward: parameters changed since train_forward");
   DeviceGuard guard(m->device);
   return backward_impl(m, static_cast<cudaStream_t>(stream), dlogits, batch, wrt, dimages);
@@ -1263,6 +1296,185 @@ int vitb200_grad_device(vitb200_model* m, const char* path, float** dev_out) {
   if (it == m->index.end()) return fail(VITB200_ERR_INVALID, std::string("grad_device: unknown parameter path '") + path + "'");
   *dev_out = grad_ptr(m, it->second);
   return 0;
+}
+
+// ---- on-device training step (optim.cu) ------------------------------------------------------------------------------
+namespace {
+
+int check_adamw(const vitb200_adamw& h) {
+  auto finite = [](float v) { return std::isfinite(v); };
+  if (!finite(h.lr) || h.lr < 0.f) return fail(VITB200_ERR_INVALID, "adamw_step: lr must be finite and >= 0");
+  if (!(h.b1 >= 0.f && h.b1 < 1.f) || !(h.b2 >= 0.f && h.b2 < 1.f))
+    return fail(VITB200_ERR_INVALID, "adamw_step: b1 and b2 must be in [0, 1)");
+  if (!finite(h.eps) || h.eps < 0.f) return fail(VITB200_ERR_INVALID, "adamw_step: eps must be finite and >= 0");
+  if (!finite(h.weight_decay) || h.weight_decay < 0.f) return fail(VITB200_ERR_INVALID, "adamw_step: weight_decay must be finite and >= 0");
+  if (!finite(h.max_grad_norm) || h.max_grad_norm < 0.f) return fail(VITB200_ERR_INVALID, "adamw_step: max_grad_norm must be finite and >= 0");
+  if (!finite(h.grad_scale) || !(h.grad_scale > 0.f)) return fail(VITB200_ERR_INVALID, "adamw_step: grad_scale must be finite and > 0");
+  return 0;
+}
+
+// moments, status and scratch of the optimiser; the moments start at zero, count at 0
+int ensure_optim(vitb200_model* m, cudaStream_t st) {
+  auto& ts = *m->train;
+  if (ts.status.n) return 0;
+  int rc;
+  if ((rc = ts.mu.alloc(ts.grads.n)) || (rc = ts.nu.alloc(ts.grads.n)) || (rc = ts.status.alloc(1))) return rc;
+  VB_CUDA(cudaMemsetAsync(ts.mu.p, 0, ts.mu.n * sizeof(float), st));
+  VB_CUDA(cudaMemsetAsync(ts.nu.p, 0, ts.nu.n * sizeof(float), st));
+  VB_CUDA(cudaMemsetAsync(ts.status.p, 0, sizeof(OptStatus), st));
+  if (m->fold && (rc = ts.fold_scratch.alloc(fold_scratch_floats(m)))) return rc;
+  return 0;
+}
+
+// chunks of OPT_CHUNK elements over the trainable leaves; rebuilt when the leaf flags change (stream-ordered upload)
+int build_chunk_table(vitb200_model* m, cudaStream_t st) {
+  auto& ts = *m->train;
+  if (!m->opt_table_dirty && ts.chunks.n) return 0;
+  ts.chunks_host.clear();
+  for (size_t i = 0; i < m->leaves.size(); ++i) {
+    if (!(m->leaf_flags[i] & VITB200_LEAF_TRAINABLE)) continue;
+    const int64_t n = m->leaves[i].numel();
+    const int32_t decay = (m->leaf_flags[i] & VITB200_LEAF_DECAY) ? 1 : 0;
+    for (int64_t s = 0; s < n; s += OPT_CHUNK)
+      ts.chunks_host.push_back({m->leaves[i].dev + s, int64_t(ts.grad_off[i]) + s, int32_t(std::min<int64_t>(OPT_CHUNK, n - s)), decay});
+  }
+  if (!ts.chunks.n) {   // sized once for every leaf trainable: a later change of the flags allocates (and syncs) nothing
+    size_t nc = 0;
+    for (const auto& l : m->leaves) nc += size_t((l.numel() + OPT_CHUNK - 1) / OPT_CHUNK);
+    int rc;
+    if ((rc = ts.chunks.alloc(std::max<size_t>(nc, 1))) || (rc = ts.partial.alloc(std::max<size_t>(nc, 1)))) return rc;
+  }
+  if (!ts.chunks_host.empty())
+    VB_CUDA(cudaMemcpyAsync(ts.chunks.p, ts.chunks_host.data(), ts.chunks_host.size() * sizeof(OptChunk), cudaMemcpyHostToDevice, st));
+  m->opt_table_dirty = false;
+  return 0;
+}
+
+// every 16-bit copy the kernels read, re-derived from the fp32 leaves into the same buffers: pointers, tensor maps and
+// the captured forward graphs stay valid, and nothing synchronises
+int refresh_packed(vitb200_model* m, cudaStream_t st) {
+  int rc;
+  if ((rc = repack_dense(m, m->patch, st))) return rc;
+  for (auto& L : m->layers)
+    if ((rc = repack_dense(m, L.qkv, st)) || (rc = repack_dense(m, L.out, st)) || (rc = repack_dense(m, L.ff1, st)) ||
+        (rc = repack_dense(m, L.ff2, st))) return rc;
+  if (m->head_tc && (rc = repack_dense(m, m->head, st))) return rc;
+  if (m->im2col) {
+    const auto& c = m->cfg;
+    if ((rc = launch_pack_weight_im2col(st, m->leaves[m->patch.leaf_kernel].dev, m->patch_wt_i2c, c.dim, c.patch_h,
+                                        c.patch_w * c.channels, m->dt))) return rc;
+  }
+  if (m->fold) {
+    float* scratch = m->train->fold_scratch.p;
+    for (auto& L : m->layers)
+      if ((rc = refold_dense(m, L.qkv, L.ln1_scale, L.ln1_bias, scratch, st)) ||
+          (rc = refold_dense(m, L.ff1, L.ln2_scale, L.ln2_bias, scratch, st))) return rc;
+  }
+  return 0;
+}
+
+}  // namespace
+
+int vitb200_set_leaf_flags(vitb200_model* m, const uint8_t* flags) {
+  if (!m || !flags) return fail(VITB200_ERR_INVALID, "set_leaf_flags: null argument");
+  for (size_t i = 0; i < m->leaves.size(); ++i)
+    if (flags[i] & ~(VITB200_LEAF_TRAINABLE | VITB200_LEAF_DECAY))
+      return fail(VITB200_ERR_INVALID, "set_leaf_flags: unknown flag bits for '" + m->leaves[i].path + "'");
+  m->leaf_flags.assign(flags, flags + m->leaves.size());
+  m->opt_table_dirty = true;
+  return 0;
+}
+
+int vitb200_adamw_step(vitb200_model* m, void* stream, const vitb200_adamw* h) {
+  if (!m || !h) return fail(VITB200_ERR_INVALID, "adamw_step: null argument");
+  int rc;
+  if ((rc = train_supported(m))) return rc;
+  if ((rc = check_adamw(*h))) return rc;
+  if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "adamw_step: parameters changed since the backward; call finalize_params");
+  if (!m->train || !m->train->grads_fresh)
+    return fail(VITB200_ERR_INVALID, "adamw_step: needs a backward with VITB200_GRAD_PARAMS since the last step");
+  DeviceGuard guard(m->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  auto& ts = *m->train;
+  if ((rc = ensure_optim(m, st)) || (rc = build_chunk_table(m, st))) return rc;
+  if ((rc = launch_adamw(st, ts.chunks.p, int(ts.chunks_host.size()), ts.grads.p, ts.mu.p, ts.nu.p, ts.partial.p,
+                         ts.status.p, *h))) return rc;
+  if ((rc = refresh_packed(m, st))) return rc;
+  ts.grads_fresh = false;
+  ++m->weights_version;
+  return 0;
+}
+
+int vitb200_optim_status(vitb200_model* m, void* stream, int32_t* count, int32_t* skipped, float* grad_norm) {
+  if (!m || !count || !skipped || !grad_norm) return fail(VITB200_ERR_INVALID, "optim_status: null argument");
+  *count = 0;
+  *skipped = 0;
+  *grad_norm = 0.f;
+  if (!m->train || !m->train->status.n) return 0;
+  DeviceGuard guard(m->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  OptStatus s;
+  VB_CUDA(cudaMemcpyAsync(&s, m->train->status.p, sizeof(s), cudaMemcpyDeviceToHost, st));
+  VB_CUDA(cudaStreamSynchronize(st));
+  *count = s.count;
+  *skipped = s.skipped;
+  *grad_norm = s.norm;
+  return 0;
+}
+
+int vitb200_optim_state(vitb200_model* m, float** mu_dev, float** nu_dev, int32_t** count_dev, int64_t* n) {
+  if (!m || !mu_dev || !nu_dev || !count_dev || !n) return fail(VITB200_ERR_INVALID, "optim_state: null argument");
+  int rc;
+  if ((rc = train_supported(m))) return rc;
+  if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "optim_state: call finalize_params first");
+  DeviceGuard guard(m->device);
+  // allocated here, the buffers are zeroed on the legacy stream; the caller may write into them at once from any stream
+  // (a checkpoint restored before the first step), so this first-allocation path waits for the zeroing to finish
+  const bool fresh = !m->train || !m->train->status.n;
+  cudaStream_t st = nullptr;
+  if ((rc = ensure_train(m, st)) || (rc = ensure_optim(m, st))) return rc;
+  if (fresh) VB_CUDA(cudaStreamSynchronize(st));
+  *mu_dev = m->train->mu.p;
+  *nu_dev = m->train->nu.p;
+  *count_dev = &m->train->status.p->count;
+  *n = int64_t(m->train->mu.n);
+  return 0;
+}
+
+int vitb200_get_param(vitb200_model* m, void* stream, const char* path, float* host_out) {
+  if (!m || !path || !host_out) return fail(VITB200_ERR_INVALID, "get_param: null argument");
+  auto it = m->index.find(path);
+  if (it == m->index.end()) return fail(VITB200_ERR_INVALID, std::string("get_param: unknown parameter path '") + path + "'");
+  const Leaf& l = m->leaves[it->second];
+  if (!l.set) return fail(VITB200_ERR_PARAM_MISSING, std::string("get_param: parameter '") + path + "' was never set");
+  DeviceGuard guard(m->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  VB_CUDA(cudaMemcpyAsync(host_out, l.dev, size_t(l.numel()) * sizeof(float), cudaMemcpyDeviceToHost, st));
+  VB_CUDA(cudaStreamSynchronize(st));
+  return 0;
+}
+
+int vitb200_softmax_xent(void* stream, const float* logits, const int32_t* labels, int batch, int classes,
+                         float label_smoothing, float dscale, float* loss_dev, float* dlogits_dev) {
+  if (!logits || !labels || !loss_dev || !dlogits_dev) return fail(VITB200_ERR_INVALID, "softmax_xent: null pointer");
+  if (batch <= 0 || classes <= 0) return fail(VITB200_ERR_INVALID, "softmax_xent: batch and classes must be positive");
+  if (!(label_smoothing >= 0.f && label_smoothing <= 1.f)) return fail(VITB200_ERR_INVALID, "softmax_xent: label_smoothing must be in [0, 1]");
+  if (!std::isfinite(dscale)) return fail(VITB200_ERR_INVALID, "softmax_xent: dscale must be finite");
+  // the kernels and their scratch go to the device that holds the buffers, whichever device is current
+  int dev = -1;
+  const void* bufs[4] = {logits, labels, loss_dev, dlogits_dev};
+  for (const void* b : bufs) {
+    cudaPointerAttributes a{};
+    VB_CUDA(cudaPointerGetAttributes(&a, b));
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+      return fail(VITB200_ERR_INVALID, "softmax_xent: logits, labels, loss and dlogits must be device memory");
+    if (dev >= 0 && a.device != dev) return fail(VITB200_ERR_INVALID, "softmax_xent: buffers on different devices");
+    dev = a.device;
+  }
+  DeviceGuard guard(dev);
+  if (!guard.ok) return fail(VITB200_ERR_CUDA, "softmax_xent: cudaSetDevice failed");
+  return launch_softmax_xent(static_cast<cudaStream_t>(stream), logits, labels, batch, classes, label_smoothing, dscale,
+                             loss_dev, dlogits_dev);
 }
 
 // ---- per-kernel entry points ------------------------------------------------

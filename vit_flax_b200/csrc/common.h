@@ -210,4 +210,26 @@ int launch_dq_convert(cudaStream_t stream, const float* dq_acc, void* dqkv, int6
 int launch_attention_bwd_rowdot(cudaStream_t stream, const void* d_out, const void* o_fwd, float* dsum, int batch, int T,
                                 int heads, int dtype);
 
+// ---- training step (optim.cu) ----
+// softmax cross-entropy of logits [B, C] with smoothed one-hot labels: mean loss -> *loss, dscale * dloss/dlogits
+int launch_softmax_xent(cudaStream_t stream, const float* logits, const int32_t* labels, int B, int C, float eps,
+                        float dscale, float* loss, float* dlogits);
+constexpr int OPT_CHUNK = 8192;   // elements of a leaf per CTA of the AdamW kernels
+struct OptChunk {                 // one chunk of a trainable leaf: p = leaf + start, off = grad offset of the leaf + start
+  float* p;
+  int64_t off;                    // into the gradient buffer and mu / nu (same layout)
+  int32_t n;                      // elements, <= OPT_CHUNK; a multiple of 4 except in a leaf's last chunk
+  int32_t decay;
+};
+struct OptStatus {                // device-side state of the optimiser, written by the step itself
+  float norm;                     // global norm of grad * grad_scale of the last step (NaN: non-finite gradients)
+  int32_t count;                  // applied updates (optax's count)
+  int32_t skipped;                // the last step was skipped
+  int32_t apply;                  // what the update kernel obeys
+  float gmul, bc1, bc2;           // grad_scale * clip, 1 - b1^t, 1 - b2^t of the last applied step
+};
+// global norm (per-chunk partials, then a fixed-order reduction), the step decision, the fused update: 3 launches
+int launch_adamw(cudaStream_t stream, const OptChunk* chunks, int nchunks, const float* grads, float* mu, float* nu,
+                 double* partial, OptStatus* status, const vitb200_adamw& h);
+
 }  // namespace vb

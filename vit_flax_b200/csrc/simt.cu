@@ -454,19 +454,34 @@ pack_weight_kernel(const float* __restrict__ W, uint16_t* __restrict__ Wt, int K
 
 // ------------------------------------------------ LayerNorm fold, weight side
 // (gemm_tc.cu header)  Ws[k, n] = gamma[k] W[k, n]; d[n] = sum_k beta[k] W[k, n] (+ bias[n]); c[n] = sum_k of the
-// 16-bit ROUNDED packed row Wt[n, :].  Run once per weight load, not on the forward path.
+// 16-bit ROUNDED packed row Wt[n, :].  Run per weight load and after every optimiser step (the in-place refresh).
+// One CTA per 32 columns: all eight warps stream FOLD_ROWS-row slabs of W (coalesced over n) into shared memory and
+// write Ws, then warp 0 carries each column's d chain through the slab -- the same fmaf sequence k = 0 .. K-1 as one
+// thread per column, with the loads of a whole CTA in flight instead of one per thread.
+constexpr int FOLD_ROWS = 128;
 __global__ void __launch_bounds__(256)
 fold_scale_kernel(const float* __restrict__ W, const float* __restrict__ gamma, const float* __restrict__ beta,
                   const float* __restrict__ bias, float* __restrict__ Ws, float* __restrict__ d, int K, int N) {
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;     // one column per thread: coalesced over n for every k
-  if (n >= N) return;
-  float acc = bias ? bias[n] : 0.f;
-  for (int k = 0; k < K; ++k) {
-    const float w = W[int64_t(k) * N + n];
-    Ws[int64_t(k) * N + n] = gamma[k] * w;
-    acc = fmaf(beta[k], w, acc);
+  __shared__ float tile[FOLD_ROWS][33];
+  __shared__ float bs[FOLD_ROWS];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int n = blockIdx.x * 32 + lane;
+  float acc = (n < N && bias) ? bias[n] : 0.f;
+  for (int k0 = 0; k0 < K; k0 += FOLD_ROWS) {
+    const int rows = min(FOLD_ROWS, K - k0);
+    for (int r = warp; r < rows; r += 8) {
+      const int64_t i = int64_t(k0 + r) * N + n;
+      const float w = n < N ? W[i] : 0.f;
+      if (n < N) Ws[i] = gamma[k0 + r] * w;
+      tile[r][lane] = w;
+    }
+    for (int r = threadIdx.x; r < rows; r += blockDim.x) bs[r] = beta[k0 + r];
+    __syncthreads();
+    if (warp == 0)
+      for (int r = 0; r < rows; ++r) acc = fmaf(bs[r], tile[r][lane], acc);
+    __syncthreads();
   }
-  d[n] = acc;
+  if (warp == 0 && n < N) d[n] = acc;
 }
 template <int kDT>
 __global__ void __launch_bounds__(256)
@@ -729,7 +744,7 @@ int launch_fold_layernorm(cudaStream_t st, const float* W, const float* gamma, c
                           void* Wt, float* c, float* d, int K, int N, int Kpad, int dtype, float* scratch) {
   if (dtype != DT_BF16 && dtype != DT_F16) return fail(VITB200_ERR_INVALID, "fold_layernorm: dtype must be bf16 or fp16");
   if (K <= 0 || N <= 0 || Kpad < K) return fail(VITB200_ERR_INVALID, "fold_layernorm: bad shape");
-  fold_scale_kernel<<<ceil_div(N, 256), 256, 0, st>>>(W, gamma, beta, bias, scratch, d, K, N);
+  fold_scale_kernel<<<ceil_div(N, 32), 256, 0, st>>>(W, gamma, beta, bias, scratch, d, K, N);
   VB_LAUNCH_CHECK("fold_scale_kernel");
   int rc = launch_pack_weight(st, scratch, Wt, K, N, Kpad, dtype);
   if (rc) return rc;

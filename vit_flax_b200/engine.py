@@ -204,6 +204,84 @@ class Engine:
             out[path] = a
         return out
 
+    # -- on-device training step (vit_flax_b200.train.Trainer) --------------------
+    def set_leaf_flags(self, flags: Dict[str, int]) -> None:
+        """``{path: LEAF_TRAINABLE | LEAF_DECAY bits}`` for every leaf of ``param_table()``."""
+        paths = list(self.param_table())
+        if set(flags) != set(paths):
+            raise ValueError(f"set_leaf_flags needs one entry per leaf: missing={sorted(set(paths) - set(flags))[:4]} "
+                             f"unexpected={sorted(set(flags) - set(paths))[:4]}")
+        arr = (C.c_uint8 * len(paths))(*[int(flags[p]) for p in paths])
+        _lib.check(self.lib.vitb200_set_leaf_flags(self.handle, arr))
+
+    def adamw_step(self, *, lr: float, b1: float, b2: float, eps: float, weight_decay: float,
+                   max_grad_norm: float = 0.0, grad_scale: float = 1.0) -> None:
+        """One AdamW update of the fp32 leaves from the gradient buffer of the last ``backward`` (scaled by
+        ``grad_scale``), with the 16-bit weight copies re-derived in place.  Asynchronous; a pending ``vjp_fn``
+        of this engine is invalidated (its forward ran on the old weights)."""
+        h = _lib.AdamW(lr=lr, b1=b1, b2=b2, eps=eps, weight_decay=weight_decay, max_grad_norm=max_grad_norm,
+                       grad_scale=grad_scale)
+        self.epoch += 1
+        _lib.check(self.lib.vitb200_adamw_step(self.handle, _stream_ptr(self._torch, self.device), C.byref(h)))
+
+    def optim_status(self):
+        """``(count, skipped, grad_norm)`` of the last step; synchronises."""
+        count, skipped, norm = C.c_int32(), C.c_int32(), C.c_float()
+        _lib.check(self.lib.vitb200_optim_status(self.handle, _stream_ptr(self._torch, self.device),
+                                                 C.byref(count), C.byref(skipped), C.byref(norm)))
+        return int(count.value), int(skipped.value), float(norm.value)
+
+    def optim_state(self):
+        """``(mu, nu, count)``: CUDA tensor views of the optimiser's buffers (mu / nu flat, in the layout of
+        ``grads_flat()`` and ``leaf_offsets()``; count a 1-element int32 tensor)."""
+        mu, nu, cnt, n = C.c_void_p(), C.c_void_p(), C.c_void_p(), C.c_int64()
+        _lib.check(self.lib.vitb200_optim_state(self.handle, C.byref(mu), C.byref(nu), C.byref(cnt), C.byref(n)))
+        return (_device_view(self._torch, self.device, mu.value, int(n.value), "<f4"),
+                _device_view(self._torch, self.device, nu.value, int(n.value), "<f4"),
+                _device_view(self._torch, self.device, cnt.value, 1, "<i4"))
+
+    def leaf_offsets(self) -> Dict[str, tuple]:
+        """``{path: (element offset, shape)}`` of every leaf in the flat gradient / moment buffers (leaves in
+        ``param_table`` order, each padded to a multiple of 64 elements)."""
+        out, off = {}, 0
+        for path, shape in self.param_table().items():
+            out[path] = (off, shape)
+            off += -(-int(np.prod(shape)) // 64) * 64
+        return out
+
+    def get_param(self, path: str) -> np.ndarray:
+        """The current fp32 value of one leaf (after optimiser steps, the trained one); synchronises."""
+        a = np.empty(self.param_table()[path], np.float32)
+        _lib.check(self.lib.vitb200_get_param(self.handle, _stream_ptr(self._torch, self.device), path.encode(), a.ctypes.data))
+        return a
+
+    def softmax_xent(self, logits, labels, *, label_smoothing: float = 0.0, dscale: float = 1.0, loss=None, dlogits=None):
+        """Mean softmax cross-entropy of ``logits`` (float32 CUDA [B, C]) against int32 CUDA ``labels`` [B] with
+        smoothed one-hot targets, and ``dscale`` times its gradient: ``(loss 0-d tensor, dlogits [B, C])``."""
+        torch = self._torch
+
+        def ok(t, dtype, shape):
+            return (isinstance(t, torch.Tensor) and t.dtype == dtype and t.is_cuda and t.is_contiguous()
+                    and tuple(t.shape) == shape and t.device == logits.device)
+        if not (isinstance(logits, torch.Tensor) and logits.dim() == 2):
+            raise ValueError("softmax_xent expects logits as a 2-D float32 CUDA tensor [B, C]")
+        b, c = int(logits.shape[0]), int(logits.shape[1])
+        if not ok(logits, torch.float32, (b, c)):
+            raise ValueError(f"softmax_xent expects logits as a contiguous float32 CUDA tensor [B, C], got "
+                             f"{logits.dtype} {tuple(logits.shape)} on {logits.device}")
+        if not ok(labels, torch.int32, (b,)):
+            raise ValueError(f"softmax_xent expects labels as a contiguous int32 tensor [{b}] on {logits.device}")
+        if loss is None:
+            loss = torch.empty((), dtype=torch.float32, device=logits.device)
+        if dlogits is None:
+            dlogits = torch.empty((b, c), dtype=torch.float32, device=logits.device)
+        if not ok(loss, torch.float32, ()) or not ok(dlogits, torch.float32, (b, c)):
+            raise ValueError(f"softmax_xent: loss must be a 0-d and dlogits a contiguous [{b}, {c}] float32 tensor on "
+                             f"{logits.device}")
+        _lib.check(self.lib.vitb200_softmax_xent(_stream_ptr(torch, logits.device), logits.data_ptr(), labels.data_ptr(),
+                                                 b, c, float(label_smoothing), float(dscale), loss.data_ptr(), dlogits.data_ptr()))
+        return loss, dlogits
+
     def forward_host(self, images: np.ndarray, out: Optional[np.ndarray] = None) -> np.ndarray:
         """End-to-end path: host fp32 images in, host fp32 logits out (H2D + D2H inside)."""
         images = np.ascontiguousarray(images, dtype=np.float32)
@@ -288,6 +366,13 @@ class Engine:
             self.close()
         except Exception:
             pass
+
+
+def _device_view(torch, device, ptr: int, n: int, typestr: str):
+    """A CUDA tensor viewing ``n`` elements of library-owned memory (no copy, no ownership)."""
+    class _Buf:
+        __cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (int(ptr), False), "version": 2}
+    return torch.as_tensor(_Buf(), device=device)
 
 
 def launch_count() -> int:

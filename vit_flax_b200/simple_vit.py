@@ -233,6 +233,13 @@ class SimpleViT:
 
         return (logits if is_cuda else logits.cpu().numpy()), vjp_fn
 
+    def trainer(self, variables: Any, tx, *, precision: Optional[str] = None, device: Optional[int] = None,
+                max_batch: Optional[int] = None):
+        """``ViT.trainer`` for SimpleViT.  The fixed sin/cos table and the zero biases SimpleViT does not have are
+        frozen; ``params()`` comes back in the layout ``variables`` came in."""
+        from .train import Trainer
+        return Trainer(self, variables, tx, precision=precision, device=device, max_batch=max_batch)
+
     # ------------------------------------------------------------------- apply
     def apply(self, variables: Any, img: Any, rngs: Any = None, *, precision: Optional[str] = None,
               device: Optional[int] = None, max_batch: Optional[int] = None, reload: bool = False):

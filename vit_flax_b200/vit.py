@@ -184,6 +184,14 @@ class ViT:
 
         return (logits if is_torch_cuda else logits.cpu().numpy()), vjp_fn
 
+    def trainer(self, variables: Any, tx, *, precision: Optional[str] = None, device: Optional[int] = None,
+                max_batch: Optional[int] = None):
+        """A ``Trainer`` (vit_flax_b200/train.py) that fine-tunes ``variables`` with ``tx`` (``vit_flax_b200.adamw``)
+        entirely on the device (ours: nothing in the reference trains).  ``max_batch``: the largest batch ``step``
+        will see (default 256).  The trainer owns its weights: ``apply(variables, x)`` still runs ``variables``."""
+        from .train import Trainer
+        return Trainer(self, variables, tx, precision=precision, device=device, max_batch=max_batch)
+
     def apply_stream(self, variables: Any, batches, *, precision: Optional[str] = None,
                      device: Optional[int] = None, max_batch: int = 256):
         """Serving-style extension of ``apply`` (ours, not in the reference): iterate host batches
