@@ -44,11 +44,16 @@ extern "C" {
 #define VITB200_PREC_FP32 1   /* fp32 everywhere (SIMT validation mode, tolerance 1e-4)        */
 #define VITB200_PREC_FP16 2   /* fp16 operands, otherwise identical to BF16 (same tcgen05
                                  kind::f16 rate; 3 more mantissa bits, see DESIGN.md)          */
+#define VITB200_PREC_FP8  3   /* inference only: E4M3 operands (tcgen05 kind::f8f6f4) on to_qkv and both
+                                 FeedForward Denses -- LayerNorm / GELU outputs unscaled, weights with one
+                                 fp32 scale per output column; everything else as FP16.  Dropout > 0 and
+                                 every training entry point return VITB200_ERR_UNSUPPORTED (DESIGN.md) */
 
 /* element types of buffers handed to the per-kernel entry points */
 #define VITB200_DT_F32  0
 #define VITB200_DT_BF16 1
 #define VITB200_DT_F16  2
+#define VITB200_DT_E4M3 3   /* one byte per element, OCP FP8 E4M3 (max 448, no infinities) */
 
 /* cfg.flags: the variations simple_vit.py needs on the same path (SURVEY.md section 8f-3) */
 #define VITB200_FLAG_NCHW   1   /* images are [B, C, H, W] (simple_vit.py:125), not [B, H, W, C]     */
@@ -248,6 +253,7 @@ int vitb200_softmax_xent(void* stream, const float* logits, const int32_t* label
 #define VITB200_EPI_TOKENS_LN       9  /* EPI_TOKENS_F32 + the same x16 / stats outputs (patch embedding, vit.py:147-153) */
 #define VITB200_EPI_LN_STORE_16     10 /* C_16 = rstd*acc - rstd*mean*c + d        (to_qkv after PreNorm, vit.py:31,68)    */
 #define VITB200_EPI_LN_GELU_16      11 /* C_16 = gelu_tanh(rstd*acc - rstd*mean*c + d)  (FeedForward Dense_0, vit.py:48-49) */
+#define VITB200_EPI_BIAS_GELU_E4M3  12 /* C_e4m3 = satfinite(e4m3(gelu_tanh(acc*wscale + bias)))  (fp8 FeedForward Dense_0)  */
 
 /* tcgen05 GEMM: acc[M,N] = A[M,K] (16-bit row-major) x Wt[N,K]^T (16-bit row-major, i.e. the
  * transposed Flax kernel), fp32 accumulation in TMEM.  dtype = VITB200_DT_BF16 | _F16.
@@ -294,13 +300,24 @@ int vitb200_gemm_tc_ln_slots(int M, int N);
  * Wt 16-bit [N,Kpad] = (diag(gamma) W)^T, c [N] = column sums of the ROUNDED W', d [N] = beta^T W + bias            */
 int vitb200_fold_layernorm(void* stream, const float* W, const float* gamma, const float* beta, const float* bias,
                            void* Wt, float* c, float* d, int K, int N, int Kpad, int dtype);
+/* fp8 tcgen05 GEMM (kind::f8f6f4): acc[M,N] = A[M,K] x Wt[N,K]^T with A and Wt E4M3 codes (row-major, K % 16 == 0 so
+ * that a row is a legal 16-byte TMA pitch), fp32 accumulation; every epilogue first multiplies acc by wscale[n] (the
+ * per-column weight scale of vitb200_quantize_weight_e4m3).  epilogue: STORE_16 (C fp16 = acc*wscale), BIAS_GELU_E4M3
+ * (C E4M3, N % 16 == 0), BIAS_RESID_F32 (C fp32 += acc*wscale + bias) or BIAS_F32 (C fp32 = acc*wscale + bias).      */
+int vitb200_gemm_tc_e4m3(void* stream, const void* A, const void* Wt, const float* wscale, const float* bias,
+                         void* C, int M, int N, int K, int epilogue);
+/* W fp32 [K,N] (Flax kernel) -> Wt E4M3 [N,Kpad] (K-major, zero for k >= K; Kpad % 16 == 0) and scale [N] fp32:
+ * scale[n] = max_k |W[k,n]| / 448 (1 for an all-zero column), Wt[n,k] = satfinite(e4m3(W[k,n] / scale[n])), rounded
+ * to nearest even.                                                                                                   */
+int vitb200_quantize_weight_e4m3(void* stream, const float* W, void* Wt, float* scale, int K, int N, int Kpad);
 /* SIMT fp32 GEMM (validation mode): acc = A[M,K] x W[K,N] (Flax layout).
  * The two "_16" epilogues write fp32 here.                                  */
 int vitb200_gemm_f32(void* stream, const float* A, const float* W, const float* bias,
                      float* C, int M, int N, int K, int epilogue,
                      const float* aux, int tokens_per_image);
 
-/* nn.LayerNorm() (vit.py:31,163): x [rows, dim] fp32 -> y of type out_dtype (VITB200_DT_*) */
+/* nn.LayerNorm() (vit.py:31,163): x [rows, dim] fp32 -> y of type out_dtype (VITB200_DT_*; E4M3 = satfinite(e4m3(.)),
+ * round to nearest even, the A operand of the fp8 GEMMs) */
 int vitb200_layernorm(void* stream, const float* x, const float* scale, const float* bias,
                       void* y, int rows, int dim, int out_dtype);
 

@@ -14,14 +14,15 @@ LIB_PATH = Path(__file__).resolve().parent / "libvitb200.so"
 ABI_VERSION = 4
 FLAG_NCHW, FLAG_NO_CLS = 1, 2
 OK = 0
-PREC_BF16, PREC_FP32, PREC_FP16 = 0, 1, 2
-DT_F32, DT_BF16, DT_F16 = 0, 1, 2
-PRECISIONS = {"bf16": PREC_BF16, "fp32": PREC_FP32, "fp16": PREC_FP16}
+PREC_BF16, PREC_FP32, PREC_FP16, PREC_FP8 = 0, 1, 2, 3
+DT_F32, DT_BF16, DT_F16, DT_E4M3 = 0, 1, 2, 3
+PRECISIONS = {"bf16": PREC_BF16, "fp32": PREC_FP32, "fp16": PREC_FP16, "fp8": PREC_FP8}
 POOL_CLS, POOL_MEAN = 0, 1
 CATEGORIES = ["patchify", "gemm_patch", "cls_rows", "layernorm", "gemm_qkv", "attention", "gemm_out",
               "gemm_ff1", "gemm_ff2", "pool_ln", "gemm_head"]
 EPI_STORE_16, EPI_BIAS_GELU_16, EPI_BIAS_RESID_F32, EPI_BIAS_F32, EPI_PATCH_F32, EPI_TOKENS_F32, EPI_BIAS_16, EPI_BIAS_PRE_GELU_16 = range(8)
 EPI_RESID_LN, EPI_TOKENS_LN, EPI_LN_STORE_16, EPI_LN_GELU_16 = range(8, 12)
+EPI_BIAS_GELU_E4M3 = 12
 GRAD_PARAMS, GRAD_IMAGES = 1, 2
 LEAF_TRAINABLE, LEAF_DECAY = 1, 2
 
@@ -95,6 +96,8 @@ SIGNATURES = {
     "vitb200_gemm_tc_ln_slots": (_i, [_i, _i]),
     "vitb200_patch_embed_im2col": (_i, [_vp, _fp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _fp]),
     "vitb200_fold_layernorm": (_i, [_vp, _fp, _fp, _fp, _fp, _vp, _fp, _fp, _i, _i, _i, _i]),
+    "vitb200_gemm_tc_e4m3": (_i, [_vp, _vp, _vp, _fp, _fp, _vp, _i, _i, _i, _i]),
+    "vitb200_quantize_weight_e4m3": (_i, [_vp, _fp, _vp, _fp, _i, _i, _i]),
     "vitb200_gemm_f32": (_i, [_vp, _fp, _fp, _fp, _fp, _i, _i, _i, _i, _fp, _i]),
     "vitb200_layernorm": (_i, [_vp, _fp, _fp, _fp, _vp, _i, _i, _i]),
     "vitb200_attention_tc": (_i, [_vp, _vp, _vp, _i, _i, _i, _i]),

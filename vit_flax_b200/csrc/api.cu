@@ -36,6 +36,8 @@ struct DenseW {
   int K = 0, N = 0, Kpad = 0;
   uint16_t* wt = nullptr;                 // bf16/fp16 [N, Kpad] (tensor-core modes)
   uint16_t* wf = nullptr;                 // bf16/fp16 [K, N], the Flax layout: the "W^T" operand of dX = dY W^T (backward only)
+  uint8_t* w8 = nullptr;                  // fp8 precision (to_qkv, FeedForward): E4M3 [N, Kpad] instead of wt; tm* map it
+  float* wscale = nullptr;                // and its per-column scales [N]
   CUtensorMap tm{};                       // box 256 x 64 over wt (one CTA per tile)
   CUtensorMap tm2{};                      // box 128 x 64 over wt (CTA pair per tile)
   CUtensorMap tm4{};                      // box 64 x 64 over wt (cluster of two pairs, multicast)
@@ -85,6 +87,7 @@ struct DevBuf {
 struct ActMaps {   // TMA descriptors over the activation workspace for one batch size
   CUtensorMap patches, xn, o, h, pooled;   // A operands
   CUtensorMap c_qkv, c_hid, c_x;           // GEMM outputs (TMA store / reduce-add)
+  CUtensorMap xn8, h8, c_hid8;             // fp8: the E4M3 views of xn_h / hid_h (A operands, FF Dense_0 output)
 };
 
 }  // namespace
@@ -105,6 +108,7 @@ struct vitb200_model {
   bool finalized = false;
   bool head_tc = false;
   bool fold = false;          // LayerNorm folded into the GEMMs around it (inference forward, dropout rates 0)
+  bool fp8 = false;           // VITB200_PREC_FP8: E4M3 to_qkv / FeedForward GEMMs on the LayerNorm-kernel schedule (dt = fp16)
   bool im2col = false;        // patch embedding as one im2col-TMA + tcgen05 kernel (patch_tc.cu), else patchify + TOKENS GEMM
   uint16_t* patch_wt_i2c = nullptr;   // Wt' [dim, ph*64] for that kernel
   CUtensorMap patch_tm_i2c{};
@@ -205,6 +209,10 @@ struct vitb200_model {
     auto free_dense = [](DenseW& d) {
       if (d.wt) cudaFree(d.wt);
       if (d.wf) cudaFree(d.wf);
+      if (d.w8) cudaFree(d.w8);
+      if (d.wscale) cudaFree(d.wscale);
+      d.w8 = nullptr;
+      d.wscale = nullptr;
       if (d.wt_ln) cudaFree(d.wt_ln);
       if (d.ln_c) cudaFree(d.ln_c);
       if (d.ln_d) cudaFree(d.ln_d);
@@ -333,6 +341,11 @@ int get_act_maps(vitb200_model* m, int batch, const ActMaps** out) {
     if ((rc = make_tmap_2d(&am.c_qkv, m->qkv_h.p, R, 3 * m->inner, 3 * m->inner, GEMM_BM, dt))) return rc;
     if ((rc = make_tmap_2d(&am.c_hid, m->hid_h.p, R, c.mlp_dim, c.mlp_dim, GEMM_BM, dt))) return rc;
     if ((rc = make_tmap_2d(&am.c_x, m->x.p, R, c.dim, c.dim, GEMM_BM, VITB200_DT_F32))) return rc;
+    if (m->fp8) {   // E4M3 codes in the first half of the 16-bit buffers' bytes: the workspace does not grow
+      if ((rc = make_tmap_2d(&am.xn8, m->xn_h.p, R, c.dim, c.dim, GEMM_BM, VITB200_DT_E4M3))) return rc;
+      if ((rc = make_tmap_2d(&am.h8, m->hid_h.p, R, c.mlp_dim, c.mlp_dim, GEMM_BM, VITB200_DT_E4M3))) return rc;
+      if ((rc = make_tmap_2d(&am.c_hid8, m->hid_h.p, R, c.mlp_dim, c.mlp_dim, GEMM_BM, VITB200_DT_E4M3, 64))) return rc;
+    }
     it = m->act_maps.emplace(batch, am).first;
   }
   *out = &it->second;
@@ -357,6 +370,19 @@ int pack_dense(vitb200_model* m, DenseW& d, cudaStream_t st) {
   if ((rc = make_tmap_2d(&d.tm, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN, m->dt))) return rc;
   if ((rc = make_tmap_2d(&d.tm2, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN / 2, m->dt))) return rc;
   return make_tmap_2d(&d.tm4, d.wt, d.N, d.Kpad, d.Kpad, GEMM_BN / 4, m->dt);
+}
+
+// fp8: the Dense as E4M3 codes [N, Kpad] + per-column scales; the tensor maps tm / tm2 / tm4 point at the codes
+int quant_dense(vitb200_model* m, DenseW& d, cudaStream_t st) {
+  if (d.w8 == nullptr) {
+    VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.w8), size_t(d.N) * d.Kpad));
+    VB_CUDA(cudaMalloc(reinterpret_cast<void**>(&d.wscale), size_t(d.N) * sizeof(float)));
+  }
+  int rc = launch_quantize_weight_e4m3(st, m->leaves[d.leaf_kernel].dev, d.w8, d.wscale, d.K, d.N, d.Kpad);
+  if (rc) return rc;
+  if ((rc = make_tmap_2d(&d.tm, d.w8, d.N, d.Kpad, d.Kpad, GEMM_BN, VITB200_DT_E4M3))) return rc;
+  if ((rc = make_tmap_2d(&d.tm2, d.w8, d.N, d.Kpad, d.Kpad, GEMM_BN / 2, VITB200_DT_E4M3))) return rc;
+  return make_tmap_2d(&d.tm4, d.w8, d.N, d.Kpad, d.Kpad, GEMM_BN / 4, VITB200_DT_E4M3);
 }
 
 inline const float* leaf_ptr(const vitb200_model* m, int idx) { return idx >= 0 ? m->leaves[idx].dev : nullptr; }
@@ -494,6 +520,7 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
   // tile mode per GEMM shape (pairs for anything that fills the machine, small tiles otherwise)
   const int cgp = gemm_tc_tile_mode(R, D);
   const int cg_qkv = gemm_tc_tile_mode(R, 3 * I), cg_d = gemm_tc_tile_mode(R, D), cg_ff1 = gemm_tc_tile_mode(R, c.mlp_dim);
+  const int ln_dt = m->fp8 ? VITB200_DT_E4M3 : m->dt;   // the LayerNorm output is the A operand of to_qkv / FF Dense_0
   if (m->im2col && (reinterpret_cast<uintptr_t>(images) & 15) == 0) {
     mark(m, st, VITB200_CAT_GEMM_PATCH);
     if ((rc = patch_embed_im2col(m, st, images, batch, nullptr))) return rc;
@@ -513,9 +540,12 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
     Layer& L = m->layers[l];
     // Residual(PreNorm(Attention))  vit.py:31,39,62-87
     mark(m, st, VITB200_CAT_LAYERNORM);
-    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln1_scale), leaf_ptr(m, L.ln1_bias), m->xn_h.p, R, D, m->dt, m->eps))) return rc;
+    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln1_scale), leaf_ptr(m, L.ln1_bias), m->xn_h.p, R, D, ln_dt, m->eps))) return rc;
     mark(m, st, VITB200_CAT_GEMM_QKV);
-    if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map(cg_qkv), &am->c_qkv, nullptr, m->qkv_h.p, R, 3 * I, D, VITB200_EPI_STORE_16, nullptr, 0, m->dt, cg_qkv))) return rc;
+    if (m->fp8) {
+      if ((rc = launch_gemm_tc(st, am->xn8, L.qkv.map(cg_qkv), &am->c_qkv, nullptr, m->qkv_h.p, R, 3 * I, D, VITB200_EPI_STORE_16,
+                               nullptr, 0, VITB200_DT_E4M3, cg_qkv, Dropout(), m->cls_off, nullptr, LnFold(), L.qkv.wscale))) return rc;
+    } else if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map(cg_qkv), &am->c_qkv, nullptr, m->qkv_h.p, R, 3 * I, D, VITB200_EPI_STORE_16, nullptr, 0, m->dt, cg_qkv))) return rc;
     mark(m, st, VITB200_CAT_ATTENTION);
     if ((rc = launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, c.heads, m->dt))) return rc;
     mark(m, st, VITB200_CAT_GEMM_OUT);
@@ -528,7 +558,18 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
     }
     // Residual(PreNorm(FeedForward))  vit.py:31,39,47-53
     mark(m, st, VITB200_CAT_LAYERNORM);
-    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln2_scale), leaf_ptr(m, L.ln2_bias), m->xn_h.p, R, D, m->dt, m->eps))) return rc;
+    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln2_scale), leaf_ptr(m, L.ln2_bias), m->xn_h.p, R, D, ln_dt, m->eps))) return rc;
+    if (m->fp8) {   // E4M3 in, E4M3 hidden activations, E4M3 in again: FF Dense_0 -> GELU -> FF Dense_1
+      mark(m, st, VITB200_CAT_GEMM_FF1);
+      if ((rc = launch_gemm_tc(st, am->xn8, L.ff1.map(cg_ff1), &am->c_hid8, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, R, c.mlp_dim, D,
+                               VITB200_EPI_BIAS_GELU_E4M3, nullptr, 0, VITB200_DT_E4M3, cg_ff1, Dropout(), m->cls_off, nullptr,
+                               LnFold(), L.ff1.wscale))) return rc;
+      mark(m, st, VITB200_CAT_GEMM_FF2);
+      if ((rc = launch_gemm_tc(st, am->h8, L.ff2.map(cg_d), &am->c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, R, D, c.mlp_dim,
+                               VITB200_EPI_BIAS_RESID_F32, nullptr, 0, VITB200_DT_E4M3, cg_d, Dropout(), m->cls_off, nullptr,
+                               LnFold(), L.ff2.wscale))) return rc;
+      continue;
+    }
     mark(m, st, VITB200_CAT_GEMM_FF1);
     if ((rc = launch_gemm_tc(st, am->xn, L.ff1.map(cg_ff1), &am->c_hid, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, R, c.mlp_dim, D, VITB200_EPI_BIAS_GELU_16, nullptr, 0, m->dt, cg_ff1, m->drop(c.dropout, 2 + 3 * l)))) return rc;
     mark(m, st, VITB200_CAT_GEMM_FF2);
@@ -646,10 +687,16 @@ int vitb200_create(const vitb200_config* cfg, int device, vitb200_model** out) {
     return fail(VITB200_ERR_INVALID, "create: image dimensions must be divisible by the patch size");
   if (c.pool != VITB200_POOL_CLS && c.pool != VITB200_POOL_MEAN)     // vit.py:137
     return fail(VITB200_ERR_INVALID, "create: pool must be cls or mean");
-  if (c.precision != VITB200_PREC_BF16 && c.precision != VITB200_PREC_FP32 && c.precision != VITB200_PREC_FP16)
+  if (c.precision != VITB200_PREC_BF16 && c.precision != VITB200_PREC_FP32 && c.precision != VITB200_PREC_FP16 &&
+      c.precision != VITB200_PREC_FP8)
     return fail(VITB200_ERR_INVALID, "create: unknown precision");
   if (!(c.dropout >= 0.f && c.dropout < 1.f) || !(c.emb_dropout >= 0.f && c.emb_dropout < 1.f))
     return fail(VITB200_ERR_INVALID, "create: dropout rates must be in [0, 1)");
+  if (c.precision == VITB200_PREC_FP8 && (c.dropout > 0.f || c.emb_dropout > 0.f))
+    return fail(VITB200_ERR_UNSUPPORTED, "create: the fp8 precision is an inference forward: dropout rates must be 0");
+  if (c.precision == VITB200_PREC_FP8 && (c.dim % 16 != 0 || c.mlp_dim % 16 != 0))
+    return fail(VITB200_ERR_UNSUPPORTED, "create: the fp8 precision needs dim and mlp_dim to be multiples of 16 (E4M3 rows "
+                                         "of a 16-byte pitch)");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
     cudaGetLastError();
@@ -672,7 +719,8 @@ int vitb200_create(const vitb200_config* cfg, int device, vitb200_model** out) {
   m->T = m->Np + m->cls_off;
   m->K0 = c.patch_h * c.patch_w * c.channels;
   m->tc = c.precision != VITB200_PREC_FP32;
-  m->dt = c.precision == VITB200_PREC_FP16 ? VITB200_DT_F16 : VITB200_DT_BF16;
+  m->fp8 = c.precision == VITB200_PREC_FP8;
+  m->dt = (c.precision == VITB200_PREC_FP16 || m->fp8) ? VITB200_DT_F16 : VITB200_DT_BF16;
   m->K0pad = m->tc ? int(round_up(m->K0, GEMM_BK)) : m->K0 + (m->K0 & 1);
   m->inner = DIM_HEAD * c.heads;
   m->project_out = !(c.heads == 1 && DIM_HEAD == c.dim);             // vit.py:65
@@ -687,7 +735,8 @@ int vitb200_create(const vitb200_config* cfg, int device, vitb200_model** out) {
   }
   {  // LayerNorm fold: on by default for the dropout-free inference forward; VITB200_LN_FOLD=0 keeps the LayerNorm kernel (A/B)
     const char* e = getenv("VITB200_LN_FOLD");
-    m->fold = m->tc && m->project_out && c.depth > 0 && c.dropout == 0.f && c.emb_dropout == 0.f && !(e && e[0] == '0');
+    // fp8 keeps the LayerNorm kernel: it holds a whole row and emits the bounded, normalised values E4M3 can carry
+    m->fold = m->tc && !m->fp8 && m->project_out && c.depth > 0 && c.dropout == 0.f && c.emb_dropout == 0.f && !(e && e[0] == '0');
   }
   if (m->tc && (c.dim % 8 != 0 || c.mlp_dim % 8 != 0))
     return fail(VITB200_ERR_UNSUPPORTED, "create: bf16/fp16 modes need dim and mlp_dim to be multiples of 8");
@@ -752,6 +801,11 @@ int vitb200_finalize_params(vitb200_model* m, void* stream) {
     int rc;
     if ((rc = pack_dense(m, m->patch, st))) return rc;
     for (auto& L : m->layers) {
+      if (m->fp8) {   // E4M3 codes + column scales for to_qkv and the FeedForward; no 16-bit packs of those three
+        if ((rc = quant_dense(m, L.qkv, st)) || (rc = quant_dense(m, L.ff1, st)) || (rc = quant_dense(m, L.ff2, st))) return rc;
+        if ((rc = pack_dense(m, L.out, st))) return rc;
+        continue;
+      }
       if ((rc = pack_dense(m, L.qkv, st))) return rc;
       if ((rc = pack_dense(m, L.out, st))) return rc;
       if ((rc = pack_dense(m, L.ff1, st))) return rc;
@@ -1030,6 +1084,7 @@ int wgrad(vitb200_model* m, cudaStream_t st, const void* X, int Dx, const void* 
 int train_supported(const vitb200_model* m) {
   const auto& c = m->cfg;
   if (!m->tc) return fail(VITB200_ERR_UNSUPPORTED, "train: the backward pass is built for the bf16/fp16 modes only");
+  if (m->fp8) return fail(VITB200_ERR_UNSUPPORTED, "train: the fp8 precision is inference only (train in fp16 or bf16)");
   if (!m->project_out) return fail(VITB200_ERR_UNSUPPORTED, "train: heads == 1 with dim == 64 (identity to_out) is not built");
   if (c.dim > 1280) return fail(VITB200_ERR_UNSUPPORTED, "train: dim > 1280 is not built for the backward pass");
   if (c.depth < 1) return fail(VITB200_ERR_UNSUPPORTED, "train: the backward pass needs at least one transformer layer");
@@ -1245,6 +1300,7 @@ int grads_ready(const vitb200_model* m, const char* who) {
 
 int vitb200_backward_ex(vitb200_model* m, void* stream, const float* dlogits, int batch, int wrt, float* dimages) {
   if (!m || !dlogits) return fail(VITB200_ERR_INVALID, "backward: null argument");
+  if (m->fp8) return fail(VITB200_ERR_UNSUPPORTED, "backward: the fp8 precision is inference only (train in fp16 or bf16)");
   if (wrt == 0 || (wrt & ~(VITB200_GRAD_PARAMS | VITB200_GRAD_IMAGES)) != 0)
     return fail(VITB200_ERR_INVALID, "backward: wrt must be a non-zero OR of VITB200_GRAD_PARAMS and VITB200_GRAD_IMAGES");
   if ((wrt & VITB200_GRAD_IMAGES) && !dimages)
@@ -1593,6 +1649,35 @@ int vitb200_fold_layernorm(void* stream, const float* W, const float* gamma, con
   const int rc = launch_fold_layernorm(st, W, gamma, beta, bias, Wt, c, d, K, N, Kpad, dtype, scratch);
   cudaFreeAsync(scratch, st);
   return rc;
+}
+
+int vitb200_gemm_tc_e4m3(void* stream, const void* A, const void* Wt, const float* wscale, const float* bias, void* C, int M,
+                         int N, int K, int epilogue) {
+  if (!A || !Wt || !wscale || !C) return fail(VITB200_ERR_INVALID, "gemm_tc_e4m3: null pointer");
+  if (M <= 0 || N <= 0 || K <= 0 || (N % 8) != 0 || (K % 16) != 0)
+    return fail(VITB200_ERR_INVALID, "gemm_tc_e4m3: M, N, K must be positive, N a multiple of 8 and K of 16");
+  int out_dt;
+  switch (epilogue) {
+    case VITB200_EPI_STORE_16: out_dt = VITB200_DT_F16; break;
+    case VITB200_EPI_BIAS_GELU_E4M3: out_dt = VITB200_DT_E4M3; break;
+    case VITB200_EPI_BIAS_RESID_F32: case VITB200_EPI_BIAS_F32: out_dt = VITB200_DT_F32; break;
+    default:
+      return fail(VITB200_ERR_UNSUPPORTED, "gemm_tc_e4m3: epilogue must be STORE_16, BIAS_GELU_E4M3, BIAS_RESID_F32 or BIAS_F32");
+  }
+  if (out_dt == VITB200_DT_E4M3 && (N % 16) != 0) return fail(VITB200_ERR_INVALID, "gemm_tc_e4m3: BIAS_GELU_E4M3 needs N % 16 == 0");
+  const int cg = gemm_tc_tile_mode(M, N);
+  CUtensorMap ta, tb, tc;
+  int rc;
+  if ((rc = make_tmap_2d(&ta, A, M, K, K, GEMM_BM, VITB200_DT_E4M3))) return rc;
+  if ((rc = make_tmap_2d(&tb, Wt, N, K, K, cg == 64 ? 64 : GEMM_BN / cg, VITB200_DT_E4M3))) return rc;
+  if ((rc = make_tmap_2d(&tc, C, M, N, N, GEMM_BM, out_dt, out_dt == VITB200_DT_E4M3 ? 64 : 128))) return rc;
+  return launch_gemm_tc(static_cast<cudaStream_t>(stream), ta, tb, &tc, bias, C, M, N, K, epilogue, nullptr, 0,
+                        VITB200_DT_E4M3, cg, Dropout(), 1, nullptr, LnFold(), wscale);
+}
+
+int vitb200_quantize_weight_e4m3(void* stream, const float* W, void* Wt, float* scale, int K, int N, int Kpad) {
+  if (!W || !Wt || !scale) return fail(VITB200_ERR_INVALID, "quantize_weight_e4m3: null pointer");
+  return launch_quantize_weight_e4m3(static_cast<cudaStream_t>(stream), W, static_cast<uint8_t*>(Wt), scale, K, N, Kpad);
 }
 
 int vitb200_gemm_f32(void* stream, const float* A, const float* W, const float* bias, float* C, int M, int N,

@@ -84,9 +84,10 @@ inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block
 
 // ---- TMA descriptors -----------------------------------------------------
 // 2-D row-major tensor [rows, cols] (cols contiguous, row pitch = ld elements) of element type
-// `dt` (VITB200_DT_*); box = [box_rows, 128 bytes of columns] with 128-byte swizzle.
+// `dt` (VITB200_DT_*, E4M3 = one byte); box = [box_rows, box_bytes of columns]: 128 bytes with the 128-byte swizzle, or
+// 64 bytes with the 64-byte swizzle (dense 64-byte rows in shared memory, 16-byte chunk bits [4,6) ^= address bits [7,9)).
 int make_tmap_2d(CUtensorMap* out, const void* base, int64_t rows, int64_t cols, int64_t ld,
-                 int box_rows, int dt);
+                 int box_rows, int dt, int box_bytes = 128);
 // 3-D [batch, rows, cols] 16-bit tensor, box = [1, box_rows, 64 cols].
 int make_tmap_3d_16(CUtensorMap* out, const void* base, int64_t batch, int64_t rows, int64_t cols,
                     int64_t ld, int box_rows, int dt);
@@ -106,7 +107,11 @@ int launch_gemm_tc(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMa
                    const CUtensorMap* tmC, const float* bias, void* C, int M, int N, int K,
                    int epilogue, const float* aux, int tokens_per_image, int dtype, int cta_group,
                    const Dropout& drop = Dropout(), int cls_off = 1, const float* cls = nullptr,
-                   const LnFold& ln = LnFold());
+                   const LnFold& ln = LnFold(), const float* wscale = nullptr);
+// dtype VITB200_DT_E4M3 (the fp8 precision): A [M, K] and Wt [N, K] are E4M3 codes (K-major, k-blocks of 128 elements,
+// K % 16 == 0), the accumulator is multiplied by the per-column weight scale `wscale` [N] before the epilogue's own math.
+// Epilogues STORE_16 (fp16 out), BIAS_RESID_F32, BIAS_F32 and BIAS_GELU_E4M3 (E4M3 out through a 64-byte-wide map);
+// no dropout, no split-K, tile modes 1, 2 and 64.
 // LayerNorm fold (gemm_tc.cu header): W' = diag(gamma) W packed to 16-bit [N, Kpad], c[n] = sum_k W'_16[n, k] (of the
 // ROUNDED values, so that rstd mean c cancels the mean part of x16 W'_16 exactly), d[n] = sum_k beta[k] W[k, n] (+ bias[n]).
 // `scratch`: K * N floats.
@@ -153,6 +158,9 @@ int launch_pool_layernorm(cudaStream_t stream, const float* x, const float* scal
                           int out_dtype, float eps = 1e-6f);
 int launch_pack_weight(cudaStream_t stream, const float* W, void* Wt, int K, int N, int Kpad,
                        int dtype);
+// W fp32 [K, N] (Flax kernel) -> Wt E4M3 [N, Kpad] = satfinite(e4m3(W[k, n] / scale[n])), zero for k >= K, and
+// scale[n] = max_k |W[k, n]| / 448 (1 for an all-zero column)
+int launch_quantize_weight_e4m3(cudaStream_t stream, const float* W, uint8_t* Wt, float* scale, int K, int N, int Kpad);
 // ---- fused patch embedding (patch_tc.cu): im2col TMA + tcgen05 GEMM + cls / pos placement (+ LayerNorm-fold outputs) ----
 bool patch_im2col_supported(int pw, int channels, int dim);
 // W fp32 [ph*pw*C, D] -> Wt' 16-bit [D, ph*64] (k-block p1 = image row p1 of the patch, padded to 64 columns)

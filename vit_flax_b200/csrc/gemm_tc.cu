@@ -1,5 +1,6 @@
-// gemm_tc.cu -- K3: persistent, warp-specialised tcgen05 GEMM (bf16 or fp16 operands) with
-// fused epilogues.  acc[M,N] = A[M,K] x Wt[N,K]^T, fp32 accumulation in TMEM.
+// gemm_tc.cu -- K3: persistent, warp-specialised tcgen05 GEMM (bf16 or fp16 operands; E4M3 for the fp8 precision's
+// to_qkv / FeedForward, kind::f8f6f4 on 128-element k-blocks) with fused epilogues.  acc[M,N] = A[M,K] x Wt[N,K]^T,
+// fp32 accumulation in TMEM.
 //
 // Replaces every flax `nn.Dense` on the hot path (vit.py:48,51,68,82,147,165) together with what
 // follows it in the reference: bias add, tanh-GELU (vit.py:49), the Residual add (vit.py:39),
@@ -115,7 +116,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                const __grid_constant__ CUtensorMap tmC,
                const float* __restrict__ bias, void* __restrict__ Cout,
                int M, int N, int K, const float* __restrict__ aux, int tpi, int dbg, Dropout drop, int cls_off,
-               const float* __restrict__ cls, LnFold ln) {
+               const float* __restrict__ cls, LnFold ln, const float* __restrict__ wscale) {
+  // fp8 precision: E4M3 operands, k-blocks of 128 elements (still 128 B per row: the stage layout, boxes, barriers and
+  // descriptors are those of the 16-bit form), the accumulator scaled per column by wscale; 16-bit outputs are fp16
+  constexpr bool kF8 = (kDT == DT_E4M3);
+  constexpr int kODT = kF8 ? DT_F16 : kDT;
+  constexpr int KB = kF8 ? 128 : BK;                          // elements per k-block
+  static_assert(!kF8 || (!kMN && !kDrop), "E4M3 operands: K-major, no dropout");
+  constexpr bool kOut8 = (kEpi == VITB200_EPI_BIAS_GELU_E4M3);   // E4M3 output, 64-byte slab rows (64 columns)
   constexpr bool kOut16 = (kEpi == VITB200_EPI_STORE_16 || kEpi == VITB200_EPI_BIAS_GELU_16 || kEpi == VITB200_EPI_BIAS_16 ||
                            kEpi == VITB200_EPI_BIAS_PRE_GELU_16 || kEpi == VITB200_EPI_LN_STORE_16 ||
                            kEpi == VITB200_EPI_LN_GELU_16);
@@ -126,7 +134,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
   constexpr int SPG = slabs_per_group<kEpi>();
   constexpr bool kDual = (kEpi == VITB200_EPI_BIAS_PRE_GELU_16);   // two outputs per slab: pre-activation and GELU
   constexpr bool kDirect = (kEpi == VITB200_EPI_PATCH_F32);   // row-remapped output: plain stores
-  constexpr int SLAB_COLS = kOut16 ? 64 : 32;                 // 128 B of output per row
+  constexpr int SLAB_COLS = (kOut16 || kOut8) ? 64 : 32;      // 128 B (E4M3: 64 B) of output per row
   constexpr int SLABS_PER_TILE = Cfg<kCG>::BN_ / SLAB_COLS;
   constexpr int STAGES = num_stages<kCG, kEpi>(), B_BYTES = Cfg<kCG>::B_BYTES;
   constexpr int STAGE_BYTES = Cfg<kCG>::STAGE_BYTES, TILE_M = Cfg<kCG>::TILE_M;
@@ -160,7 +168,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
   const int lane = threadIdx.x & 31;
   const int m_tiles = ((M + TILE_M - 1) / TILE_M + PAIRS - 1) / PAIRS;   // cluster steps along M
   const int n_tiles = (N + BN - 1) / BN;
-  const int num_kb = (K + BK - 1) / BK;
+  const int num_kb = (K + KB - 1) / KB;
   // split-K (BIAS_RESID_F32 only, `tpi` carries the factor): split sp of a tile accumulates k-blocks
   // [sp * kb_per, min(num_kb, (sp + 1) * kb_per)) and reduce-adds its partial sum; split 0 adds the bias
   const int splits = (kEpi == VITB200_EPI_BIAS_RESID_F32 && tpi > 1) ? tpi : 1;
@@ -219,8 +227,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
               for (int j = 0; j < Cfg<kCG>::B_ROWS / 64; ++j)
                 tma_load_2d(sB + stage * B_BYTES + j * 8192, &tmB, full_bar(stage), b_row + j * 64, kb * BK);
             } else {
-              tma_load_2d(sA + stage * A_BYTES, &tmA, full_bar(stage), kb * BK, a_row);
-              tma_load_2d(sB + stage * B_BYTES, &tmB, full_bar(stage), kb * BK, b_row);
+              tma_load_2d(sA + stage * A_BYTES, &tmA, full_bar(stage), kb * KB, a_row);
+              tma_load_2d(sB + stage * B_BYTES, &tmB, full_bar(stage), kb * KB, b_row);
             }
           } else {
             // Both CTAs' loads complete on the pair LEADER's full barrier (the MMA issuer waits there).
@@ -239,9 +247,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
               for (int j = 0; j < Cfg<kCG>::B_ROWS / 64; ++j)
                 tma_load_2d_cg2(sB + stage * B_BYTES + j * 8192, &tmB, lead_full, b_row + j * 64, kb * BK);
             } else {
-            tma_load_2d_cg2(sA + stage * A_BYTES, &tmA, lead_full, kb * BK, a_row);
+            tma_load_2d_cg2(sA + stage * A_BYTES, &tmA, lead_full, kb * KB, a_row);
             if constexpr (CL == 2) {
-              tma_load_2d_cg2(sB + stage * B_BYTES, &tmB, lead_full, kb * BK, b_row);
+              tma_load_2d_cg2(sB + stage * B_BYTES, &tmB, lead_full, kb * KB, b_row);
             } else {
               // 64 of this CTA's 128 weight rows, delivered to the same smem offset here and in the
               // CTA of equal rank in the other pair; each destination signals its own pair leader.
@@ -258,7 +266,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA only in pair mode) =====================
     if (rank == 0 && elect_one()) {
-      constexpr uint32_t idesc = umma_idesc_16(TILE_M, BN, kDT == DT_F16 ? 0 : 1, kMN ? 1 : 0, kMN ? 1 : 0);
+      constexpr uint32_t idesc = kF8 ? umma_idesc_e4m3(TILE_M, BN)
+                                     : umma_idesc_16(TILE_M, BN, kDT == DT_F16 ? 0 : 1, kMN ? 1 : 0, kMN ? 1 : 0);
       const uint16_t pair_mask = uint16_t(0x3u << lead);               // both CTAs of this pair
       const uint16_t all_mask = uint16_t((1u << CL) - 1u);             // every CTA whose smem the stage's loads touch
       int stage = 0;
@@ -276,8 +285,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
           tc_fence_after();
           const uint32_t a0 = sA + stage * A_BYTES, b0 = sB + stage * B_BYTES;
 #pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k) {
-            if constexpr (kMN)   // 16 K-rows of 128 B further per step
+          for (int k = 0; k < BK / UMMA_K; ++k) {   // E4M3: 4 x K = 32, the same 32-byte steps
+            if constexpr (kF8)
+              umma_f8_ss<MMA_CG>(d_tmem, umma_desc_k_sw128(a0 + k * UMMA_K * 2), umma_desc_k_sw128(b0 + k * UMMA_K * 2),
+                                 idesc, (kb != kb0 || k != 0) ? 1u : 0u);
+            else if constexpr (kMN)   // 16 K-rows of 128 B further per step
               umma_bf16_ss<MMA_CG>(d_tmem, umma_desc_mn_sw128_wide(a0 + k * UMMA_K * 128, 8192),
                                    umma_desc_mn_sw128_wide(b0 + k * UMMA_K * 128, 8192), idesc,
                                    (kb != kb0 || k != 0) ? 1u : 0u);
@@ -441,6 +453,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                 float v[8];
 #pragma unroll
                 for (int e = 0; e < 8; ++e) v[e] = __uint_as_float(r[j * 8 + e]);
+                if constexpr (kF8) {   // STORE_16 (to_qkv): acc * the weight's column scale
+                  const int nb = n0 + half * 32 + j * 8;
+                  if (nb < N) {
+                    const float4 w0 = __ldg(reinterpret_cast<const float4*>(wscale + nb));
+                    const float4 w1 = __ldg(reinterpret_cast<const float4*>(wscale + nb + 4));
+                    v[0] *= w0.x; v[1] *= w0.y; v[2] *= w0.z; v[3] *= w0.w;
+                    v[4] *= w1.x; v[5] *= w1.y; v[6] *= w1.z; v[7] *= w1.w;
+                  }
+                }
                 if constexpr (kEpi == VITB200_EPI_BIAS_16 || kDual) {   // pre-activation kept for the backward pass
                   const int nb = n0 + half * 32 + j * 8;
                   if (nb < N) {
@@ -509,8 +530,47 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                   }
                 }
                 const int chunk = half * 4 + j;
-                st_shared_v4(srow + (uint32_t(chunk ^ sw) << 4), pack2<kDT>(v[0], v[1]),
-                             pack2<kDT>(v[2], v[3]), pack2<kDT>(v[4], v[5]), pack2<kDT>(v[6], v[7]));
+                st_shared_v4(srow + (uint32_t(chunk ^ sw) << 4), pack2<kODT>(v[0], v[1]),
+                             pack2<kODT>(v[2], v[3]), pack2<kODT>(v[4], v[5]), pack2<kODT>(v[6], v[7]));
+              }
+            }
+          } else if constexpr (kOut8) {
+            // ---- BIAS_GELU_E4M3 (fp8 FeedForward Dense_0): e4m3(gelu(acc * wscale + bias)); the slab is 128 rows of 64 B
+            // (64 columns) through a TMA map with a 64-byte box and the 64-byte swizzle: 16-byte chunk bits [4,6) of the
+            // linear offset row * 64 + byte ^= its bits [7,9) ----
+#pragma unroll
+            for (int half = 0; half < 2; ++half) {
+              uint32_t r[32];
+              tmem_ld_32x32b_x32(t_row + uint32_t(s * SLAB_COLS + half * 32), r);
+              tmem_ld_wait();
+#pragma unroll
+              for (int j = 0; j < 2; ++j) {            // 16 columns -> one 16-byte chunk of codes
+                uint32_t q[4];
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {          // 8 columns at a time (register pressure)
+                  const int nb = n0 + half * 32 + j * 16 + h * 8;   // N % 16 == 0: a chunk is wholly in or out
+                  float4 w0 = make_float4(0.f, 0.f, 0.f, 0.f), w1 = w0, b0 = w0, b1 = w0;
+                  if (nb < N) {
+                    w0 = __ldg(reinterpret_cast<const float4*>(wscale + nb));
+                    w1 = __ldg(reinterpret_cast<const float4*>(wscale + nb + 4));
+                    b0 = __ldg(reinterpret_cast<const float4*>(bias + nb));
+                    b1 = __ldg(reinterpret_cast<const float4*>(bias + nb + 4));
+                  }
+                  const float ws[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
+                  const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+                  float v[8];
+#pragma unroll
+                  for (int e = 0; e < 8; e += 2) {
+                    const int c = j * 16 + h * 8 + e;
+                    const unsigned long long y2 = fma_f32x2(pack_f32x2(__uint_as_float(r[c]), __uint_as_float(r[c + 1])),
+                                                            pack_f32x2(ws[e], ws[e + 1]), pack_f32x2(bb[e], bb[e + 1]));
+                    unpack_f32x2(gelu_tanh_fast2(y2), v[e], v[e + 1]);
+                  }
+                  q[h * 2] = pack4_e4m3(v[0], v[1], v[2], v[3]);
+                  q[h * 2 + 1] = pack4_e4m3(v[4], v[5], v[6], v[7]);
+                }
+                const uint32_t lin = uint32_t(lrow) * 64u + uint32_t(half * 2 + j) * 16u;
+                st_shared_v4(slab + (lin ^ (((lin >> 7) & 3u) << 4)), q[0], q[1], q[2], q[3]);
               }
             }
           } else {
@@ -532,6 +592,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
               if (nb < N && sp == 0 && bias != nullptr) b4 = __ldg(reinterpret_cast<const float4*>((cls_row ? cls : bias) + nb));
               float o0 = __uint_as_float(r[j * 4 + 0]), o1 = __uint_as_float(r[j * 4 + 1]);
               float o2 = __uint_as_float(r[j * 4 + 2]), o3 = __uint_as_float(r[j * 4 + 3]);
+              if constexpr (kF8) {   // acc * the weight's column scale, then the bias below
+                if (nb < N) {
+                  const float4 w4 = __ldg(reinterpret_cast<const float4*>(wscale + nb));
+                  o0 *= w4.x; o1 *= w4.y; o2 *= w4.z; o3 *= w4.w;
+                }
+              }
               if constexpr (kTokens) {
                 if (cls_row) o0 = o1 = o2 = o3 = 0.f;   // the slot row of the patch matrix holds no data
                 if (nb < N) {
@@ -622,7 +688,8 @@ int gemm_dbg() {   // VITB200_GEMM_DBG bit 0: no TMA loads, bit 1: no output sto
 template <int kEpi, int kDT, int kCG, bool kDrop, bool kMN = false>
 int launch_cg(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tmB,
               const CUtensorMap& tmC, const float* bias, void* C, int M, int N, int K,
-              const float* aux, int tpi, const Dropout& drop, int cls_off, const float* cls, const LnFold& ln = LnFold()) {
+              const float* aux, int tpi, const Dropout& drop, int cls_off, const float* cls, const LnFold& ln = LnFold(),
+              const float* wscale = nullptr) {
   static PerDevice<bool> configured_on;   // the smem opt-in is per (function, device)
   static PerDevice<int> max_units_on;   // clusters (CTAs for kCG == 1) that can be resident at once, per device
   int& max_units = max_units_on.here();
@@ -654,7 +721,7 @@ int launch_cg(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tm
   const int tiles = ceil_div(ceil_div(M, Cfg<kCG>::TILE_M), Cfg<kCG>::PAIRS) * ceil_div(N, Cfg<kCG>::BN_) * splits;
   const int units = tiles < max_units ? tiles : max_units;
   VB_CUDA(launch_kernel(gemm_tc_kernel<kEpi, kDT, kCG, kDrop, kMN>, dim3(units * Cfg<kCG>::CL), dim3(NUM_THREADS), smem_bytes<kCG, kEpi>(),
-                        stream, Cfg<kCG>::CL, tmA, tmB, tmC, bias, C, M, N, K, aux, tpi, gemm_dbg(), drop, cls_off, cls, ln));
+                        stream, Cfg<kCG>::CL, tmA, tmB, tmC, bias, C, M, N, K, aux, tpi, gemm_dbg(), drop, cls_off, cls, ln, wscale));
   VB_LAUNCH_CHECK("gemm_tc_kernel");
   return 0;
 }
@@ -745,6 +812,41 @@ int dispatch_epi(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap&
   }
 }
 
+// the fp8 GEMMs (E4M3 operands): the four epilogues of the fp8 forward, tile modes 1, 2 and 64, no dropout, no split-K
+template <int kEpi>
+int launch_e4m3(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC,
+                const float* bias, void* C, int M, int N, int K, int cta_group, const float* wscale) {
+  if (cta_group == 64)
+    return launch_cg<kEpi, DT_E4M3, 64, false>(stream, tmA, tmB, tmC, bias, C, M, N, K, nullptr, 0, Dropout(), 1, nullptr, LnFold(), wscale);
+  if (cta_group == 1)
+    return launch_cg<kEpi, DT_E4M3, 1, false>(stream, tmA, tmB, tmC, bias, C, M, N, K, nullptr, 0, Dropout(), 1, nullptr, LnFold(), wscale);
+  if (cta_group == 2)
+    return launch_cg<kEpi, DT_E4M3, 2, false>(stream, tmA, tmB, tmC, bias, C, M, N, K, nullptr, 0, Dropout(), 1, nullptr, LnFold(), wscale);
+  return fail(VITB200_ERR_UNSUPPORTED, "gemm_tc: E4M3 operands are built for tile modes 1, 2 and 64");
+}
+
+int dispatch_e4m3(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC,
+                  const float* bias, void* C, int M, int N, int K, int epilogue, int cta_group, const Dropout& drop,
+                  const float* wscale) {
+  if (wscale == nullptr) return fail(VITB200_ERR_INVALID, "gemm_tc: E4M3 operands need the per-column weight scales");
+  if (drop.threshold != 0) return fail(VITB200_ERR_UNSUPPORTED, "gemm_tc: E4M3 operands have no dropout variant");
+  if ((K % 16) != 0) return fail(VITB200_ERR_INVALID, "gemm_tc: E4M3 operands need K % 16 == 0 (16-byte row pitch)");
+  switch (epilogue) {
+    case VITB200_EPI_STORE_16:
+      return launch_e4m3<VITB200_EPI_STORE_16>(stream, tmA, tmB, tmC, bias, C, M, N, K, cta_group, wscale);
+    case VITB200_EPI_BIAS_GELU_E4M3:
+      if ((N % 16) != 0) return fail(VITB200_ERR_INVALID, "gemm_tc: BIAS_GELU_E4M3 needs N % 16 == 0");
+      return launch_e4m3<VITB200_EPI_BIAS_GELU_E4M3>(stream, tmA, tmB, tmC, bias, C, M, N, K, cta_group, wscale);
+    case VITB200_EPI_BIAS_RESID_F32:
+      return launch_e4m3<VITB200_EPI_BIAS_RESID_F32>(stream, tmA, tmB, tmC, bias, C, M, N, K, cta_group, wscale);
+    case VITB200_EPI_BIAS_F32:
+      return launch_e4m3<VITB200_EPI_BIAS_F32>(stream, tmA, tmB, tmC, bias, C, M, N, K, cta_group, wscale);
+    default:
+      return fail(VITB200_ERR_UNSUPPORTED, "gemm_tc: E4M3 operands take the STORE_16, BIAS_GELU_E4M3, BIAS_RESID_F32 and "
+                                           "BIAS_F32 epilogues");
+  }
+}
+
 }  // namespace
 
 int gemm_tc_cta_group(int M) { return gemm_tc_tile_mode(M, 1 << 20); }
@@ -787,7 +889,7 @@ int launch_gemm_tc_wgrad(cudaStream_t stream, const CUtensorMap& tmX, const CUte
 int launch_gemm_tc(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMap& tmB,
                    const CUtensorMap* tmC, const float* bias, void* C, int M, int N, int K,
                    int epilogue, const float* aux, int tpi, int dtype, int cta_group, const Dropout& drop,
-                   int cls_off, const float* cls, const LnFold& ln) {
+                   int cls_off, const float* cls, const LnFold& ln, const float* wscale) {
   if (cta_group != 1 && cta_group != 2 && cta_group != 4 && cta_group != 64)
     return fail(VITB200_ERR_INVALID, "gemm_tc: tile mode must be 1, 2, 4 or 64");
   if (M <= 0 || N <= 0 || K <= 0) return fail(VITB200_ERR_INVALID, "gemm_tc: empty problem");
@@ -797,6 +899,11 @@ int launch_gemm_tc(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMa
     return fail(VITB200_ERR_INVALID, "gemm_tc: epilogue needs a bias");
   if (epilogue != VITB200_EPI_PATCH_F32 && tmC == nullptr)
     return fail(VITB200_ERR_INVALID, "gemm_tc: output tensor map missing");
+  if (dtype == DT_E4M3) {
+    if (tmC == nullptr) return fail(VITB200_ERR_INVALID, "gemm_tc: output tensor map missing");
+    if (epilogue != VITB200_EPI_STORE_16 && bias == nullptr) return fail(VITB200_ERR_INVALID, "gemm_tc: epilogue needs a bias");
+    return dispatch_e4m3(stream, tmA, tmB, *tmC, bias, C, M, N, K, epilogue, cta_group, drop, wscale);
+  }
   if (epilogue == VITB200_EPI_BIAS_RESID_F32) {
     // `tpi` = split-K factor: clamp so that every split owns at least one k-block
     const int num_kb = ceil_div(K, GEMM_BK);
@@ -811,7 +918,7 @@ int launch_gemm_tc(cudaStream_t stream, const CUtensorMap& tmA, const CUtensorMa
     return dispatch_epi<DT_BF16>(stream, tmA, tmB, c, bias, C, M, N, K, epilogue, aux, tpi, cta_group, drop, cls_off, cls_p, ln);
   if (dtype == DT_F16)
     return dispatch_epi<DT_F16>(stream, tmA, tmB, c, bias, C, M, N, K, epilogue, aux, tpi, cta_group, drop, cls_off, cls_p, ln);
-  return fail(VITB200_ERR_INVALID, "gemm_tc: dtype must be bf16 or fp16");
+  return fail(VITB200_ERR_INVALID, "gemm_tc: dtype must be bf16, fp16 or E4M3");
 }
 
 }  // namespace vb

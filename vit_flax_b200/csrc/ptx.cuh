@@ -258,6 +258,24 @@ __device__ __forceinline__ void umma_bf16_ss(uint32_t d_tmem, uint64_t adesc, ui
         ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
   }
 }
+// The same with 8-bit floating-point operands (kind::f8f6f4: K = 32 per instruction, still 32 bytes of a 128-byte row)
+template <int kCtaGroup>
+__device__ __forceinline__ void umma_f8_ss(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc,
+                                           uint32_t idesc, uint32_t accumulate) {
+  if constexpr (kCtaGroup == 1) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+  } else {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
+  }
+}
 // D[tmem] (+)= A[tmem] * B[smem desc]
 __device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc,
                                              uint32_t idesc, uint32_t accumulate) {
@@ -398,6 +416,16 @@ __host__ __device__ constexpr uint32_t umma_idesc_16(int M, int N, int fmt, int 
          | (uint32_t(N >> 3) << 17)      // N >> 3
          | (uint32_t(M >> 4) << 24);     // M >> 4
 }
+// kind::f8f6f4 instruction descriptor, both operands E4M3 and K-major, D fp32.  The PTX ISA's table for .kind::f8f6f4
+// puts the A / B formats in bits [7,10) / [10,13) with E4M3 = 0, E5M2 = 1, E2M3 = 3, E3M2 = 4, E2M1 = 5; the other
+// fields sit where they do for kind::f16.
+__host__ __device__ constexpr uint32_t umma_idesc_e4m3(int M, int N) {
+  return (1u << 4)                       // D format  : F32
+         | (0u << 7)                     // A format  : E4M3
+         | (0u << 10)                    // B format  : E4M3
+         | (uint32_t(N >> 3) << 17)      // N >> 3
+         | (uint32_t(M >> 4) << 24);     // M >> 4
+}
 
 // ------------------------------------------------------------------- cluster
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -412,6 +440,15 @@ __device__ __forceinline__ void cluster_sync_all() {
 
 // 16-bit storage formats of the tensor-core path (values of VITB200_DT_*)
 constexpr int DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2;
+constexpr int DT_E4M3 = 3;   // 8-bit E4M3 operands of the fp8 precision (1 byte per element)
+
+// four fp32 -> four E4M3 codes (round to nearest even, saturated to +-448), v0 in bits [0,8)
+__device__ __forceinline__ uint32_t pack4_e4m3(float v0, float v1, float v2, float v3) {
+  uint16_t lo, hi;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(v1), "f"(v0));
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(v3), "f"(v2));
+  return uint32_t(lo) | (uint32_t(hi) << 16);
+}
 
 // two fp32 -> packed 16-bit pair (lo in bits [0,16)); fp16 saturates to +-65504 instead of inf
 template <int kDT>

@@ -76,22 +76,24 @@ static bool load_encoder() {
 static CUtensorMapDataType tmap_type(int dt) {
   return dt == VITB200_DT_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
          : dt == VITB200_DT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+         : dt == VITB200_DT_E4M3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8     // E4M3 codes: TMA only moves the bytes
                                 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
 }
 
 int make_tmap_2d(CUtensorMap* out, const void* base, int64_t rows, int64_t cols, int64_t ld,
-                 int box_rows, int dt) {
+                 int box_rows, int dt, int box_bytes) {
   if (!load_encoder()) return fail(VITB200_ERR_CUDA, "cuTensorMapEncodeTiled entry point unavailable");
-  const int esz = dt == VITB200_DT_F32 ? 4 : 2;
+  const int esz = dt == VITB200_DT_F32 ? 4 : (dt == VITB200_DT_E4M3 ? 1 : 2);
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0 || (ld * esz) % 16 != 0)
     return fail(VITB200_ERR_INVALID, "TMA operand must be 16-byte aligned with a 16-byte row pitch");
   if (box_rows < 1 || box_rows > 256) return fail(VITB200_ERR_INVALID, "TMA box rows out of range");
+  if (box_bytes != 128 && box_bytes != 64) return fail(VITB200_ERR_INVALID, "TMA box width must be 64 or 128 bytes");
   cuuint64_t gdim[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
   cuuint64_t gstride[1] = {static_cast<cuuint64_t>(ld) * esz};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(128 / esz), static_cast<cuuint32_t>(box_rows)};
+  cuuint32_t box[2] = {static_cast<cuuint32_t>(box_bytes / esz), static_cast<cuuint32_t>(box_rows)};
   cuuint32_t estr[2] = {1u, 1u};
   CUresult r = g_encode(out, tmap_type(dt), 2, const_cast<void*>(base), gdim, gstride, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, box_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS)
     return fail(VITB200_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string(int(r)));

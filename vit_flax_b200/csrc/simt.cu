@@ -83,7 +83,9 @@ layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ sca
       o.y = (v[i].y - mean) * rstd * g.y + b.y;
       o.z = (v[i].z - mean) * rstd * g.z + b.z;
       o.w = (v[i].w - mean) * rstd * g.w + b.w;
-      if constexpr (kDT != DT_F32) {
+      if constexpr (kDT == DT_E4M3) {   // the A operand of the fp8 GEMMs: normalised, unscaled, saturated
+        reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(y) + int64_t(row) * dim)[c] = pack4_e4m3(o.x, o.y, o.z, o.w);
+      } else if constexpr (kDT != DT_F32) {
         uint2 p;
         p.x = pack2<kDT>(o.x, o.y);
         p.y = pack2<kDT>(o.z, o.w);
@@ -114,7 +116,8 @@ layernorm_generic_kernel(const float* __restrict__ x, const float* __restrict__ 
   const float rstd = rsqrtf(warp_sum(ss) / float(dim) + eps);
   for (int c = lane; c < dim; c += 32) {
     const float o = (xr[c] - mean) * rstd * scale[c] + bias[c];
-    if constexpr (kDT != DT_F32) reinterpret_cast<uint16_t*>(y)[int64_t(row) * dim + c] = cvt16<kDT>(o);
+    if constexpr (kDT == DT_E4M3) reinterpret_cast<uint8_t*>(y)[int64_t(row) * dim + c] = uint8_t(pack4_e4m3(o, 0.f, 0.f, 0.f) & 0xFFu);
+    else if constexpr (kDT != DT_F32) reinterpret_cast<uint16_t*>(y)[int64_t(row) * dim + c] = cvt16<kDT>(o);
     else reinterpret_cast<float*>(y)[int64_t(row) * dim + c] = o;
   }
 }
@@ -483,6 +486,43 @@ fold_scale_kernel(const float* __restrict__ W, const float* __restrict__ gamma, 
   }
   if (warp == 0 && n < N) d[n] = acc;
 }
+// ------------------------------------------------ E4M3 weight quantisation (fp8)
+// W fp32 [K, N] -> Wt E4M3 [N, Kpad], scale[n] = amax_k |W[k, n]| / 448 (1 for an all-zero column).  One CTA per 32
+// columns like fold_scale_kernel: the eight warps stream rows (coalesced over n) for the column maxima, then 32 x 32
+// tiles are transposed through shared memory so that the byte rows of Wt are written along k.
+__global__ void __launch_bounds__(256)
+quantize_e4m3_kernel(const float* __restrict__ W, uint8_t* __restrict__ Wt, float* __restrict__ scale, int K, int N, int Kpad) {
+  __shared__ float tile[32][33];
+  __shared__ float red[8][32];
+  __shared__ float sc[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int n0 = blockIdx.x * 32, n = n0 + lane;
+  float amax = 0.f;
+  if (n < N)
+    for (int k = warp; k < K; k += 8) amax = fmaxf(amax, fabsf(W[int64_t(k) * N + n]));
+  red[warp][lane] = amax;
+  __syncthreads();
+  if (warp == 0) {
+    for (int w = 1; w < 8; ++w) amax = fmaxf(amax, red[w][lane]);
+    const float s = amax > 0.f ? amax / 448.0f : 1.0f;
+    sc[lane] = s;
+    if (n < N) scale[n] = s;
+  }
+  __syncthreads();
+  for (int k0 = 0; k0 < Kpad; k0 += 32) {
+    for (int r = warp; r < 32; r += 8) {
+      const int k = k0 + r;
+      tile[r][lane] = (k < K && n < N) ? __fdiv_rn(W[int64_t(k) * N + n], sc[lane]) : 0.f;
+    }
+    __syncthreads();
+    for (int r = warp; r < 32; r += 8) {   // row n0 + r of Wt, bytes k0 + lane
+      const int nn = n0 + r, k = k0 + lane;
+      if (nn < N && k < Kpad) Wt[int64_t(nn) * Kpad + k] = uint8_t(pack4_e4m3(tile[lane][r], 0.f, 0.f, 0.f) & 0xFFu);
+    }
+    __syncthreads();
+  }
+}
+
 template <int kDT>
 __global__ void __launch_bounds__(256)
 fold_rowsum16_kernel(const uint16_t* __restrict__ Wt, float* __restrict__ c, int N, int Kpad) {
@@ -655,6 +695,7 @@ attention_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out, int
 int launch_layernorm(cudaStream_t st, const float* x, const float* g, const float* b, void* y,
                      int rows, int dim, int out_dtype, float eps, float* copy) {
   if (rows <= 0 || dim <= 0) return fail(VITB200_ERR_INVALID, "layernorm: empty problem");
+  if (out_dtype == DT_E4M3) return launch_ln_t<DT_E4M3>(st, x, g, b, y, rows, dim, eps, copy);   // only this launcher takes E4M3
   VB_DT_DISPATCH(out_dtype, return launch_ln_t<kDT>(st, x, g, b, y, rows, dim, eps, copy));
   return 0;
 }
@@ -737,6 +778,14 @@ int launch_pack_weight(cudaStream_t st, const float* W, void* Wt, int K, int N, 
   if (dtype == DT_BF16) pack_weight_kernel<DT_BF16><<<grid, 256, 0, st>>>(W, static_cast<uint16_t*>(Wt), K, N, Kpad);
   else pack_weight_kernel<DT_F16><<<grid, 256, 0, st>>>(W, static_cast<uint16_t*>(Wt), K, N, Kpad);
   VB_LAUNCH_CHECK("pack_weight_kernel");
+  return 0;
+}
+
+int launch_quantize_weight_e4m3(cudaStream_t st, const float* W, uint8_t* Wt, float* scale, int K, int N, int Kpad) {
+  if (K <= 0 || N <= 0 || Kpad < K || (Kpad % 16) != 0)
+    return fail(VITB200_ERR_INVALID, "quantize_weight_e4m3: K, N > 0 and Kpad >= K, a multiple of 16");
+  quantize_e4m3_kernel<<<ceil_div(N, 32), 256, 0, st>>>(W, Wt, scale, K, N, Kpad);
+  VB_LAUNCH_CHECK("quantize_e4m3_kernel");
   return 0;
 }
 

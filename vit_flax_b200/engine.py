@@ -39,6 +39,8 @@ class Engine:
         assert pool in {"cls", "mean"}, "pool type must be either cls (cls token) or mean (mean pooling)"
         if precision not in _lib.PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(_lib.PRECISIONS)}, got {precision!r}")
+        if precision == "fp8" and (dropout or emb_dropout):
+            raise ValueError("precision='fp8' is an inference forward: it is built for dropout rates 0 only")
         self.cfg = _lib.Config(
             image_h=ih, image_w=iw, patch_h=ph, patch_w=pw, channels=channels,
             num_classes=num_classes, dim=dim, depth=depth, heads=heads, mlp_dim=mlp_dim,
@@ -119,11 +121,16 @@ class Engine:
         return out
 
     # -- training (SURVEY.md section 8f-4) --------------------------------------
+    def _inference_only(self, what: str) -> None:
+        if self.precision == "fp8":
+            raise ValueError(f"{what}: precision='fp8' is inference only; train in 'fp16' or 'bf16'")
+
     def train_forward(self, images, out=None):
         """Forward that keeps every activation the backward pass needs; same arguments as ``forward``.
         (The FeedForward pre-activation is rounded to 16 bits before the GELU here, so the logits can
         differ from ``forward``'s in the last 16-bit digit.)"""
         torch = self._torch
+        self._inference_only("train_forward")
         self._check_images(images.shape)
         if images.dtype != torch.float32 or not images.is_cuda or not images.is_contiguous():
             raise ValueError("train_forward expects a contiguous float32 CUDA tensor")
@@ -145,6 +152,7 @@ class Engine:
         the images in ``wrt`` the image gradient is written to ``dimages`` (a contiguous float32 CUDA tensor of the
         images' shape and layout; allocated when None) and returned; otherwise None is returned."""
         torch = self._torch
+        self._inference_only("backward")
         flags = _WRT.get(wrt)
         if flags is None:
             raise ValueError(f"wrt must be one of {sorted(_WRT)}, got {wrt!r}")
@@ -219,6 +227,7 @@ class Engine:
         """One AdamW update of the fp32 leaves from the gradient buffer of the last ``backward`` (scaled by
         ``grad_scale``), with the 16-bit weight copies re-derived in place.  Asynchronous; a pending ``vjp_fn``
         of this engine is invalidated (its forward ran on the old weights)."""
+        self._inference_only("adamw_step")
         h = _lib.AdamW(lr=lr, b1=b1, b2=b2, eps=eps, weight_decay=weight_decay, max_grad_norm=max_grad_norm,
                        grad_scale=grad_scale)
         self.epoch += 1

@@ -34,7 +34,7 @@ from typing import Any, Dict, Optional, Tuple, Union
 import numpy as np
 
 from .params import _lecun_normal as lecun_normal, geometry, leaf_to_numpy
-from .vit import _current_device, _parse_wrt, _seed_from_key, _unscale_images
+from .vit import _check_trainable_precision, _current_device, _parse_wrt, _seed_from_key, _unscale_images
 
 
 def posemb_sincos_2d(h: int, w: int, dim: int, temperature: float = 10000.0) -> np.ndarray:
@@ -206,6 +206,8 @@ class SimpleViT:
         ``wrt="input"`` gives the float32 image gradient in the NCHW layout of ``img`` instead, ``wrt="both"``
         ``({'params': tree}, dimg)`` (``ViT.vjp``)."""
         want_params, want_input = _parse_wrt(wrt)
+        from . import vit as _vit
+        _check_trainable_precision(precision or _vit._DEFAULT_PRECISION, "vjp")
         import torch
         is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
         eng = self._engine(variables, img, precision, device, max_batch)

@@ -114,7 +114,8 @@ class ViT:
         back as a numpy array; a CUDA ``torch.Tensor`` stays on the device and
         a CUDA tensor is returned.  ``rngs`` is accepted and ignored at dropout
         rate 0 (Flax draws nothing there).  Keyword-only extras are ours:
-        ``precision`` ('fp16' / 'bf16' tcgen05 paths, 'fp32' validation path)."""
+        ``precision`` ('fp16' / 'bf16' tcgen05 paths, 'fp8' -- E4M3 operands on to_qkv and the FeedForward,
+        inference only, DESIGN.md -- and 'fp32', the validation path)."""
         from .runtime import get_engine   # deferred: needs torch + CUDA
         key = self._dropout_key(rngs)
 
@@ -149,6 +150,7 @@ class ViT:
         FGSM / PGD); the weight-gradient GEMMs are skipped -- or ``"both"`` -- ``({'params': tree}, dx)``, the
         order of ``jax.vjp(v.apply, variables, x)``.  ``dx`` is a CUDA tensor when ``x`` is one, numpy otherwise."""
         want_params, want_input = _parse_wrt(wrt)
+        _check_trainable_precision(precision or _DEFAULT_PRECISION, "vjp")
         from .runtime import get_engine
         import torch
         key = self._dropout_key(rngs)          # rates > 0 need rngs={'dropout': key}, like apply
@@ -229,6 +231,12 @@ def _parse_wrt(wrt: str) -> Tuple[bool, bool]:
     if wrt not in choices:
         raise ValueError(f"wrt must be one of 'params', 'input' or 'both', got {wrt!r}")
     return choices[wrt]
+
+
+def _check_trainable_precision(precision: str, what: str) -> None:
+    """fp8 is an inference forward: refused before any device work by everything that differentiates."""
+    if precision == "fp8":
+        raise ValueError(f"{what}: precision='fp8' is inference only; use 'fp16' or 'bf16' to differentiate or train")
 
 
 def _unscale_images(dx, scale: float, as_cuda: bool):
