@@ -132,6 +132,15 @@ int vitb200_forward_host(vitb200_model* m, void* stream, const float* images_hos
  * two jobs may be in flight, so the H2D copy of batch k+1 overlaps the forward of batch k.
  * wait_host blocks until the OLDEST submitted job's logits are in `logits_host`.  Host buffers
  * should be pinned and must stay valid until the job has been waited for.                     */
+/* vitb200_forward that also records the attention weights softmax(Q K^T * 64^-0.5) (vit.py:73-75) of the layers
+ * layers[0 .. n_layers) (HOST array of distinct indices in [0, depth), any order) into maps_dev, fp32 on DEVICE,
+ * [batch, n_layers, heads, T, T] in that order (T counts the class token; vit-pytorch's Recorder layout).  The logits
+ * are those of vitb200_forward; unrecorded layers run what vitb200_forward runs.  A recorded layer passes a row
+ * log-sum-exp buffer to its attention kernel and recomputes P from the same 16-bit q / k right after it, on tcgen05.
+ * Never replays or captures the forward graphs.  The first call allocates a [max_batch * heads, T] fp32 scratch kept
+ * with the model.  fp32 models: VITB200_ERR_UNSUPPORTED.                                                           */
+int vitb200_forward_attn(vitb200_model* m, void* stream, const float* images_dev, int batch, float* logits_dev,
+                         const int* layers, int n_layers, float* maps_dev);
 int vitb200_submit_host(vitb200_model* m, void* stream, const float* images_host, int batch,
                         float* logits_host);
 int vitb200_wait_host(vitb200_model* m);
@@ -326,6 +335,14 @@ int vitb200_layernorm(void* stream, const float* x, const float* scale, const fl
  * out is [batch*T, heads*64].  _tc = flash-style tensor-core kernel on 16-bit data. */
 int vitb200_attention_tc(void* stream, const void* qkv, void* out, int batch, int T, int heads,
                          int dtype);
+/* The same kernel, also writing lse [batch*heads, T] fp32 = log2 sum_j exp2(s_ij * 64^-0.5 * log2(e)), the row
+ * log-sum-exp in the log2 domain (row b*heads + h, column i); `out` is the same bits as vitb200_attention_tc's. */
+int vitb200_attention_tc_lse(void* stream, const void* qkv, void* out, float* lse, int batch, int T, int heads,
+                             int dtype);
+/* The attention weights alone: maps [batch, heads, T, T] fp32 = exp2(s_ij * 64^-0.5 * log2(e) - lse_i) with s = q k^T
+ * of the 16-bit qkv and lse from vitb200_attention_tc_lse on the same qkv.  Every element inside [T, T] is written. */
+int vitb200_attention_probs(void* stream, const void* qkv, const float* lse, float* maps, int batch, int T, int heads,
+                            int dtype);
 int vitb200_attention_f32(void* stream, const float* qkv, float* out, int batch, int T, int heads);
 
 /* weight gradient dW[M, N] += X[K, M]^T dY[K, N]: X and dY are the row-major 16-bit activations

@@ -70,6 +70,7 @@ SIGNATURES = {
     "vitb200_set_dropout_key": (_i, [_vp, C.c_uint64]),
     "vitb200_forward": (_i, [_vp, _vp, _fp, _i, _fp]),
     "vitb200_forward_host": (_i, [_vp, _vp, _fp, _i, _fp]),
+    "vitb200_forward_attn": (_i, [_vp, _vp, _fp, _i, _fp, C.POINTER(C.c_int), _i, _fp]),
     "vitb200_submit_host": (_i, [_vp, _vp, _fp, _i, _fp]),
     "vitb200_wait_host": (_i, [_vp]),
     "vitb200_profile_forward": (_i, [_vp, _vp, _fp, _i, _fp, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
@@ -101,6 +102,8 @@ SIGNATURES = {
     "vitb200_gemm_f32": (_i, [_vp, _fp, _fp, _fp, _fp, _i, _i, _i, _i, _fp, _i]),
     "vitb200_layernorm": (_i, [_vp, _fp, _fp, _fp, _vp, _i, _i, _i]),
     "vitb200_attention_tc": (_i, [_vp, _vp, _vp, _i, _i, _i, _i]),
+    "vitb200_attention_tc_lse": (_i, [_vp, _vp, _vp, _fp, _i, _i, _i, _i]),
+    "vitb200_attention_probs": (_i, [_vp, _vp, _fp, _fp, _i, _i, _i, _i]),
     "vitb200_attention_f32": (_i, [_vp, _fp, _fp, _i, _i, _i]),
     "vitb200_patchify": (_i, [_vp, _fp, _vp, _i, _i, _i, _i, _i, _i, _i, _i]),
     "vitb200_patchify_tokens": (_i, [_vp, _fp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i]),

@@ -20,7 +20,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 OUT = PKG / "libvitb200.so"
 OBJ_DIR = PKG / "build"
-SOURCES = ["runtime.cu", "gemm_tc.cu", "attention.cu", "attention_tc5.cu", "attention_tc5m.cu", "simt.cu", "patch_tc.cu", "backward.cu", "attention_bwd_tc5.cu", "optim.cu", "api.cu"]
+SOURCES = ["runtime.cu", "gemm_tc.cu", "attention.cu", "attention_tc5.cu", "attention_tc5m.cu", "simt.cu", "patch_tc.cu", "backward.cu", "attention_bwd_tc5.cu", "attention_probs_tc5.cu", "optim.cu", "api.cu"]
 HEADERS = [CSRC / "common.h", CSRC / "ptx.cuh", PKG.parent / "include" / "vitb200.h"]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -145,6 +145,8 @@ struct vitb200_model {
   DevBuf<float> stats_a, stats_b;                    // LayerNorm fold: per-row partial (sum, sum sq) of x for LN1 / LN2
   int stats_slots_cap = 0;                           // float pairs per row the two buffers hold
   DevBuf<float> img_stage, logit_stage;              // forward_host staging
+  DevBuf<float> attn_lse;                            // attention row log-sum-exp [max_batch*heads, T] of a recording
+                                                     // forward (vitb200_forward_attn), allocated by the first one
   // submit_host / wait_host: two jobs in flight (H2D of job k+1 overlaps the forward of job k)
   struct HostJob {
     DevBuf<float> img, logit;
@@ -230,7 +232,7 @@ struct vitb200_model {
     x.release();
     patches_h.release(); xn_h.release(); qkv_h.release(); o_h.release(); hid_h.release(); pooled_h.release();
     patches_f.release(); xn_f.release(); qkv_f.release(); o_f.release(); hid_f.release(); pooled_f.release();
-    img_stage.release(); logit_stage.release();
+    img_stage.release(); logit_stage.release(); attn_lse.release();
     for (auto& j : job) {
       j.img.release(); j.logit.release();
       if (j.h2d_done) cudaEventDestroy(j.h2d_done);
@@ -430,6 +432,28 @@ __global__ void add_f32_into_f32_kernel(const float* __restrict__ a, float* __re
 
 int forward_head(vitb200_model* m, cudaStream_t st, const ActMaps* am, int batch, float* logits);
 
+// Layers whose attention weights a forward records (vitb200_forward_attn): slot[l] = position of layer l in `maps`
+// [batch, n, heads, T, T] fp32, or -1.
+struct AttnRecord {
+  std::vector<int> slot;
+  int n = 0;
+  float* maps = nullptr;
+};
+
+// The attention of layer l (vit.py:69-79).  A recorded layer also keeps the row log-sum-exp and, while qkv_h still
+// holds this layer's q / k, recomputes P = exp2(s sl2 - lse2) into its slice of the maps (attention_probs_tc5.cu); one
+// lse buffer serves every layer, the probabilities kernel has consumed it before the next layer's attention runs.
+int attention_layer(vitb200_model* m, cudaStream_t st, int batch, int l, const AttnRecord* rec) {
+  const int T = m->T, heads = m->cfg.heads;
+  const int slot = rec ? rec->slot[l] : -1;
+  if (slot < 0) return launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, heads, m->dt);
+  int rc;
+  if ((rc = launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, heads, m->dt, m->attn_lse.p))) return rc;
+  const int64_t per_layer = int64_t(heads) * T * T;
+  return launch_attention_probs(st, m->qkv_h.p, m->attn_lse.p, rec->maps + slot * per_layer, rec->n * per_layer, batch, T,
+                                heads, m->dt);
+}
+
 // vit.py:146-153 as one kernel (patch_tc.cu): im2col TMA over the caller's images + GEMM + cls / pos placement; `ln` non-null
 // adds the LayerNorm-fold outputs.  The im2col map depends on the images pointer: kept per (pointer, batch), a handful.
 int patch_embed_im2col(vitb200_model* m, cudaStream_t st, const float* images, int batch, const LnFold* ln) {
@@ -452,7 +476,8 @@ int patch_embed_im2col(vitb200_model* m, cudaStream_t st, const float* images, i
 // patchify | patch GEMM (TOKENS_LN: x, x16, stats_a) | per layer: to_qkv (LN_STORE_16 on x16 / stats_a) | attention |
 // to_out (RESID_LN: x, x16, stats_b) | FF Dense_0 (LN_GELU_16 on x16 / stats_b) | FF Dense_1 (RESID_LN -> stats_a; plain
 // RESID in the last layer) | pool + LayerNorm | head.  x16 lives in the buffer the LayerNorm kernel used to write.
-int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int batch, float* logits) {
+int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int batch, float* logits,
+                    const AttnRecord* rec = nullptr) {
   const auto& c = m->cfg;
   const int D = c.dim, I = m->inner, T = m->T;
   const int R = batch * T;
@@ -487,7 +512,7 @@ int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int 
     if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map_ln(cg_qkv), &am->c_qkv, L.qkv.ln_d, m->qkv_h.p, R, 3 * I, D,
                              VITB200_EPI_LN_STORE_16, nullptr, 0, m->dt, cg_qkv, Dropout(), m->cls_off, nullptr, in_a))) return rc;
     mark(m, st, VITB200_CAT_ATTENTION);
-    if ((rc = launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, c.heads, m->dt))) return rc;
+    if ((rc = attention_layer(m, st, batch, l, rec))) return rc;
     mark(m, st, VITB200_CAT_GEMM_OUT);
     if ((rc = launch_gemm_tc(st, am->o, L.out.map(cg_d), &am->c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, R, D, I,
                              VITB200_EPI_RESID_LN, nullptr, 0, m->dt, cg_d, Dropout(), m->cls_off, nullptr, out_b))) return rc;
@@ -509,8 +534,10 @@ int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int 
 }
 
 // ---- the forward schedule, bf16 / tcgen05 flavour ---------------------------
-int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch, float* logits) {
-  if (m->fold) return forward_tc_fold(m, st, images, batch, logits);
+// `rec` (vitb200_forward_attn): record the attention weights of some layers; null = the plain forward
+int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch, float* logits,
+               const AttnRecord* rec = nullptr) {
+  if (m->fold) return forward_tc_fold(m, st, images, batch, logits, rec);
   const auto& c = m->cfg;
   const int D = c.dim, I = m->inner, T = m->T;
   const int R = batch * T;
@@ -547,7 +574,7 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
                                nullptr, 0, VITB200_DT_E4M3, cg_qkv, Dropout(), m->cls_off, nullptr, LnFold(), L.qkv.wscale))) return rc;
     } else if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map(cg_qkv), &am->c_qkv, nullptr, m->qkv_h.p, R, 3 * I, D, VITB200_EPI_STORE_16, nullptr, 0, m->dt, cg_qkv))) return rc;
     mark(m, st, VITB200_CAT_ATTENTION);
-    if ((rc = launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, c.heads, m->dt))) return rc;
+    if ((rc = attention_layer(m, st, batch, l, rec))) return rc;
     mark(m, st, VITB200_CAT_GEMM_OUT);
     if (m->project_out) {
       if ((rc = launch_gemm_tc(st, am->o, L.out.map(cg_d), &am->c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, R, D, I, VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d, m->drop(c.dropout, 1 + 3 * l)))) return rc;
@@ -922,6 +949,36 @@ int vitb200_forward(vitb200_model* m, void* stream, const float* images_dev, int
   if (!m->tc) return forward_f32(m, st, images_dev, batch, logits_dev);
   if (graph_eligible(m, st, batch)) return forward_graph(m, st, images_dev, batch, logits_dev);
   return forward_tc(m, st, images_dev, batch, logits_dev);
+}
+
+int vitb200_forward_attn(vitb200_model* m, void* stream, const float* images_dev, int batch, float* logits_dev,
+                         const int* layers, int n_layers, float* maps_dev) {
+  if (!m || !images_dev || !logits_dev || !layers || !maps_dev) return fail(VITB200_ERR_INVALID, "forward_attn: null argument");
+  if (!m->finalized) return fail(VITB200_ERR_PARAM_MISSING, "forward_attn: call finalize_params first");
+  if (batch <= 0 || batch > m->cfg.max_batch) return fail(VITB200_ERR_INVALID, "forward_attn: batch must be in [1, max_batch]");
+  const int depth = m->cfg.depth;
+  if (n_layers <= 0 || n_layers > depth) return fail(VITB200_ERR_INVALID, "forward_attn: n_layers must be in [1, depth]");
+  AttnRecord rec;
+  rec.slot.assign(size_t(depth), -1);
+  rec.n = n_layers;
+  rec.maps = maps_dev;
+  for (int i = 0; i < n_layers; ++i) {
+    const int l = layers[i];
+    if (l < 0 || l >= depth) return fail(VITB200_ERR_INVALID, "forward_attn: layer index outside [0, depth)");
+    if (rec.slot[size_t(l)] >= 0) return fail(VITB200_ERR_INVALID, "forward_attn: a layer is listed twice");
+    rec.slot[size_t(l)] = i;
+  }
+  if (!m->tc) return fail(VITB200_ERR_UNSUPPORTED, "forward_attn: the fp32 validation path does not record attention maps");
+  DeviceGuard guard(m->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (m->attn_lse.n == 0) {
+    int rc;
+    if ((rc = m->attn_lse.alloc(size_t(m->cfg.max_batch) * m->cfg.heads * m->T))) return rc;
+  }
+  // the same workspace as vitb200_forward: a pending backward is refused afterwards
+  if (m->train && m->train->fwd_batch != 0) { m->train->fwd_batch = 0; m->train->stale = true; }
+  // launched directly: a recording forward neither replays nor captures the forward graphs
+  return forward_tc(m, st, images_dev, batch, logits_dev, &rec);
 }
 
 int vitb200_forward_host(vitb200_model* m, void* stream, const float* images_host, int batch, float* logits_host) {
@@ -1695,6 +1752,17 @@ int vitb200_layernorm(void* stream, const float* x, const float* scale, const fl
 int vitb200_attention_tc(void* stream, const void* qkv, void* out, int batch, int T, int heads, int dtype) {
   if (!qkv || !out) return fail(VITB200_ERR_INVALID, "attention_tc: null pointer");
   return launch_attention_tc(static_cast<cudaStream_t>(stream), qkv, out, batch, T, heads, dtype);
+}
+
+int vitb200_attention_tc_lse(void* stream, const void* qkv, void* out, float* lse, int batch, int T, int heads, int dtype) {
+  if (!qkv || !out || !lse) return fail(VITB200_ERR_INVALID, "attention_tc_lse: null pointer");
+  return launch_attention_tc(static_cast<cudaStream_t>(stream), qkv, out, batch, T, heads, dtype, lse);
+}
+
+int vitb200_attention_probs(void* stream, const void* qkv, const float* lse, float* maps, int batch, int T, int heads,
+                            int dtype) {
+  return launch_attention_probs(static_cast<cudaStream_t>(stream), qkv, lse, maps, int64_t(heads) * T * T, batch, T, heads,
+                                dtype);
 }
 
 int vitb200_attention_f32(void* stream, const float* qkv, float* out, int batch, int T, int heads) {

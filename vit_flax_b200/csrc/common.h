@@ -134,7 +134,8 @@ int launch_gemm_f32(cudaStream_t stream, const float* A, const float* W, const f
 int launch_layernorm(cudaStream_t stream, const float* x, const float* scale, const float* bias,
                      void* y, int rows, int dim, int out_dtype, float eps = 1e-6f, float* copy = nullptr);
 // `copy` (training): the kernel also writes x to `copy`, the residual buffer the following GEMM adds into
-// `lse` (optional, T <= 208 only): [batch*heads, T] fp32, the row log-sum-exp in the log2 domain, kept for the adjoint
+// `lse` (optional): [batch*heads, T] fp32, the row log-sum-exp in the log2 domain, kept for the adjoint and the
+// attention maps
 int launch_attention_tc(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
                         int heads, int dtype, float* lse = nullptr);
 bool attention_tc5_supports(int T);
@@ -145,6 +146,11 @@ int launch_attention_tc5m(cudaStream_t stream, const void* qkv, void* out, int b
                           int heads, int dtype, float* lse = nullptr);
 int launch_attention_f32(cudaStream_t stream, const float* qkv, float* out, int batch, int T,
                          int heads);
+// Attention weights P = exp2(Q K^T sl2 - lse2) of one layer, recomputed on tcgen05 from the to_qkv output and the row
+// log-sum-exp of launch_attention_tc (attention_probs_tc5.cu): fp32 element (b, h, i, j) at
+// out[b * img_stride + (h * T + i) * T + j], so one launch fills a layer's slice of a [batch, layers, heads, T, T] tensor.
+int launch_attention_probs(cudaStream_t stream, const void* qkv, const float* lse2, float* out, int64_t img_stride,
+                           int batch, int T, int heads, int dtype);
 int launch_patchify(cudaStream_t stream, const float* images, void* patches, int batch, int H,
                     int W, int C, int ph, int pw, int Kpad, int out_dtype, int nchw = 0, int tok_off = 0);
 // adjoint of launch_patchify for fp32 patches: images (NHWC, or NCHW) <- patches [batch*(Np+tok_off), Kpad]; every

@@ -7,7 +7,7 @@ compute happens inside ``libvitb200.so``.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import numpy as np
 
@@ -119,6 +119,32 @@ class Engine:
         _lib.check(self.lib.vitb200_forward(self.handle, _stream_ptr(torch, images.device),
                                             images.data_ptr(), b, out.data_ptr()))
         return out
+
+    def forward_attn(self, images, layers, out=None, maps=None):
+        """``forward`` that also records the attention weights ``softmax(q k^T * 64^-0.5)`` of ``layers`` (distinct
+        indices in ``[0, depth)``, in the order given): returns ``(logits, maps)``, ``maps`` a float32 CUDA tensor
+        ``[B, len(layers), heads, T, T]`` (allocated when None).  The logits are ``forward``'s."""
+        torch = self._torch
+        if self.precision == "fp32":
+            raise ValueError("forward_attn: the fp32 validation path does not record attention maps; use 'fp16', "
+                             "'bf16' or 'fp8'")
+        layers = check_layers(layers, self.cfg.depth)
+        self._check_images(images.shape)
+        if images.dtype != torch.float32 or not images.is_cuda or not images.is_contiguous():
+            raise ValueError("forward_attn expects a contiguous float32 CUDA tensor")
+        b = images.shape[0]
+        shape = (b, len(layers), self.cfg.heads, self.tokens, self.tokens)
+        if maps is not None:
+            check_maps(torch, maps, shape, images.device)
+        else:
+            maps = torch.empty(shape, dtype=torch.float32, device=images.device)
+        if out is None:
+            out = torch.empty((b, self.num_classes), dtype=torch.float32, device=images.device)
+        arr = (C.c_int * len(layers))(*layers)
+        self.epoch += 1
+        _lib.check(self.lib.vitb200_forward_attn(self.handle, _stream_ptr(torch, images.device), images.data_ptr(), b,
+                                                 out.data_ptr(), arr, len(layers), maps.data_ptr()))
+        return out, maps
 
     # -- training (SURVEY.md section 8f-4) --------------------------------------
     def _inference_only(self, what: str) -> None:
@@ -375,6 +401,35 @@ class Engine:
             self.close()
         except Exception:
             pass
+
+
+def check_layers(layers, depth: int) -> List[int]:
+    """The ``layers`` of an attention-map request as a list of ints: distinct, each in ``[0, depth)``, at least one;
+    ``None`` means every layer.  Anything else is a ``ValueError`` (raised before any device work)."""
+    if layers is None:
+        return list(range(depth))
+    if isinstance(layers, (int, np.integer)) or isinstance(layers, (str, bytes)):
+        raise ValueError(f"layers must be a sequence of layer indices, got {layers!r}")
+    out = []
+    for l in layers:
+        if isinstance(l, (bool, np.bool_)) or not isinstance(l, (int, np.integer)):
+            raise ValueError(f"layers must hold ints, got {l!r}")
+        if not 0 <= int(l) < depth:
+            raise ValueError(f"layer {int(l)} outside [0, depth={depth})")
+        out.append(int(l))
+    if not out:
+        raise ValueError("layers must name at least one layer")
+    if len(set(out)) != len(out):
+        raise ValueError(f"layers must be distinct, got {out}")
+    return out
+
+
+def check_maps(torch, maps, shape, device) -> None:
+    """A caller's ``maps`` buffer must be a contiguous float32 tensor of ``shape`` on ``device``."""
+    if not (isinstance(maps, torch.Tensor) and maps.dtype == torch.float32 and maps.is_contiguous()
+            and tuple(maps.shape) == tuple(shape) and maps.device == torch.device(device)):
+        got = f"{maps.dtype} {tuple(maps.shape)} on {maps.device}" if isinstance(maps, torch.Tensor) else type(maps).__name__
+        raise ValueError(f"maps must be a contiguous float32 tensor of shape {tuple(shape)} on {device}, got {got}")
 
 
 def _device_view(torch, device, ptr: int, n: int, typestr: str):

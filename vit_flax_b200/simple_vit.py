@@ -242,6 +242,26 @@ class SimpleViT:
         from .train import Trainer
         return Trainer(self, variables, tx, precision=precision, device=device, max_batch=max_batch)
 
+    def attention_maps(self, variables: Any, img: Any, rngs: Any = None, *, layers=None, precision: Optional[str] = None,
+                       device: Optional[int] = None, max_batch: Optional[int] = None):
+        """``ViT.attention_maps`` for SimpleViT: ``(logits, maps)``, ``maps`` float32 ``[B, len(layers), heads, T, T]``
+        with ``T = num_patches`` (no class token); ``img`` is NCHW."""
+        from . import vit as _vit
+        from .engine import check_layers
+        if (precision or _vit._DEFAULT_PRECISION) == "fp32":
+            raise ValueError("attention_maps: the fp32 validation path does not record attention maps; use 'fp16', "
+                             "'bf16' or 'fp8'")
+        layers = check_layers(layers, self.depth)
+        import torch
+        is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
+        eng = self._engine(variables, img, precision, device, max_batch)
+        if is_cuda:
+            x = img if (img.dtype == torch.float32 and img.is_contiguous()) else img.float().contiguous()
+            return eng.forward_attn(x, layers)
+        x = torch.as_tensor(np.asarray(img, dtype=np.float32), device=eng.device)
+        logits, maps = eng.forward_attn(x, layers)
+        return logits.cpu().numpy(), maps.cpu().numpy()
+
     # ------------------------------------------------------------------- apply
     def apply(self, variables: Any, img: Any, rngs: Any = None, *, precision: Optional[str] = None,
               device: Optional[int] = None, max_batch: Optional[int] = None, reload: bool = False):

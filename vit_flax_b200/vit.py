@@ -116,23 +116,52 @@ class ViT:
         rate 0 (Flax draws nothing there).  Keyword-only extras are ours:
         ``precision`` ('fp16' / 'bf16' tcgen05 paths, 'fp8' -- E4M3 operands on to_qkv and the FeedForward,
         inference only, DESIGN.md -- and 'fp32', the validation path)."""
+        eng, xin = self._forward_engine(variables, x, rngs, precision, device, max_batch, reload)
+        if xin is not None:
+            return eng.forward(xin)
+        return eng.forward_host(np.asarray(x, dtype=np.float32))
+
+    def _forward_engine(self, variables, x, rngs, precision, device, max_batch, reload):
+        """What ``apply`` and ``attention_maps`` share: the dropout key (checked first), the image checks, the device,
+        the cached engine with ``variables`` loaded and the key set.  Returns ``(engine, x as a contiguous float32 CUDA
+        tensor)`` for a CUDA ``x``, ``(engine, None)`` for a host array."""
         from .runtime import get_engine   # deferred: needs torch + CUDA
         key = self._dropout_key(rngs)
-
         is_torch_cuda = hasattr(x, "is_cuda") and bool(x.is_cuda)
         channels = self._validate(tuple(x.shape) if hasattr(x, "shape") else np.shape(x))
         batch = int(x.shape[0])
         if device is None:
             device = x.device.index if is_torch_cuda and x.device.index is not None else _current_device()
-        eng = get_engine(self, channels, precision or _DEFAULT_PRECISION, device,
-                         max_batch or batch, variables, reload)
+        eng = get_engine(self, channels, precision or _DEFAULT_PRECISION, device, max_batch or batch, variables, reload)
         if key is not None:
             eng.set_dropout_key(key)
-        if is_torch_cuda:
-            import torch
-            xin = x if (x.dtype == torch.float32 and x.is_contiguous()) else x.float().contiguous()
-            return eng.forward(xin)
-        return eng.forward_host(np.asarray(x, dtype=np.float32))
+        if not is_torch_cuda:
+            return eng, None
+        import torch
+        return eng, (x if (x.dtype == torch.float32 and x.is_contiguous()) else x.float().contiguous())
+
+    def attention_maps(self, variables: Any, x: Any, rngs: Any = None, *, layers=None, precision: Optional[str] = None,
+                       device: Optional[int] = None, max_batch: Optional[int] = None, reload: bool = False):
+        """``apply`` that also returns the attention weights ``softmax(q k^T * dim_head^-0.5)`` (vit.py:73-75) of
+        ``layers`` (ours; vit-pytorch's ``Recorder`` returns the same): ``(logits, maps)``, ``maps`` float32
+        ``[B, len(layers), heads, T, T]`` with ``T = num_patches + 1`` (the class token is row and column 0).
+
+        ``layers``: distinct layer indices in ``[0, depth)``, recorded in the order given; default every layer.
+        ``logits`` are ``apply``'s, bit for bit.  A CUDA tensor in gives CUDA tensors out, a host array numpy.  With
+        dropout > 0 pass ``rngs={'dropout': key}`` as for ``apply``: the maps are those of that dropped forward (the
+        reference drops no attention weights, vit.py:75-83).  The maps are recomputed on the tensor cores from the
+        16-bit q / k of the forward (precision 'fp16', 'bf16' or 'fp8'); 'fp32' is refused.  ``reload`` as for ``apply``."""
+        from .engine import check_layers
+        if (precision or _DEFAULT_PRECISION) == "fp32":
+            raise ValueError("attention_maps: the fp32 validation path does not record attention maps; use 'fp16', "
+                             "'bf16' or 'fp8'")
+        layers = check_layers(layers, self.depth)
+        eng, xin = self._forward_engine(variables, x, rngs, precision, device, max_batch, reload)
+        if xin is not None:
+            return eng.forward_attn(xin, layers)
+        import torch
+        logits, maps = eng.forward_attn(torch.as_tensor(np.asarray(x, dtype=np.float32), device=eng.device), layers)
+        return logits.cpu().numpy(), maps.cpu().numpy()
 
     def vjp(self, variables: Any, x: Any, rngs: Any = None, *, wrt: str = "params", precision: Optional[str] = None,
             device: Optional[int] = None, max_batch: Optional[int] = None):
