@@ -161,7 +161,12 @@ int vitb200_wait_host(vitb200_model* m);
 int vitb200_profile_forward(vitb200_model* m, void* stream, const float* images_dev, int batch,
                             float* logits_dev, float* ms_by_category, int* launches_by_category);
 /* Copy the token stream after the last block ([batch, T, dim] fp32, device to
- * host) -- parity checks of Transformer.__call__ (vit.py:98-112).            */
+ * host) -- parity checks of Transformer.__call__ (vit.py:98-112).  A dropout-free
+ * tcgen05 forward with pool = cls computes the last block for the class-token rows
+ * only (DESIGN.md section 3, class-token tail): after such a forward this returns
+ * VITB200_ERR_UNSUPPORTED rather than stale rows.  A forward that records the last
+ * layer (vitb200_forward_attn), mean pooling, dropout > 0 and fp32 models run the
+ * whole block, and the stream is readable after them.                          */
 int vitb200_debug_tokens(vitb200_model* m, void* stream, float* tokens_host, int batch);
 
 /* ---- training: forward that keeps its activations + backward (SURVEY.md section 8f-4) -----

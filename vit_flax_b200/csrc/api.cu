@@ -88,6 +88,7 @@ struct ActMaps {   // TMA descriptors over the activation workspace for one batc
   CUtensorMap patches, xn, o, h, pooled;   // A operands
   CUtensorMap c_qkv, c_hid, c_x;           // GEMM outputs (TMA store / reduce-add)
   CUtensorMap xn8, h8, c_hid8;             // fp8: the E4M3 views of xn_h / hid_h (A operands, FF Dense_0 output)
+  CUtensorMap o_cls, c_x_cls;              // class-token tail: rows b*T of o_h [B, I] and of x [B, D] (row pitch T*I, T*D)
 };
 
 }  // namespace
@@ -147,6 +148,8 @@ struct vitb200_model {
   DevBuf<float> img_stage, logit_stage;              // forward_host staging
   DevBuf<float> attn_lse;                            // attention row log-sum-exp [max_batch*heads, T] of a recording
                                                      // forward (vitb200_forward_attn), allocated by the first one
+  bool tokens_partial = false;                       // the last inference forward ran the class-token tail: only rows
+                                                     // b*T of x hold the output of the last block (vitb200_debug_tokens)
   // submit_host / wait_host: two jobs in flight (H2D of job k+1 overlaps the forward of job k)
   struct HostJob {
     DevBuf<float> img, logit;
@@ -343,6 +346,9 @@ int get_act_maps(vitb200_model* m, int batch, const ActMaps** out) {
     if ((rc = make_tmap_2d(&am.c_qkv, m->qkv_h.p, R, 3 * m->inner, 3 * m->inner, GEMM_BM, dt))) return rc;
     if ((rc = make_tmap_2d(&am.c_hid, m->hid_h.p, R, c.mlp_dim, c.mlp_dim, GEMM_BM, dt))) return rc;
     if ((rc = make_tmap_2d(&am.c_x, m->x.p, R, c.dim, c.dim, GEMM_BM, VITB200_DT_F32))) return rc;
+    const int64_t T = m->T;
+    if ((rc = make_tmap_2d(&am.o_cls, m->o_h.p, batch, m->inner, T * m->inner, GEMM_BM, dt))) return rc;
+    if ((rc = make_tmap_2d(&am.c_x_cls, m->x.p, batch, c.dim, T * c.dim, GEMM_BM, VITB200_DT_F32))) return rc;
     if (m->fp8) {   // E4M3 codes in the first half of the 16-bit buffers' bytes: the workspace does not grow
       if ((rc = make_tmap_2d(&am.xn8, m->xn_h.p, R, c.dim, c.dim, GEMM_BM, VITB200_DT_E4M3))) return rc;
       if ((rc = make_tmap_2d(&am.h8, m->hid_h.p, R, c.mlp_dim, c.mlp_dim, GEMM_BM, VITB200_DT_E4M3))) return rc;
@@ -443,10 +449,11 @@ struct AttnRecord {
 // The attention of layer l (vit.py:69-79).  A recorded layer also keeps the row log-sum-exp and, while qkv_h still
 // holds this layer's q / k, recomputes P = exp2(s sl2 - lse2) into its slice of the maps (attention_probs_tc5.cu); one
 // lse buffer serves every layer, the probabilities kernel has consumed it before the next layer's attention runs.
-int attention_layer(vitb200_model* m, cudaStream_t st, int batch, int l, const AttnRecord* rec) {
+// `q_tiles` as launch_attention_tc: 1 in the class-token tail, which never records.
+int attention_layer(vitb200_model* m, cudaStream_t st, int batch, int l, const AttnRecord* rec, int q_tiles = 0) {
   const int T = m->T, heads = m->cfg.heads;
   const int slot = rec ? rec->slot[l] : -1;
-  if (slot < 0) return launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, heads, m->dt);
+  if (slot < 0) return launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, heads, m->dt, nullptr, q_tiles);
   int rc;
   if ((rc = launch_attention_tc(st, m->qkv_h.p, m->o_h.p, batch, T, heads, m->dt, m->attn_lse.p))) return rc;
   const int64_t per_layer = int64_t(heads) * T * T;
@@ -472,10 +479,25 @@ int patch_embed_im2col(vitb200_model* m, cudaStream_t st, const float* images, i
                                    c.channels, c.dim, m->cls_off, m->dt, ln);
 }
 
+// The class-token tail (DESIGN.md section 3).  With pool = 'cls' the logits read row b*T of the token stream alone, and in
+// the last block that row depends on the other rows only through their keys and values: to_qkv runs over every row,
+// attention over q tile 0 (which holds the class query) of every (image, head), and to_out, FF Dense_0 and FF Dense_1 as
+// GEMMs of M = batch rows over the class-token rows.  Their tile mode and statistics slots stay those of the [B*T, N]
+// GEMMs, so the class rows see the same MMA shape and the same summation order: the logits are bit-identical.  Kept off
+// where other rows matter or are indexed: mean pooling, dropout (masks by token row), an identity to_out, the fp32 path,
+// and a forward that records the last layer's attention weights (every query row; the whole tail then runs in full).
+bool cls_tail(const vitb200_model* m, const AttnRecord* rec) {
+  const auto& c = m->cfg;
+  return m->tc && c.pool == VITB200_POOL_CLS && m->cls_off == 1 && m->project_out && c.depth > 0 && c.dropout == 0.f &&
+         c.emb_dropout == 0.f && !(rec && rec->slot[size_t(c.depth - 1)] >= 0);
+}
+
 // ---- the forward schedule with every PreNorm LayerNorm folded into the GEMMs around it: 4 + 5L launches ----
 // patchify | patch GEMM (TOKENS_LN: x, x16, stats_a) | per layer: to_qkv (LN_STORE_16 on x16 / stats_a) | attention |
 // to_out (RESID_LN: x, x16, stats_b) | FF Dense_0 (LN_GELU_16 on x16 / stats_b) | FF Dense_1 (RESID_LN -> stats_a; plain
 // RESID in the last layer) | pool + LayerNorm | head.  x16 lives in the buffer the LayerNorm kernel used to write.
+// In the class-token tail the last layer's to_out / FF GEMMs write x16, stats_b and hid compact ([batch, ...]); its to_qkv
+// has consumed xn_h and stats_a before.
 int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int batch, float* logits,
                     const AttnRecord* rec = nullptr) {
   const auto& c = m->cfg;
@@ -504,29 +526,34 @@ int forward_tc_fold(vitb200_model* m, cudaStream_t st, const float* images, int 
                              R, D, m->K0pad, VITB200_EPI_TOKENS_LN, leaf_ptr(m, m->leaf_pos), T, m->dt, cg_d,
                              Dropout(), m->cls_off, leaf_ptr(m, m->leaf_cls), out_a))) return rc;
   }
+  const bool tail = cls_tail(m, rec);
   for (int l = 0; l < c.depth; ++l) {   // vit.py:108-110
     Layer& L = m->layers[l];
+    const bool cls_rows = tail && l + 1 == c.depth;   // rows after attention: the class tokens alone
+    const int M = cls_rows ? batch : R;
+    const CUtensorMap& a_o = cls_rows ? am->o_cls : am->o;
+    const CUtensorMap& c_x = cls_rows ? am->c_x_cls : am->c_x;
     // Residual(PreNorm(Attention))  vit.py:31,39,62-87
     mark(m, st, VITB200_CAT_GEMM_QKV);
     in_a.c = L.qkv.ln_c;
     if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map_ln(cg_qkv), &am->c_qkv, L.qkv.ln_d, m->qkv_h.p, R, 3 * I, D,
                              VITB200_EPI_LN_STORE_16, nullptr, 0, m->dt, cg_qkv, Dropout(), m->cls_off, nullptr, in_a))) return rc;
     mark(m, st, VITB200_CAT_ATTENTION);
-    if ((rc = attention_layer(m, st, batch, l, rec))) return rc;
+    if ((rc = attention_layer(m, st, batch, l, rec, cls_rows ? 1 : 0))) return rc;
     mark(m, st, VITB200_CAT_GEMM_OUT);
-    if ((rc = launch_gemm_tc(st, am->o, L.out.map(cg_d), &am->c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, R, D, I,
+    if ((rc = launch_gemm_tc(st, a_o, L.out.map(cg_d), &c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, M, D, I,
                              VITB200_EPI_RESID_LN, nullptr, 0, m->dt, cg_d, Dropout(), m->cls_off, nullptr, out_b))) return rc;
     // Residual(PreNorm(FeedForward))  vit.py:31,39,47-53
     mark(m, st, VITB200_CAT_GEMM_FF1);
     in_b.c = L.ff1.ln_c;
-    if ((rc = launch_gemm_tc(st, am->xn, L.ff1.map_ln(cg_ff1), &am->c_hid, L.ff1.ln_d, m->hid_h.p, R, c.mlp_dim, D,
+    if ((rc = launch_gemm_tc(st, am->xn, L.ff1.map_ln(cg_ff1), &am->c_hid, L.ff1.ln_d, m->hid_h.p, M, c.mlp_dim, D,
                              VITB200_EPI_LN_GELU_16, nullptr, 0, m->dt, cg_ff1, Dropout(), m->cls_off, nullptr, in_b))) return rc;
     mark(m, st, VITB200_CAT_GEMM_FF2);
     if (l + 1 < c.depth) {
       if ((rc = launch_gemm_tc(st, am->h, L.ff2.map(cg_d), &am->c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, R, D, c.mlp_dim,
                                VITB200_EPI_RESID_LN, nullptr, 0, m->dt, cg_d, Dropout(), m->cls_off, nullptr, out_a))) return rc;
     } else {   // nothing normalises the last layer's output row by row: pool + head LayerNorm read x itself
-      if ((rc = launch_gemm_tc(st, am->h, L.ff2.map(cg_d), &am->c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, R, D, c.mlp_dim,
+      if ((rc = launch_gemm_tc(st, am->h, L.ff2.map(cg_d), &c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, M, D, c.mlp_dim,
                                VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d))) return rc;
     }
   }
@@ -563,8 +590,14 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
                                R, D, m->K0pad, VITB200_EPI_TOKENS_F32, leaf_ptr(m, m->leaf_pos), T, m->dt, cgp,
                                m->drop(c.emb_dropout, 0), m->cls_off, leaf_ptr(m, m->leaf_cls)))) return rc;
   }
+  const bool tail = cls_tail(m, rec);
   for (int l = 0; l < c.depth; ++l) {   // vit.py:108-110
     Layer& L = m->layers[l];
+    // class-token tail: after attention the last layer works on rows b*T alone, its second LayerNorm writes xn_h compact
+    const bool cls_rows = tail && l + 1 == c.depth;
+    const int M = cls_rows ? batch : R;
+    const CUtensorMap& a_o = cls_rows ? am->o_cls : am->o;
+    const CUtensorMap& c_x = cls_rows ? am->c_x_cls : am->c_x;
     // Residual(PreNorm(Attention))  vit.py:31,39,62-87
     mark(m, st, VITB200_CAT_LAYERNORM);
     if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln1_scale), leaf_ptr(m, L.ln1_bias), m->xn_h.p, R, D, ln_dt, m->eps))) return rc;
@@ -574,10 +607,10 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
                                nullptr, 0, VITB200_DT_E4M3, cg_qkv, Dropout(), m->cls_off, nullptr, LnFold(), L.qkv.wscale))) return rc;
     } else if ((rc = launch_gemm_tc(st, am->xn, L.qkv.map(cg_qkv), &am->c_qkv, nullptr, m->qkv_h.p, R, 3 * I, D, VITB200_EPI_STORE_16, nullptr, 0, m->dt, cg_qkv))) return rc;
     mark(m, st, VITB200_CAT_ATTENTION);
-    if ((rc = attention_layer(m, st, batch, l, rec))) return rc;
+    if ((rc = attention_layer(m, st, batch, l, rec, cls_rows ? 1 : 0))) return rc;
     mark(m, st, VITB200_CAT_GEMM_OUT);
     if (m->project_out) {
-      if ((rc = launch_gemm_tc(st, am->o, L.out.map(cg_d), &am->c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, R, D, I, VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d, m->drop(c.dropout, 1 + 3 * l)))) return rc;
+      if ((rc = launch_gemm_tc(st, a_o, L.out.map(cg_d), &c_x, leaf_ptr(m, L.out.leaf_bias), m->x.p, M, D, I, VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d, m->drop(c.dropout, 1 + 3 * l)))) return rc;
     } else {   // heads == 1 and dim == 64: to_out is the identity (vit.py:65,85)
       const int64_t n = int64_t(R) * D;
       add_16_into_f32_kernel<<<unsigned((n + 255) / 256), 256, 0, st>>>(m->o_h.p, m->x.p, n, m->dt);
@@ -585,22 +618,23 @@ int forward_tc(vitb200_model* m, cudaStream_t st, const float* images, int batch
     }
     // Residual(PreNorm(FeedForward))  vit.py:31,39,47-53
     mark(m, st, VITB200_CAT_LAYERNORM);
-    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln2_scale), leaf_ptr(m, L.ln2_bias), m->xn_h.p, R, D, ln_dt, m->eps))) return rc;
+    if ((rc = launch_layernorm(st, m->x.p, leaf_ptr(m, L.ln2_scale), leaf_ptr(m, L.ln2_bias), m->xn_h.p, M, D, ln_dt, m->eps,
+                               nullptr, cls_rows ? int64_t(T) * D : D))) return rc;
     if (m->fp8) {   // E4M3 in, E4M3 hidden activations, E4M3 in again: FF Dense_0 -> GELU -> FF Dense_1
       mark(m, st, VITB200_CAT_GEMM_FF1);
-      if ((rc = launch_gemm_tc(st, am->xn8, L.ff1.map(cg_ff1), &am->c_hid8, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, R, c.mlp_dim, D,
+      if ((rc = launch_gemm_tc(st, am->xn8, L.ff1.map(cg_ff1), &am->c_hid8, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, M, c.mlp_dim, D,
                                VITB200_EPI_BIAS_GELU_E4M3, nullptr, 0, VITB200_DT_E4M3, cg_ff1, Dropout(), m->cls_off, nullptr,
                                LnFold(), L.ff1.wscale))) return rc;
       mark(m, st, VITB200_CAT_GEMM_FF2);
-      if ((rc = launch_gemm_tc(st, am->h8, L.ff2.map(cg_d), &am->c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, R, D, c.mlp_dim,
+      if ((rc = launch_gemm_tc(st, am->h8, L.ff2.map(cg_d), &c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, M, D, c.mlp_dim,
                                VITB200_EPI_BIAS_RESID_F32, nullptr, 0, VITB200_DT_E4M3, cg_d, Dropout(), m->cls_off, nullptr,
                                LnFold(), L.ff2.wscale))) return rc;
       continue;
     }
     mark(m, st, VITB200_CAT_GEMM_FF1);
-    if ((rc = launch_gemm_tc(st, am->xn, L.ff1.map(cg_ff1), &am->c_hid, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, R, c.mlp_dim, D, VITB200_EPI_BIAS_GELU_16, nullptr, 0, m->dt, cg_ff1, m->drop(c.dropout, 2 + 3 * l)))) return rc;
+    if ((rc = launch_gemm_tc(st, am->xn, L.ff1.map(cg_ff1), &am->c_hid, leaf_ptr(m, L.ff1.leaf_bias), m->hid_h.p, M, c.mlp_dim, D, VITB200_EPI_BIAS_GELU_16, nullptr, 0, m->dt, cg_ff1, m->drop(c.dropout, 2 + 3 * l)))) return rc;
     mark(m, st, VITB200_CAT_GEMM_FF2);
-    if ((rc = launch_gemm_tc(st, am->h, L.ff2.map(cg_d), &am->c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, R, D, c.mlp_dim, VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d, m->drop(c.dropout, 3 + 3 * l)))) return rc;
+    if ((rc = launch_gemm_tc(st, am->h, L.ff2.map(cg_d), &c_x, leaf_ptr(m, L.ff2.leaf_bias), m->x.p, M, D, c.mlp_dim, VITB200_EPI_BIAS_RESID_F32, nullptr, 0, m->dt, cg_d, m->drop(c.dropout, 3 + 3 * l)))) return rc;
   }
   return forward_head(m, st, am, batch, logits);
 }
@@ -946,6 +980,7 @@ int vitb200_forward(vitb200_model* m, void* stream, const float* images_dev, int
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // an inference forward re-uses the patch matrix a pending backward would read: that backward is now refused
   if (m->train && m->train->fwd_batch != 0) { m->train->fwd_batch = 0; m->train->stale = true; }
+  m->tokens_partial = cls_tail(m, nullptr);
   if (!m->tc) return forward_f32(m, st, images_dev, batch, logits_dev);
   if (graph_eligible(m, st, batch)) return forward_graph(m, st, images_dev, batch, logits_dev);
   return forward_tc(m, st, images_dev, batch, logits_dev);
@@ -977,6 +1012,7 @@ int vitb200_forward_attn(vitb200_model* m, void* stream, const float* images_dev
   }
   // the same workspace as vitb200_forward: a pending backward is refused afterwards
   if (m->train && m->train->fwd_batch != 0) { m->train->fwd_batch = 0; m->train->stale = true; }
+  m->tokens_partial = cls_tail(m, &rec);
   // launched directly: a recording forward neither replays nor captures the forward graphs
   return forward_tc(m, st, images_dev, batch, logits_dev, &rec);
 }
@@ -1083,6 +1119,10 @@ int vitb200_profile_forward(vitb200_model* m, void* stream, const float* images_
 int vitb200_debug_tokens(vitb200_model* m, void* stream, float* tokens_host, int batch) {
   if (!m || !tokens_host) return fail(VITB200_ERR_INVALID, "debug_tokens: null argument");
   if (batch <= 0 || batch > m->cfg.max_batch) return fail(VITB200_ERR_INVALID, "debug_tokens: bad batch");
+  if (m->tokens_partial)
+    return fail(VITB200_ERR_UNSUPPORTED, "debug_tokens: the last forward ran the class-token tail (pool = 'cls'): its last "
+                                         "block computed only the class-token rows, the other rows are stale.  A forward that "
+                                         "records the last layer's attention weights (vitb200_forward_attn) runs it in full");
   DeviceGuard guard(m->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   VB_CUDA(cudaMemcpyAsync(tokens_host, m->x.p, size_t(batch) * m->T * m->cfg.dim * sizeof(float), cudaMemcpyDeviceToHost, st));

@@ -11,11 +11,11 @@
 namespace vb {
 
 int launch_attention_tc(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads,
-                        int dtype, float* lse) {
+                        int dtype, float* lse, int q_tiles) {
   if (batch <= 0 || T <= 0 || heads <= 0)
     return fail(VITB200_ERR_INVALID, "attention_tc: empty problem");
-  if (attention_tc5_supports(T)) return launch_attention_tc5(stream, qkv, out, batch, T, heads, dtype, lse);
-  return launch_attention_tc5m(stream, qkv, out, batch, T, heads, dtype, lse);
+  if (attention_tc5_supports(T)) return launch_attention_tc5(stream, qkv, out, batch, T, heads, dtype, lse, q_tiles);
+  return launch_attention_tc5m(stream, qkv, out, batch, T, heads, dtype, lse, q_tiles);
 }
 
 }  // namespace vb

@@ -480,7 +480,7 @@ int attn_turns() {
 }
 
 template <int kDT, int KP>
-int launch_kp(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse) {
+int launch_kp(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse, int q_tiles) {
   using L = Smem<KP>;
   static PerDevice<bool> configured_on;   // the smem opt-in is per (function, device)
   if (bool& configured = configured_on.here(); !configured) {
@@ -493,7 +493,9 @@ int launch_kp(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
   if ((rc = make_tmap_3d_16(&tq, qkv, batch, T, 3 * inner, 3 * inner, QT, kDT))) return rc;
   if ((rc = make_tmap_3d_16(&tkv, qkv, batch, T, 3 * inner, 3 * inner, KP, kDT))) return rc;
   if ((rc = make_tmap_3d_16(&to, out, batch, T, inner, inner, QT, kDT))) return rc;
-  const int nqt = ceil_div(T, QT);
+  // items are (image, head, q tile) with nqt q tiles per (image, head): fewer than ceil(T / QT) computes only the first
+  // query rows of every image (the class-token tail of the forward needs q tile 0 alone)
+  const int nqt = q_tiles > 0 && q_tiles < ceil_div(T, QT) ? q_tiles : ceil_div(T, QT);
   const int64_t items64 = int64_t(batch) * heads * nqt;
   if (items64 > 0x7fffffff) return fail(VITB200_ERR_INVALID, "attention: too many work items");
   const int items = int(items64);
@@ -505,10 +507,10 @@ int launch_kp(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
 }
 
 template <int kDT>
-int launch_dt(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse) {
-  if (T <= 64) return launch_kp<kDT, 64>(stream, qkv, out, batch, T, heads, lse);      // KMIN: T > 0 / 64 / 128
-  if (T <= 128) return launch_kp<kDT, 128>(stream, qkv, out, batch, T, heads, lse);
-  return launch_kp<kDT, 208>(stream, qkv, out, batch, T, heads, lse);
+int launch_dt(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse, int q_tiles) {
+  if (T <= 64) return launch_kp<kDT, 64>(stream, qkv, out, batch, T, heads, lse, q_tiles);      // KMIN: T > 0 / 64 / 128
+  if (T <= 128) return launch_kp<kDT, 128>(stream, qkv, out, batch, T, heads, lse, q_tiles);
+  return launch_kp<kDT, 208>(stream, qkv, out, batch, T, heads, lse, q_tiles);
 }
 
 }  // namespace
@@ -524,11 +526,11 @@ namespace vb {
 bool attention_tc5_supports(int T) { return T >= 1 && T <= 208; }
 
 int launch_attention_tc5(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads,
-                         int dtype, float* lse) {
+                         int dtype, float* lse, int q_tiles) {
   if (batch <= 0 || T <= 0 || heads <= 0) return fail(VITB200_ERR_INVALID, "attention: empty problem");
   if (!attention_tc5_supports(T)) return fail(VITB200_ERR_UNSUPPORTED, "attention_tc5: T > 208");
-  if (dtype == DT_BF16) return launch_dt<DT_BF16>(stream, qkv, out, batch, T, heads, lse);
-  if (dtype == DT_F16) return launch_dt<DT_F16>(stream, qkv, out, batch, T, heads, lse);
+  if (dtype == DT_BF16) return launch_dt<DT_BF16>(stream, qkv, out, batch, T, heads, lse, q_tiles);
+  if (dtype == DT_F16) return launch_dt<DT_F16>(stream, qkv, out, batch, T, heads, lse, q_tiles);
   return fail(VITB200_ERR_INVALID, "attention: dtype must be bf16 or fp16");
 }
 

@@ -422,7 +422,7 @@ int attn_m_turns() {   // VITB200_ATTN_TURNS=0: free-running groups (A/B tests)
 }
 
 template <int kDT, int KP>
-int launch_m(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse) {
+int launch_m(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse, int q_tiles) {
   using L = SmemM<KP>;
   static PerDevice<bool> configured_on;   // the smem opt-in is per (function, device)
   if (bool& configured = configured_on.here(); !configured) {
@@ -436,7 +436,8 @@ int launch_m(cudaStream_t stream, const void* qkv, void* out, int batch, int T, 
   if ((rc = make_tmap_3d_16(&tq, qkv, batch, T, 3 * inner, 3 * inner, QT, kDT))) return rc;
   if ((rc = make_tmap_3d_16(&tkv, qkv, batch, T, 3 * inner, 3 * inner, KP, kDT))) return rc;
   if ((rc = make_tmap_3d_16(&to, out, batch, T, inner, inner, QT, kDT))) return rc;
-  const int nqt = ceil_div(T, QT), nkb = ceil_div(T, KP);
+  // nqt q tiles per (image, head): fewer than ceil(T / QT) computes only the first query rows of every image
+  const int nqt = q_tiles > 0 && q_tiles < ceil_div(T, QT) ? q_tiles : ceil_div(T, QT), nkb = ceil_div(T, KP);
   const int64_t items64 = int64_t(batch) * heads * nqt;
   if (items64 > 0x7fffffff / nkb) return fail(VITB200_ERR_INVALID, "attention: too many work items");
   const int items = int(items64);
@@ -448,19 +449,19 @@ int launch_m(cudaStream_t stream, const void* qkv, void* out, int batch, int T, 
 }
 
 template <int kDT>
-int launch_m_dt(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse) {
+int launch_m_dt(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads, float* lse, int q_tiles) {
   // two blocks of 144 cover T <= 288 (ViT-H/14: 257) with less padding than two of 192
-  if (T <= 288) return launch_m<kDT, 144>(stream, qkv, out, batch, T, heads, lse);
-  return launch_m<kDT, 192>(stream, qkv, out, batch, T, heads, lse);
+  if (T <= 288) return launch_m<kDT, 144>(stream, qkv, out, batch, T, heads, lse, q_tiles);
+  return launch_m<kDT, 192>(stream, qkv, out, batch, T, heads, lse, q_tiles);
 }
 
 }  // namespace
 
 int launch_attention_tc5m(cudaStream_t stream, const void* qkv, void* out, int batch, int T, int heads,
-                          int dtype, float* lse) {
+                          int dtype, float* lse, int q_tiles) {
   if (batch <= 0 || T <= 0 || heads <= 0) return fail(VITB200_ERR_INVALID, "attention: empty problem");
-  if (dtype == DT_BF16) return launch_m_dt<DT_BF16>(stream, qkv, out, batch, T, heads, lse);
-  if (dtype == DT_F16) return launch_m_dt<DT_F16>(stream, qkv, out, batch, T, heads, lse);
+  if (dtype == DT_BF16) return launch_m_dt<DT_BF16>(stream, qkv, out, batch, T, heads, lse, q_tiles);
+  if (dtype == DT_F16) return launch_m_dt<DT_F16>(stream, qkv, out, batch, T, heads, lse, q_tiles);
   return fail(VITB200_ERR_INVALID, "attention: dtype must be bf16 or fp16");
 }
 

@@ -132,18 +132,22 @@ int launch_gemm_f32(cudaStream_t stream, const float* A, const float* W, const f
                     float* C, int M, int N, int K, int epilogue, const float* aux,
                     int tokens_per_image, const Dropout& drop = Dropout(), int cls_off = 1);
 int launch_layernorm(cudaStream_t stream, const float* x, const float* scale, const float* bias,
-                     void* y, int rows, int dim, int out_dtype, float eps = 1e-6f, float* copy = nullptr);
+                     void* y, int rows, int dim, int out_dtype, float eps = 1e-6f, float* copy = nullptr,
+                     int64_t ldx = 0);
 // `copy` (training): the kernel also writes x to `copy`, the residual buffer the following GEMM adds into
+// `ldx`: row pitch of x in elements (0 = dim); y (and copy) stay dense [rows, dim]
 // `lse` (optional): [batch*heads, T] fp32, the row log-sum-exp in the log2 domain, kept for the adjoint and the
 // attention maps
+// `q_tiles` (> 0): only the first q_tiles 128-query tiles of every (image, head) are computed, the other rows of `out`
+// (and of `lse`) are left as they were; 0 = all ceil(T / 128)
 int launch_attention_tc(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
-                        int heads, int dtype, float* lse = nullptr);
+                        int heads, int dtype, float* lse = nullptr, int q_tiles = 0);
 bool attention_tc5_supports(int T);
 int launch_attention_tc5(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
-                         int heads, int dtype, float* lse = nullptr);
+                         int heads, int dtype, float* lse = nullptr, int q_tiles = 0);
 // tcgen05 kernel for T > 208: streamed key blocks, online softmax (attention_tc5m.cu)
 int launch_attention_tc5m(cudaStream_t stream, const void* qkv, void* out, int batch, int T,
-                          int heads, int dtype, float* lse = nullptr);
+                          int heads, int dtype, float* lse = nullptr, int q_tiles = 0);
 int launch_attention_f32(cudaStream_t stream, const float* qkv, float* out, int batch, int T,
                          int heads);
 // Attention weights P = exp2(Q K^T sl2 - lse2) of one layer, recomputed on tcgen05 from the to_qkv output and the row

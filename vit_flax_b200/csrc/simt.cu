@@ -36,7 +36,8 @@ template <int NV, int kDT, bool kCopy>
 __global__ void __launch_bounds__(256)
 layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ scale,
                       const float* __restrict__ bias, void* __restrict__ y, int rows, int dim, int reverse, float eps,
-                      float* __restrict__ copy) {   // copy != null (training): also x -> copy, the next residual buffer
+                      float* __restrict__ copy,     // copy != null (training): also x -> copy, the next residual buffer
+                      int64_t ldx) {                // row pitch of x (y and copy are dense)
   pdl_launch_dependents();
   pdl_wait();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -45,7 +46,7 @@ layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ sca
   // GEMM that follows starts with the row blocks this kernel wrote last (VITB200_LN_REVERSE=0: off).
   const int row = reverse ? rows - 1 - (blockIdx.x * 8 + warp) : blockIdx.x * 8 + warp;
   if (row < 0 || row >= rows) return;
-  const float4* xr = reinterpret_cast<const float4*>(x + int64_t(row) * dim);
+  const float4* xr = reinterpret_cast<const float4*>(x + int64_t(row) * ldx);
   const int nvec = dim >> 2;
   float4 v[NV];
   float s = 0.f;
@@ -101,13 +102,13 @@ layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ sca
 template <int kDT>
 __global__ void __launch_bounds__(256)
 layernorm_generic_kernel(const float* __restrict__ x, const float* __restrict__ scale,
-                         const float* __restrict__ bias, void* __restrict__ y, int rows, int dim, float eps) {
+                         const float* __restrict__ bias, void* __restrict__ y, int rows, int dim, float eps, int64_t ldx) {
   pdl_launch_dependents();
   pdl_wait();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int row = blockIdx.x * 8 + warp;
   if (row >= rows) return;
-  const float* xr = x + int64_t(row) * dim;
+  const float* xr = x + int64_t(row) * ldx;
   float s = 0.f;
   for (int c = lane; c < dim; c += 32) s += xr[c];
   const float mean = warp_sum(s) / float(dim);
@@ -133,26 +134,26 @@ int ln_reverse() {
 
 template <int kDT>
 int launch_ln_t(cudaStream_t st, const float* x, const float* g, const float* b, void* y, int rows,
-                int dim, float eps, float* copy) {
+                int dim, float eps, float* copy, int64_t ldx) {
   const int grid = ceil_div(rows, 8);
-  const bool vec = (dim % 4 == 0) && dim <= 2048 &&
+  const bool vec = (dim % 4 == 0) && (ldx % 4 == 0) && dim <= 2048 &&
                    ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) |
                      reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(b)) & 15) == 0;
   if (!vec || (reinterpret_cast<uintptr_t>(copy) & 15) != 0) {
     if (copy != nullptr) VB_CUDA(cudaMemcpyAsync(copy, x, size_t(rows) * dim * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    VB_CUDA(launch_kernel(layernorm_generic_kernel<kDT>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, eps));
+    VB_CUDA(launch_kernel(layernorm_generic_kernel<kDT>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, eps, ldx));
   } else {
     const int nv = ceil_div(dim, 128);
-    if (nv <= 4) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<4, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy));
-                   else VB_CUDA(launch_kernel(layernorm_rows_kernel<4, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy)); }
-    else if (nv <= 6) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<6, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy));
-                        else VB_CUDA(launch_kernel(layernorm_rows_kernel<6, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy)); }
-    else if (nv <= 8) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<8, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy));
-                        else VB_CUDA(launch_kernel(layernorm_rows_kernel<8, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy)); }
-    else if (nv <= 10) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<10, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy));
-                         else VB_CUDA(launch_kernel(layernorm_rows_kernel<10, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy)); }
-    else { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<16, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy));
-           else VB_CUDA(launch_kernel(layernorm_rows_kernel<16, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy)); }
+    if (nv <= 4) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<4, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx));
+                   else VB_CUDA(launch_kernel(layernorm_rows_kernel<4, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx)); }
+    else if (nv <= 6) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<6, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx));
+                        else VB_CUDA(launch_kernel(layernorm_rows_kernel<6, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx)); }
+    else if (nv <= 8) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<8, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx));
+                        else VB_CUDA(launch_kernel(layernorm_rows_kernel<8, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx)); }
+    else if (nv <= 10) { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<10, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx));
+                         else VB_CUDA(launch_kernel(layernorm_rows_kernel<10, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx)); }
+    else { if (copy) VB_CUDA(launch_kernel(layernorm_rows_kernel<16, kDT, true>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx));
+           else VB_CUDA(launch_kernel(layernorm_rows_kernel<16, kDT, false>, dim3(grid), dim3(256), 0, st, 1, x, g, b, y, rows, dim, ln_reverse(), eps, copy, ldx)); }
   }
   VB_LAUNCH_CHECK("layernorm");
   return 0;
@@ -693,10 +694,12 @@ attention_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out, int
   }
 
 int launch_layernorm(cudaStream_t st, const float* x, const float* g, const float* b, void* y,
-                     int rows, int dim, int out_dtype, float eps, float* copy) {
+                     int rows, int dim, int out_dtype, float eps, float* copy, int64_t ldx) {
   if (rows <= 0 || dim <= 0) return fail(VITB200_ERR_INVALID, "layernorm: empty problem");
-  if (out_dtype == DT_E4M3) return launch_ln_t<DT_E4M3>(st, x, g, b, y, rows, dim, eps, copy);   // only this launcher takes E4M3
-  VB_DT_DISPATCH(out_dtype, return launch_ln_t<kDT>(st, x, g, b, y, rows, dim, eps, copy));
+  if (ldx == 0) ldx = dim;
+  if (ldx < dim || (copy != nullptr && ldx != dim)) return fail(VITB200_ERR_INVALID, "layernorm: bad row pitch of x");
+  if (out_dtype == DT_E4M3) return launch_ln_t<DT_E4M3>(st, x, g, b, y, rows, dim, eps, copy, ldx);   // only this launcher takes E4M3
+  VB_DT_DISPATCH(out_dtype, return launch_ln_t<kDT>(st, x, g, b, y, rows, dim, eps, copy, ldx));
   return 0;
 }
 

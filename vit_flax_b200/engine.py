@@ -385,6 +385,11 @@ class Engine:
         return {name: (float(ms[i]), int(cnt[i])) for i, name in enumerate(_lib.CATEGORIES)}
 
     def tokens_after_transformer(self, batch: int) -> np.ndarray:
+        """The token stream ``[batch, T, dim]`` after the last block of the last forward (vit.py:157).
+
+        Raises ``VitB200Error`` after a forward that ran the class-token tail (pool='cls', no dropout, fp16 / bf16 /
+        fp8): its last block computed the class-token rows only (DESIGN.md section 3).  ``forward_attn`` with the last
+        layer among ``layers`` runs that block in full, after which the stream is readable."""
         out = np.empty((batch, self.tokens, self.dim), np.float32)
         _lib.check(self.lib.vitb200_debug_tokens(self.handle, _stream_ptr(self._torch, self.device),
                                                  out.ctypes.data, batch))
