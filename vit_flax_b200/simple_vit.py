@@ -34,7 +34,8 @@ from typing import Any, Dict, Optional, Tuple, Union
 import numpy as np
 
 from .params import _lecun_normal as lecun_normal, geometry, leaf_to_numpy
-from .vit import _check_trainable_precision, _current_device, _parse_wrt, _seed_from_key, _unscale_images
+from .runtime import _FrontEnd, clear_cache  # noqa: F401  (the one engine cache; importable here as before)
+from .vit import _seed_from_key
 
 
 def posemb_sincos_2d(h: int, w: int, dim: int, temperature: float = 10000.0) -> np.ndarray:
@@ -49,7 +50,7 @@ def posemb_sincos_2d(h: int, w: int, dim: int, temperature: float = 10000.0) -> 
 
 
 @dataclasses.dataclass(frozen=True)
-class SimpleViT:
+class SimpleViT(_FrontEnd):
     """Same fields, order and defaults as simple_vit.py:99-108."""
     image_size: Union[int, Tuple[int, int]]
     patch_size: Union[int, Tuple[int, int]]
@@ -67,11 +68,28 @@ class SimpleViT:
             raise NotImplementedError("the attention kernels are built for dim_head = 64")
         return ih, iw, ph, pw, n
 
-    def _validate(self, shape):
+    def _validate(self, shape) -> int:
         ih, iw, _, _, _ = self._geometry()
         if len(shape) != 4 or tuple(int(s) for s in shape[1:]) != (self.channels, ih, iw):
             raise ValueError(f"expected images [B, {self.channels}, {ih}, {iw}] (NCHW, simple_vit.py:125), "
                              f"got {tuple(shape)}")
+        return self.channels
+
+    # the hooks of runtime._FrontEnd (the params tree and its two layouts are below)
+    def _engine_kwargs(self, channels: int) -> Dict[str, Any]:
+        ih, iw, ph, pw, _ = self._geometry()
+        return dict(image_size=(ih, iw), patch_size=(ph, pw), num_classes=self.num_classes, dim=self.dim,
+                    depth=self.depth, heads=self.heads, mlp_dim=self.mlp_dim, pool="mean", channels=channels,
+                    nchw=True, cls_token=False, ln_eps=1e-5)
+
+    def _param_channels(self, variables) -> int:
+        return self.channels
+
+    def _dropout_key(self, rngs) -> None:
+        return None                                   # simple_vit.py has no dropout
+
+    def _layout(self, variables) -> str:
+        return self._split_tree(variables)[0]
 
     # ------------------------------------------------------------------ params
     def init(self, rngs: Any, x: Any) -> Dict[str, Dict]:
@@ -150,39 +168,10 @@ class SimpleViT:
             "LayerNorm_0": {"scale": f(norm["scale"]), "bias": z(self.dim)},
             "Dense_1": {k: f(v) for k, v in head.items()}}}
 
-    def _engine(self, variables, img, precision, device, max_batch, reload=False):
-        from . import vit as _vit
-        from .engine import Engine
-        from .runtime import ParamsStamp
-        is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
-        self._validate(tuple(img.shape) if hasattr(img, "shape") else np.shape(img))
-        batch = int(img.shape[0])
-        if device is None:
-            device = img.device.index if is_cuda and img.device.index is not None else _current_device()
-        key = (self, precision or _vit._DEFAULT_PRECISION, device)
-        eng, loaded = _ENGINES.get(key, (None, None))
-        if eng is None or eng.max_batch < (max_batch or batch):
-            if eng is not None:
-                eng.close()
-            ih, iw, ph, pw, _ = self._geometry()
-            eng = Engine(image_size=(ih, iw), patch_size=(ph, pw), num_classes=self.num_classes, dim=self.dim,
-                         depth=self.depth, heads=self.heads, mlp_dim=self.mlp_dim, pool="mean",
-                         channels=self.channels, precision=precision or _vit._DEFAULT_PRECISION,
-                         max_batch=max_batch or batch, device=device, nchw=True, cls_token=False, ln_eps=1e-5)
-            loaded = None
-        # identity by strong reference + content probe (runtime.ParamsStamp): an id() alone is recycled by
-        # CPython for the temporary dict of ``v.apply({'params': p}, x)``
-        stamp = ParamsStamp(variables)
-        if reload or not stamp.matches(loaded):
-            eng.load_params(self._engine_tree(variables))
-            loaded = stamp
-        _ENGINES[key] = (eng, loaded)
-        return eng
-
     def _grads_tree(self, flat: Dict[str, np.ndarray], layout: str = "construction") -> Dict[str, Any]:
-        """Engine gradients (vit.py leaf names) -> the SimpleViT pytree in the layout the caller's params
-        came in; the gradients of leaves SimpleViT does not have (zero biases, the fixed sin/cos table, the
-        unused cls) are dropped."""
+        """Engine-path leaves (vit.py leaf names: gradients, or a Trainer's weights and moments) -> the SimpleViT
+        pytree in the layout the caller's params came in; the leaves SimpleViT does not have (zero biases, the fixed
+        sin/cos table, the unused cls) are dropped."""
         t = {}
         for l in range(self.depth):
             pre = "Transformer_0/"
@@ -205,35 +194,7 @@ class SimpleViT:
         ``(logits, vjp_fn)``, ``vjp_fn(dlogits)`` -> ``{'params': tree}`` of float32 gradients in SimpleViT's names.
         ``wrt="input"`` gives the float32 image gradient in the NCHW layout of ``img`` instead, ``wrt="both"``
         ``({'params': tree}, dimg)`` (``ViT.vjp``)."""
-        want_params, want_input = _parse_wrt(wrt)
-        from . import vit as _vit
-        _check_trainable_precision(precision or _vit._DEFAULT_PRECISION, "vjp")
-        import torch
-        is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
-        eng = self._engine(variables, img, precision, device, max_batch)
-        layout = self._split_tree(variables)[0]
-        batch = int(img.shape[0])
-        x = img if is_cuda else torch.as_tensor(np.asarray(img, dtype=np.float32), device=eng.device)
-        x = x if (x.dtype == torch.float32 and x.is_contiguous()) else x.float().contiguous()
-        logits = eng.train_forward(x)
-        epoch = eng.epoch      # any later forward / reload on this engine invalidates vjp_fn
-
-        def vjp_fn(dlogits):
-            d = dlogits if hasattr(dlogits, "is_cuda") else torch.as_tensor(np.asarray(dlogits, dtype=np.float32))
-            d = d.to(device=eng.device, dtype=torch.float32).contiguous()
-            if tuple(d.shape) != (batch, self.num_classes):
-                raise ValueError(f"vjp_fn expects a cotangent of shape ({batch}, {self.num_classes})")
-            peak = float(d.abs().max())
-            scale = 1.0 if peak == 0.0 or not np.isfinite(peak) else float(2.0 ** -np.round(np.log2(peak)))
-            dx = eng.backward(d * scale if scale != 1.0 else d, epoch=epoch, wrt=wrt)
-            out = []
-            if want_params:
-                out.append(self._grads_tree({k: g / np.float32(scale) for k, g in eng.grads().items()}, layout))
-            if want_input:
-                out.append(_unscale_images(dx, scale, is_cuda))
-            return out[0] if len(out) == 1 else tuple(out)
-
-        return (logits if is_cuda else logits.cpu().numpy()), vjp_fn
+        return self._vjp(variables, img, None, wrt, precision, device, max_batch)
 
     def trainer(self, variables: Any, tx, *, precision: Optional[str] = None, device: Optional[int] = None,
                 max_batch: Optional[int] = None):
@@ -246,40 +207,11 @@ class SimpleViT:
                        device: Optional[int] = None, max_batch: Optional[int] = None):
         """``ViT.attention_maps`` for SimpleViT: ``(logits, maps)``, ``maps`` float32 ``[B, len(layers), heads, T, T]``
         with ``T = num_patches`` (no class token); ``img`` is NCHW."""
-        from . import vit as _vit
-        from .engine import check_layers
-        if (precision or _vit._DEFAULT_PRECISION) == "fp32":
-            raise ValueError("attention_maps: the fp32 validation path does not record attention maps; use 'fp16', "
-                             "'bf16' or 'fp8'")
-        layers = check_layers(layers, self.depth)
-        import torch
-        is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
-        eng = self._engine(variables, img, precision, device, max_batch)
-        if is_cuda:
-            x = img if (img.dtype == torch.float32 and img.is_contiguous()) else img.float().contiguous()
-            return eng.forward_attn(x, layers)
-        x = torch.as_tensor(np.asarray(img, dtype=np.float32), device=eng.device)
-        logits, maps = eng.forward_attn(x, layers)
-        return logits.cpu().numpy(), maps.cpu().numpy()
+        return self._attention_maps(variables, img, rngs, layers, precision, device, max_batch, False)
 
     # ------------------------------------------------------------------- apply
     def apply(self, variables: Any, img: Any, rngs: Any = None, *, precision: Optional[str] = None,
               device: Optional[int] = None, max_batch: Optional[int] = None, reload: bool = False):
         """``v.apply(params, img)`` -> logits ``[B, num_classes]`` float32; ``img`` is NCHW.  ``reload=True``
         forces the weights to be re-packed (after an in-place edit the content probe did not see)."""
-        is_cuda = hasattr(img, "is_cuda") and bool(img.is_cuda)
-        eng = self._engine(variables, img, precision, device, max_batch, reload)
-        if is_cuda:
-            import torch
-            x = img if (img.dtype == torch.float32 and img.is_contiguous()) else img.float().contiguous()
-            return eng.forward(x)
-        return eng.forward_host(np.asarray(img, dtype=np.float32))
-
-
-_ENGINES: Dict[Any, Any] = {}
-
-
-def clear_cache() -> None:
-    for eng, _ in _ENGINES.values():
-        eng.close()
-    _ENGINES.clear()
+        return self._apply(variables, img, rngs, precision, device, max_batch, reload)

@@ -10,8 +10,9 @@ Loss scaling: the cotangent of a mean cross-entropy over B images is at most 1/B
 intermediates at large B; the kernel scales it by S = 2^round(log2 B) and the optimiser divides the gradient buffer
 by S (times the data-parallel world size) as it reads it.
 
-The Trainer owns its ``Engine``.  It is not one from the cache behind ``ViT.apply``: that cache recognises a params
-tree by its leaves, and after training it would otherwise hand the trained weights to ``ViT.apply(params0, x)``.
+The Trainer owns its ``Engine``.  It is not one from the cache behind ``model.apply`` (runtime.py): that cache
+recognises a params tree by its leaves, and after training it would otherwise hand the trained weights to
+``model.apply(params0, x)``.
 """
 from __future__ import annotations
 
@@ -21,10 +22,9 @@ from typing import Any, Dict, Optional
 import numpy as np
 
 from . import _lib
-from .checkpoint import _unflatten
-from .engine import Engine
 from .optim import AdamW
-from .params import flatten_params, geometry, leaf_to_numpy
+from .params import flatten_params, leaf_to_numpy
+from .runtime import _DEFAULT_PRECISION, _device_images, _is_cuda, _new_engine
 
 
 def _fold_in(seed: int, step: int) -> int:
@@ -60,40 +60,22 @@ class Trainer:
     def __init__(self, model, variables, tx: AdamW, *, precision: Optional[str] = None, device: Optional[int] = None,
                  max_batch: Optional[int] = None):
         import torch
-        from . import vit as _vit
-        from .simple_vit import SimpleViT
         if not isinstance(tx, AdamW):
             raise ValueError("tx must come from vit_flax_b200.adamw(...)")
-        precision = precision or _vit._DEFAULT_PRECISION
+        precision = precision or _DEFAULT_PRECISION
         if precision not in ("fp16", "bf16"):
             raise ValueError(f"training runs in the fp16 or bf16 precision, got {precision!r}")
         self._torch = torch
         self.model = model
         self.tx = tx
-        self._simple = isinstance(model, SimpleViT)
         device = torch.cuda.current_device() if device is None else int(device)
         max_batch = 256 if max_batch is None else int(max_batch)
-        if self._simple:
-            ih, iw, ph, pw, _ = model._geometry()
-            self._layout = model._split_tree(variables)[0]
-            eng = Engine(image_size=(ih, iw), patch_size=(ph, pw), num_classes=model.num_classes, dim=model.dim,
-                         depth=model.depth, heads=model.heads, mlp_dim=model.mlp_dim, pool="mean", channels=model.channels,
-                         precision=precision, max_batch=max_batch, device=device, nchw=True, cls_token=False, ln_eps=1e-5)
-            table = eng.param_table()
-            # caller's path -> engine path; the engine leaves SimpleViT lacks (zero biases, sin/cos table, cls) are frozen
-            ident = model._grads_tree({p: p for p in table}, self._layout)
-            self._to_engine = dict(flatten_params(ident))
-            eng.load_params(model._engine_tree(variables))
-        else:
-            _, _, ph, pw, _ = geometry(model.image_size, model.patch_size)
-            k0 = int(np.shape(flatten_params(variables)["Dense_0/kernel"])[0])
-            eng = Engine(image_size=model.image_size, patch_size=model.patch_size, num_classes=model.num_classes,
-                         dim=model.dim, depth=model.depth, heads=model.heads, mlp_dim=model.mlp_dim, pool=model.pool,
-                         channels=k0 // (ph * pw), precision=precision, max_batch=max_batch, device=device,
-                         dropout=model.dropout, emb_dropout=model.emb_dropout)
-            table = eng.param_table()
-            self._to_engine = {p: p for p in table}
-            eng.load_params(variables)
+        self._layout = model._layout(variables)
+        eng = _new_engine(model, model._param_channels(variables), precision, device, max_batch)
+        table = eng.param_table()
+        # caller's path -> engine path; engine leaves the model lacks (SimpleViT: zero biases, sin/cos table, cls) are frozen
+        self._to_engine = dict(flatten_params(model._grads_tree({p: p for p in table}, self._layout)))
+        eng.load_params(model._engine_tree(variables))
         self._eng = eng
         self._offsets = eng.leaf_offsets()
         decay = tx.decay_mask({cp: table[ep] for cp, ep in self._to_engine.items()})
@@ -107,18 +89,8 @@ class Trainer:
 
     # ------------------------------------------------------------------ inputs
     def _images(self, x):
-        torch = self._torch
-        is_cuda = hasattr(x, "is_cuda") and bool(x.is_cuda)
-        shape = tuple(x.shape) if hasattr(x, "shape") else np.shape(x)
-        if self._simple:
-            self.model._validate(shape)
-        self._eng._check_images(shape)
-        if is_cuda:
-            return x if (x.dtype == torch.float32 and x.is_contiguous()) else x.float().contiguous()
-        return torch.as_tensor(np.asarray(x, dtype=np.float32), device=self._eng.device)
-
-    def _dropout_key(self, rngs):
-        return None if self._simple else self.model._dropout_key(rngs)
+        self._eng._check_images(np.shape(x))      # the whole image shape, in the model's layout, and the batch
+        return _device_images(self._eng, x)
 
     # -------------------------------------------------------------------- step
     def step(self, x, labels, *, rngs: Any = None, label_smoothing: float = 0.0):
@@ -132,7 +104,7 @@ class Trainer:
             raise ValueError(f"label_smoothing must be in [0, 1], got {label_smoothing!r}")
         b = int((x.shape if hasattr(x, "shape") else np.shape(x))[0])
         y = check_labels(labels, b)
-        key = self._dropout_key(rngs)
+        key = self.model._dropout_key(rngs)
         lr = self.tx.lr(self._step)
         x = self._images(x)
         y = y.to(device=self._eng.device, dtype=self._torch.int32).contiguous()
@@ -159,12 +131,11 @@ class Trainer:
     def apply(self, x, rngs: Any = None):
         """The forward with the current weights, like ``model.apply``: a CUDA tensor in gives CUDA logits, a host
         array numpy logits."""
-        key = self._dropout_key(rngs)
+        key = self.model._dropout_key(rngs)
         if key is not None:
             self._eng.set_dropout_key(key)
-        is_cuda = hasattr(x, "is_cuda") and bool(x.is_cuda)
-        xin = self._images(x)
-        return self._eng.forward(xin) if is_cuda else self._eng.forward(xin).cpu().numpy()
+        logits = self._eng.forward(self._images(x))
+        return logits if _is_cuda(x) else logits.cpu().numpy()
 
     def last_step(self):
         """``(count, skipped, grad_norm)``: applied updates so far, whether the last step was skipped (non-finite
@@ -174,9 +145,7 @@ class Trainer:
     # ------------------------------------------------------------------ state
     def _caller_tree(self, flat: Dict[str, np.ndarray]):
         """Engine-path leaves -> ``{'params': tree}`` in the caller's layout."""
-        if self._simple:
-            return self.model._grads_tree(flat, self._layout)
-        return {"params": _unflatten(flat)}
+        return self.model._grads_tree(flat, self._layout)
 
     def params(self) -> Dict[str, Any]:
         """``{'params': tree}`` of the current weights, numpy float32, in the layout the params came in (what
@@ -198,7 +167,7 @@ class Trainer:
         """Restore a ``state_dict()`` (of a Trainer of the same model and layout)."""
         torch = self._torch
         eng = self._eng
-        eng.load_params(self.model._engine_tree(state["params"]) if self._simple else state["params"])
+        eng.load_params(self.model._engine_tree(state["params"]))
         mu, nu, cnt = eng.optim_state()
         for dst, tree in ((mu, state["mu"]), (nu, state["nu"])):
             flat = flatten_params(tree)

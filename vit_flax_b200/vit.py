@@ -16,16 +16,13 @@ key -- a pure function of the key like Flax's, but not bit-equal to JAX's threef
 from __future__ import annotations
 
 import dataclasses
-import os
 from typing import Any, Dict, Optional, Tuple, Union
 
 import numpy as np
 
+from .checkpoint import _unflatten
 from .params import count_params, flatten_params, geometry, init_params
-
-# 16-bit tensor-core operand format used when `precision` is not given: "fp16" (default; same
-# tcgen05 rate as bf16, 8x smaller logit error -- DESIGN.md "Operand format"), "bf16", or "fp32".
-_DEFAULT_PRECISION = os.environ.get("VITB200_PRECISION", "fp16")
+from .runtime import _DEFAULT_PRECISION, _FrontEnd, get_engine
 
 
 def _seed_from_key(key: Any) -> int:
@@ -42,7 +39,7 @@ def _seed_from_key(key: Any) -> int:
 
 
 @dataclasses.dataclass(frozen=True)
-class ViT:
+class ViT(_FrontEnd):
     """``ViT(image_size, patch_size, num_classes, dim, depth, heads, mlp_dim, pool='cls',
     dropout=0., emb_dropout=0.)`` -- vit.py:114-125.  ``dim_head`` is a class constant
     (un-annotated in the reference, vit.py:123), so passing it is a ``TypeError`` here too."""
@@ -89,6 +86,23 @@ class ViT:
                              "(deterministic=False): pass rngs={'dropout': key}")
         return _seed_from_key(key)
 
+    # the hooks of runtime._FrontEnd: the engine takes the tree as it is
+    def _engine_kwargs(self, channels: int) -> Dict[str, Any]:
+        return dict(self._cfg(channels), pool=self.pool, dropout=self.dropout, emb_dropout=self.emb_dropout)
+
+    def _param_channels(self, variables) -> int:
+        _, _, ph, pw, _ = geometry(self.image_size, self.patch_size)
+        return int(np.shape(flatten_params(variables)["Dense_0/kernel"])[0]) // (ph * pw)
+
+    def _engine_tree(self, variables):
+        return variables
+
+    def _layout(self, variables) -> None:
+        return None
+
+    def _grads_tree(self, flat: Dict[str, Any], layout: None = None) -> Dict[str, Any]:
+        return {"params": _unflatten(flat)}
+
     def num_params(self, channels: int = 3) -> int:
         """What the reference's demo prints (vit.py:195-197)."""
         return count_params(**self._cfg(channels))
@@ -116,29 +130,7 @@ class ViT:
         rate 0 (Flax draws nothing there).  Keyword-only extras are ours:
         ``precision`` ('fp16' / 'bf16' tcgen05 paths, 'fp8' -- E4M3 operands on to_qkv and the FeedForward,
         inference only, DESIGN.md -- and 'fp32', the validation path)."""
-        eng, xin = self._forward_engine(variables, x, rngs, precision, device, max_batch, reload)
-        if xin is not None:
-            return eng.forward(xin)
-        return eng.forward_host(np.asarray(x, dtype=np.float32))
-
-    def _forward_engine(self, variables, x, rngs, precision, device, max_batch, reload):
-        """What ``apply`` and ``attention_maps`` share: the dropout key (checked first), the image checks, the device,
-        the cached engine with ``variables`` loaded and the key set.  Returns ``(engine, x as a contiguous float32 CUDA
-        tensor)`` for a CUDA ``x``, ``(engine, None)`` for a host array."""
-        from .runtime import get_engine   # deferred: needs torch + CUDA
-        key = self._dropout_key(rngs)
-        is_torch_cuda = hasattr(x, "is_cuda") and bool(x.is_cuda)
-        channels = self._validate(tuple(x.shape) if hasattr(x, "shape") else np.shape(x))
-        batch = int(x.shape[0])
-        if device is None:
-            device = x.device.index if is_torch_cuda and x.device.index is not None else _current_device()
-        eng = get_engine(self, channels, precision or _DEFAULT_PRECISION, device, max_batch or batch, variables, reload)
-        if key is not None:
-            eng.set_dropout_key(key)
-        if not is_torch_cuda:
-            return eng, None
-        import torch
-        return eng, (x if (x.dtype == torch.float32 and x.is_contiguous()) else x.float().contiguous())
+        return self._apply(variables, x, rngs, precision, device, max_batch, reload)
 
     def attention_maps(self, variables: Any, x: Any, rngs: Any = None, *, layers=None, precision: Optional[str] = None,
                        device: Optional[int] = None, max_batch: Optional[int] = None, reload: bool = False):
@@ -151,17 +143,7 @@ class ViT:
         dropout > 0 pass ``rngs={'dropout': key}`` as for ``apply``: the maps are those of that dropped forward (the
         reference drops no attention weights, vit.py:75-83).  The maps are recomputed on the tensor cores from the
         16-bit q / k of the forward (precision 'fp16', 'bf16' or 'fp8'); 'fp32' is refused.  ``reload`` as for ``apply``."""
-        from .engine import check_layers
-        if (precision or _DEFAULT_PRECISION) == "fp32":
-            raise ValueError("attention_maps: the fp32 validation path does not record attention maps; use 'fp16', "
-                             "'bf16' or 'fp8'")
-        layers = check_layers(layers, self.depth)
-        eng, xin = self._forward_engine(variables, x, rngs, precision, device, max_batch, reload)
-        if xin is not None:
-            return eng.forward_attn(xin, layers)
-        import torch
-        logits, maps = eng.forward_attn(torch.as_tensor(np.asarray(x, dtype=np.float32), device=eng.device), layers)
-        return logits.cpu().numpy(), maps.cpu().numpy()
+        return self._attention_maps(variables, x, rngs, layers, precision, device, max_batch, reload)
 
     def vjp(self, variables: Any, x: Any, rngs: Any = None, *, wrt: str = "params", precision: Optional[str] = None,
             device: Optional[int] = None, max_batch: Optional[int] = None):
@@ -178,42 +160,7 @@ class ViT:
         ``"input"`` -- ``dx``, the float32 gradient of the images with the shape of ``x`` (saliency maps,
         FGSM / PGD); the weight-gradient GEMMs are skipped -- or ``"both"`` -- ``({'params': tree}, dx)``, the
         order of ``jax.vjp(v.apply, variables, x)``.  ``dx`` is a CUDA tensor when ``x`` is one, numpy otherwise."""
-        want_params, want_input = _parse_wrt(wrt)
-        _check_trainable_precision(precision or _DEFAULT_PRECISION, "vjp")
-        from .runtime import get_engine
-        import torch
-        key = self._dropout_key(rngs)          # rates > 0 need rngs={'dropout': key}, like apply
-        is_torch_cuda = hasattr(x, "is_cuda") and bool(x.is_cuda)
-        channels = self._validate(tuple(x.shape) if hasattr(x, "shape") else np.shape(x))
-        batch = int(x.shape[0])
-        if device is None:
-            device = x.device.index if is_torch_cuda and x.device.index is not None else _current_device()
-        eng = get_engine(self, channels, precision or _DEFAULT_PRECISION, device, max_batch or batch, variables, False)
-        dev = torch.device("cuda", device)
-        xin = x if is_torch_cuda else torch.as_tensor(np.asarray(x, dtype=np.float32), device=dev)
-        xin = xin if (xin.dtype == torch.float32 and xin.is_contiguous()) else xin.float().contiguous()
-        if key is not None:
-            eng.set_dropout_key(key)           # the backward replays the masks of this key
-        logits = eng.train_forward(xin)
-        epoch = eng.epoch      # any later forward / reload on this engine invalidates vjp_fn
-
-        def vjp_fn(dlogits):
-            d = dlogits if hasattr(dlogits, "is_cuda") else torch.as_tensor(np.asarray(dlogits, dtype=np.float32))
-            d = d.to(device=dev, dtype=torch.float32).contiguous()
-            if tuple(d.shape) != (batch, self.num_classes):
-                raise ValueError(f"vjp_fn expects a cotangent of shape ({batch}, {self.num_classes})")
-            peak = float(d.abs().max())
-            scale = 1.0 if peak == 0.0 or not np.isfinite(peak) else float(2.0 ** -np.round(np.log2(peak)))
-            dx = eng.backward(d * scale if scale != 1.0 else d, epoch=epoch, wrt=wrt)
-            out = []
-            if want_params:
-                from .checkpoint import _unflatten
-                out.append({"params": _unflatten({k: g / np.float32(scale) for k, g in eng.grads().items()})})
-            if want_input:
-                out.append(_unscale_images(dx, scale, is_torch_cuda))
-            return out[0] if len(out) == 1 else tuple(out)
-
-        return (logits if is_torch_cuda else logits.cpu().numpy()), vjp_fn
+        return self._vjp(variables, x, rngs, wrt, precision, device, max_batch)
 
     def trainer(self, variables: Any, tx, *, precision: Optional[str] = None, device: Optional[int] = None,
                 max_batch: Optional[int] = None):
@@ -231,7 +178,6 @@ class ViT:
         are staging buffers re-used two batches later."""
         if self.dropout != 0.0 or self.emb_dropout != 0.0:
             raise NotImplementedError("apply_stream is an inference path: construct ViT with the default rates 0.0")
-        from .runtime import get_engine
 
         it = iter(batches)
         try:
@@ -240,7 +186,8 @@ class ViT:
             return
         channels = self._validate(np.shape(first))
         if device is None:
-            device = _current_device()
+            import torch
+            device = torch.cuda.current_device()
         eng = get_engine(self, channels, precision or _DEFAULT_PRECISION, device, max_batch, variables, False)
 
         def chain():
@@ -252,32 +199,6 @@ class ViT:
 
     def __call__(self, *a, **k):  # flax modules are called through init/apply
         raise TypeError("call ViT through .init(rngs, x) / .apply(variables, x), like the flax module")
-
-
-def _parse_wrt(wrt: str) -> Tuple[bool, bool]:
-    """``vjp(wrt=...)`` -> (parameter gradients?, image gradient?); checked before any device work."""
-    choices = {"params": (True, False), "input": (False, True), "both": (True, True)}
-    if wrt not in choices:
-        raise ValueError(f"wrt must be one of 'params', 'input' or 'both', got {wrt!r}")
-    return choices[wrt]
-
-
-def _check_trainable_precision(precision: str, what: str) -> None:
-    """fp8 is an inference forward: refused before any device work by everything that differentiates."""
-    if precision == "fp8":
-        raise ValueError(f"{what}: precision='fp8' is inference only; use 'fp16' or 'bf16' to differentiate or train")
-
-
-def _unscale_images(dx, scale: float, as_cuda: bool):
-    """Undo the power-of-two cotangent scaling on an image gradient (exact) and hand it out like the logits."""
-    if scale != 1.0:
-        dx.div_(scale)
-    return dx if as_cuda else dx.cpu().numpy()
-
-
-def _current_device() -> int:
-    import torch
-    return torch.cuda.current_device()
 
 
 def tree_shapes(variables) -> Dict[str, Tuple[int, ...]]:
