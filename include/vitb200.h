@@ -364,6 +364,44 @@ int vitb200_attention_bwd(void* stream, const void* qkv, const void* out, const 
 int vitb200_layernorm_bwd(void* stream, const void* dy, const float* x, const float* scale,
                           float* dx, float* dscale, float* dbias, int rows, int dim, int dtype,
                           float eps, int accumulate);
+/* The same with the outputs the training backward fuses into it.  dx (fp32) is stored WITHOUT the mask.  dx16 (NULL or
+ * [rows, dim] of `dtype`) = the new dx with the Dropout mask (rate, key, site; as in vitb200_gemm_tc_dropout, flat index
+ * r * dim + c) applied in fp32, rounded once; dbias_next (NULL, or non-NULL only with dx16) += column sums of those masked
+ * fp32 values.  vitb200_layernorm_bwd(...) == vitb200_layernorm_bwd_ex(..., NULL, NULL, 0, 0, 0).                */
+int vitb200_layernorm_bwd_ex(void* stream, const void* dy, const float* x, const float* scale,
+                             float* dx, float* dscale, float* dbias, int rows, int dim, int dtype,
+                             float eps, int accumulate, void* dx16, float* dbias_next,
+                             float rate, uint64_t key, uint32_t site);
+/* Bias-gradient row passes (cols % 8 == 0; the Dropout triple as above, replayed on the flat index r * cols + c):
+ * cast16_colsum:   y16 = round(Dropout(x)),                          sums[c] += sum_r Dropout(x)[r, c]   (fp32 values)
+ * gelu_bwd_colsum: dpre16 = round(Dropout(dhid16 * gelu_tanh'(pre16))), sums[c] += sum_r dpre16[r, c]   (ROUNDED values)
+ * gelu' uses tanh.approx (2^-11 relative).  dpre may be dhid (in place).  sums accumulate.                           */
+int vitb200_cast16_colsum(void* stream, const float* x, void* y16, float* sums, int rows, int cols, int dtype,
+                          float rate, uint64_t key, uint32_t site);
+int vitb200_gelu_bwd_colsum(void* stream, const void* pre, const void* dhid, void* dpre, float* sums, int rows,
+                            int cols, int dtype, float rate, uint64_t key, uint32_t site);
+/* hid16 = round(Dropout(gelu_tanh(pre16))) over n elements (n % 8 == 0, flat index i): the FF activation of a training
+ * forward that keeps the GELU out of the GEMM epilogue (VITB200_TRAIN_DUAL=0)                                     */
+int vitb200_gelu_fwd(void* stream, const void* pre, void* hid, int64_t n, int dtype, float rate, uint64_t key,
+                     uint32_t site);
+/* x = Dropout(x) in place, fp32, n % 4 == 0 (the embedding dropout's mask in the backward pass); rate 0: nothing */
+int vitb200_dropout_inplace(void* stream, float* x, int64_t n, float rate, uint64_t key, uint32_t site);
+/* Adjoint of vitb200_pool_layernorm (fp32; pool 0 = cls, 1 = mean): x [batch, T, dim] the pooled input, dy [batch, dim]
+ * the cotangent of the LayerNorm output -> dpooled [batch, dim] = the gradient of one token row (cls: of row 0; mean: of
+ * every row, i.e. the pooled gradient / T), dx [batch, T, dim] fully overwritten (cls: zero rows for t > 0), dscale /
+ * dbias +=.  dim % 4 == 0.  dpooled may be dy.                                                                      */
+int vitb200_pool_layernorm_bwd(void* stream, const float* x, const float* dy, const float* scale, float* dpooled,
+                               float* dx, float* dscale, float* dbias, int batch, int T, int dim, int pool, float eps);
+/* Head Dense backward (fp32): pooled [batch, dim], dlogits [batch, classes], W [dim, classes] (Flax kernel) ->
+ * dpooled [batch, dim] = dlogits W^T (overwritten); dW (NULL: skipped) += pooled^T dlogits; dbias (NULL: skipped) +=
+ * column sums of dlogits.                                                                                          */
+int vitb200_head_bwd(void* stream, const float* pooled, const float* dlogits, const float* W, float* dW, float* dbias,
+                     float* dpooled, int batch, int dim, int classes);
+/* Token-embedding gradients (vit.py:151-153) from dx [batch, T, dim] fp32: dpos [T, dim] = sum_b dx[b].  dpos MUST be
+ * zero on entry: its sums are written with plain adds and then read back for the others.  cls_slot 1: dcls [dim] +=
+ * dpos[0], dbias [dim] += sum_{t >= 1} dpos[t]; cls_slot 0: dbias += sum_t dpos[t], dcls unused (may be NULL).      */
+int vitb200_token_grads(void* stream, const float* dx, float* dpos, float* dcls, float* dbias, int batch, int T,
+                        int dim, int cls_slot);
 
 /* patchify (vit.py:146): images [batch,H,W,C] fp32 -> patches [batch*Np, Kpad] of out_dtype,
  * feature f = (p1*pw + p2)*C + c, zero padded to Kpad. */

@@ -90,6 +90,15 @@ SIGNATURES = {
     "vitb200_gemm_tc_wgrad": (_i, [_vp, _vp, _vp, _fp, _i, _i, _i, _i, _i]),
     "vitb200_attention_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
     "vitb200_layernorm_bwd": (_i, [_vp, _vp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i, C.c_float, _i]),
+    "vitb200_layernorm_bwd_ex": (_i, [_vp, _vp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i, C.c_float, _i, _vp, _fp,
+                                      C.c_float, C.c_uint64, C.c_uint32]),
+    "vitb200_cast16_colsum": (_i, [_vp, _fp, _vp, _fp, _i, _i, _i, C.c_float, C.c_uint64, C.c_uint32]),
+    "vitb200_gelu_bwd_colsum": (_i, [_vp, _vp, _vp, _vp, _fp, _i, _i, _i, C.c_float, C.c_uint64, C.c_uint32]),
+    "vitb200_gelu_fwd": (_i, [_vp, _vp, _vp, _i64, _i, C.c_float, C.c_uint64, C.c_uint32]),
+    "vitb200_dropout_inplace": (_i, [_vp, _fp, _i64, C.c_float, C.c_uint64, C.c_uint32]),
+    "vitb200_pool_layernorm_bwd": (_i, [_vp, _fp, _fp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i, _i, C.c_float]),
+    "vitb200_head_bwd": (_i, [_vp, _fp, _fp, _fp, _fp, _fp, _fp, _i, _i, _i]),
+    "vitb200_token_grads": (_i, [_vp, _fp, _fp, _fp, _fp, _i, _i, _i, _i]),
     "vitb200_gemm_tc": (_i, [_vp, _vp, _vp, _fp, _vp, _i, _i, _i, _i, _fp, _i, _i]),
     "vitb200_gemm_tc_dropout": (_i, [_vp, _vp, _vp, _fp, _vp, _i, _i, _i, _i, _fp, _i, _i, C.c_float, C.c_uint64, C.c_uint32]),
     "vitb200_gemm_tc_tokens": (_i, [_vp, _vp, _vp, _fp, _vp, _i, _i, _i, _i, _fp, _i, _fp, _i, C.c_float, C.c_uint64, C.c_uint32]),

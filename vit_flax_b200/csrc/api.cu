@@ -96,6 +96,22 @@ struct ActMaps {   // TMA descriptors over the activation workspace for one batc
 
 using namespace vb;
 
+namespace {
+// nn.Dropout instance `site` of the 'dropout' key at `rate` (rate 0 => off); kept values are scaled by 1 / (1 - rate) in fp32
+Dropout make_dropout(float rate, uint64_t key, uint32_t site) {
+  Dropout d;
+  if (rate > 0.f) {
+    d.key_lo = uint32_t(key);
+    d.key_hi = uint32_t(key >> 32);
+    d.site = site;
+    const double t = double(rate) * 4294967296.0;
+    d.threshold = t >= 4294967295.0 ? 0xFFFFFFFFu : uint32_t(t);
+    d.inv_keep = 1.0f / (1.0f - rate);
+  }
+  return d;
+}
+}  // namespace
+
 struct vitb200_model {
   vitb200_config cfg{};
   int device = 0;
@@ -120,18 +136,7 @@ struct vitb200_model {
   bool opt_table_dirty = true;       // the AdamW chunk table must be rebuilt from leaf_flags
 
   // the Dropout instance `site` of this model (rate 0 => off)
-  Dropout drop(float rate, uint32_t site) const {
-    Dropout d;
-    if (rate > 0.f) {
-      d.key_lo = uint32_t(dropout_key);
-      d.key_hi = uint32_t(dropout_key >> 32);
-      d.site = site;
-      const double t = double(rate) * 4294967296.0;
-      d.threshold = t >= 4294967295.0 ? 0xFFFFFFFFu : uint32_t(t);
-      d.inv_keep = 1.0f / (1.0f - rate);
-    }
-    return d;
-  }
+  Dropout drop(float rate, uint32_t site) const { return make_dropout(rate, dropout_key, site); }
 
   std::vector<Leaf> leaves;
   std::map<std::string, int> index;
@@ -1647,15 +1652,7 @@ int vitb200_gemm_tc_tokens(void* stream, const void* A, const void* Wt, const fl
                            int K, int epilogue, const float* aux, int tokens_per_image, const float* cls, int dtype,
                            float rate, uint64_t key, uint32_t site) {
   if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "gemm_tc: dropout rate must be in [0, 1)");
-  Dropout drop;
-  if (rate > 0.f) {
-    drop.key_lo = uint32_t(key);
-    drop.key_hi = uint32_t(key >> 32);
-    drop.site = site;
-    const double t = double(rate) * 4294967296.0;
-    drop.threshold = t >= 4294967295.0 ? 0xFFFFFFFFu : uint32_t(t);
-    drop.inv_keep = 1.0f / (1.0f - rate);
-  }
+  const Dropout drop = make_dropout(rate, key, site);
   if (!A || !Wt || !C) return fail(VITB200_ERR_INVALID, "gemm_tc: null pointer");
   if (M <= 0 || N <= 0 || K <= 0) return fail(VITB200_ERR_INVALID, "gemm_tc: empty problem");
   if ((N % 8) != 0 || (K % 8) != 0)
@@ -1833,9 +1830,70 @@ int vitb200_attention_bwd(void* stream, const void* qkv, const void* out, const 
 
 int vitb200_layernorm_bwd(void* stream, const void* dy, const float* x, const float* scale, float* dx, float* dscale,
                           float* dbias, int rows, int dim, int dtype, float eps, int accumulate) {
+  return vitb200_layernorm_bwd_ex(stream, dy, x, scale, dx, dscale, dbias, rows, dim, dtype, eps, accumulate, nullptr, nullptr,
+                                  0.f, 0, 0);
+}
+
+int vitb200_layernorm_bwd_ex(void* stream, const void* dy, const float* x, const float* scale, float* dx, float* dscale,
+                             float* dbias, int rows, int dim, int dtype, float eps, int accumulate, void* dx16,
+                             float* dbias_next, float rate, uint64_t key, uint32_t site) {
   if (!dy || !x || !scale || !dx || !dscale || !dbias) return fail(VITB200_ERR_INVALID, "layernorm_bwd: null pointer");
+  if (dbias_next && !dx16) return fail(VITB200_ERR_INVALID, "layernorm_bwd: dbias_next needs dx16");
+  if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "layernorm_bwd: dropout rate must be in [0, 1)");
   return launch_ln_bwd(static_cast<cudaStream_t>(stream), dy, x, scale, dx, dscale, dbias, rows, dim, dtype,
-                       eps > 0.f ? eps : 1e-6f, accumulate);
+                       eps > 0.f ? eps : 1e-6f, accumulate, dx16, dbias_next, make_dropout(rate, key, site));
+}
+
+int vitb200_cast16_colsum(void* stream, const float* x, void* y16, float* sums, int rows, int cols, int dtype, float rate,
+                          uint64_t key, uint32_t site) {
+  if (!x || !y16 || !sums) return fail(VITB200_ERR_INVALID, "cast16_colsum: null pointer");
+  if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "cast16_colsum: dropout rate must be in [0, 1)");
+  return launch_cast16_colsum(static_cast<cudaStream_t>(stream), x, y16, sums, rows, cols, dtype, make_dropout(rate, key, site));
+}
+
+int vitb200_gelu_bwd_colsum(void* stream, const void* pre, const void* dhid, void* dpre, float* sums, int rows, int cols,
+                            int dtype, float rate, uint64_t key, uint32_t site) {
+  if (!pre || !dhid || !dpre || !sums) return fail(VITB200_ERR_INVALID, "gelu_bwd_colsum: null pointer");
+  if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "gelu_bwd_colsum: dropout rate must be in [0, 1)");
+  return launch_gelu_bwd_colsum(static_cast<cudaStream_t>(stream), pre, dhid, dpre, sums, rows, cols, dtype,
+                                make_dropout(rate, key, site));
+}
+
+int vitb200_gelu_fwd(void* stream, const void* pre, void* hid, int64_t n, int dtype, float rate, uint64_t key, uint32_t site) {
+  if (!pre || !hid) return fail(VITB200_ERR_INVALID, "gelu_fwd: null pointer");
+  if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "gelu_fwd: dropout rate must be in [0, 1)");
+  return launch_gelu_fwd(static_cast<cudaStream_t>(stream), pre, hid, n, dtype, make_dropout(rate, key, site));
+}
+
+int vitb200_dropout_inplace(void* stream, float* x, int64_t n, float rate, uint64_t key, uint32_t site) {
+  if (!x) return fail(VITB200_ERR_INVALID, "dropout_inplace: null pointer");
+  if (!(rate >= 0.f && rate < 1.f)) return fail(VITB200_ERR_INVALID, "dropout_inplace: rate must be in [0, 1)");
+  if (n <= 0 || (n & 3)) return fail(VITB200_ERR_INVALID, "dropout_inplace: element count must be a positive multiple of 4");
+  return launch_mask_inplace(static_cast<cudaStream_t>(stream), x, n, make_dropout(rate, key, site));
+}
+
+int vitb200_pool_layernorm_bwd(void* stream, const float* x, const float* dy, const float* scale, float* dpooled, float* dx,
+                               float* dscale, float* dbias, int batch, int T, int dim, int pool, float eps) {
+  if (!x || !dy || !scale || !dpooled || !dx || !dscale || !dbias) return fail(VITB200_ERR_INVALID, "pool_layernorm_bwd: null pointer");
+  if (pool != VITB200_POOL_CLS && pool != VITB200_POOL_MEAN) return fail(VITB200_ERR_INVALID, "pool_layernorm_bwd: pool must be cls or mean");
+  if (batch <= 0 || T <= 0 || dim <= 0) return fail(VITB200_ERR_INVALID, "pool_layernorm_bwd: empty problem");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (dpooled != dy) VB_CUDA(cudaMemcpyAsync(dpooled, dy, size_t(batch) * dim * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return launch_pool_ln_bwd(st, x, dpooled, scale, dx, dscale, dbias, batch, T, dim, pool == VITB200_POOL_MEAN,
+                            eps > 0.f ? eps : 1e-6f);
+}
+
+int vitb200_head_bwd(void* stream, const float* pooled, const float* dlogits, const float* W, float* dW, float* dbias,
+                     float* dpooled, int batch, int dim, int classes) {
+  if (!dlogits || !W || !dpooled || (dW && !pooled)) return fail(VITB200_ERR_INVALID, "head_bwd: null pointer");
+  return launch_head_bwd(static_cast<cudaStream_t>(stream), pooled, dlogits, W, dW, dbias, dpooled, batch, dim, classes);
+}
+
+int vitb200_token_grads(void* stream, const float* dx, float* dpos, float* dcls, float* dbias, int batch, int T, int dim,
+                        int cls_slot) {
+  if (!dx || !dpos || !dbias || (cls_slot && !dcls)) return fail(VITB200_ERR_INVALID, "token_grads: null pointer");
+  if (cls_slot != 0 && cls_slot != 1) return fail(VITB200_ERR_INVALID, "token_grads: cls_slot is 0 or 1");
+  return launch_token_grads(static_cast<cudaStream_t>(stream), dx, dpos, dcls, dbias, batch, T, dim, cls_slot);
 }
 
 int vitb200_patchify(void* stream, const float* images, void* patches, int batch, int H, int W, int C, int ph,

@@ -458,30 +458,37 @@ attention_bwd_tc5_kernel(const __grid_constant__ CUtensorMap tmQKV,   // qkv [B,
   }
 }
 
-// D[item, t] = sum_d dO[b, t, h, d] O[b, t, h, d], item = b * heads + h: one warp per token row, eight lanes per head
+// D[item, t] = sum_d dO[b, t, h, d] O[b, t, h, d], item = b * heads + h: one warp per token row, eight lanes per head.
+// The chunk loop has the same trip count on every lane (heads * 8 rounded up to the warp), so the full-mask shuffles
+// always see all 32 lanes; lanes past the row's last chunk load nothing and store nothing.
 template <int kDT>
 __global__ void __launch_bounds__(256)
 attn_bwd_rowdot_kernel(const uint16_t* __restrict__ d_out, const uint16_t* __restrict__ o_fwd, float* __restrict__ dsum,
                        int rows, int T, int heads) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int inner = heads * DH;
+  const int nchunk = heads * 8, nchunk_warp = (nchunk + 31) & ~31;
   for (int64_t row = int64_t(blockIdx.x) * 8 + warp; row < rows; row += int64_t(gridDim.x) * 8) {
     const int b = int(row / T), t = int(row - int64_t(b) * T);
     const uint4* dr = reinterpret_cast<const uint4*>(d_out + row * inner);
     const uint4* orow = reinterpret_cast<const uint4*>(o_fwd + row * inner);
-    for (int c = lane; c < heads * 8; c += 32) {         // 16-byte chunk c = 8 values of head c / 8
-      const uint4 dv = __ldg(dr + c), ov = __ldg(orow + c);
-      const uint32_t dd[4] = {dv.x, dv.y, dv.z, dv.w}, oo[4] = {ov.x, ov.y, ov.z, ov.w};
+    for (int c0 = 0; c0 < nchunk_warp; c0 += 32) {
+      const int c = c0 + lane;                           // 16-byte chunk c = 8 values of head c / 8
+      const bool active = c < nchunk;                    // uniform over each group of 8 lanes (nchunk % 8 == 0)
       float acc = 0.f;
+      if (active) {
+        const uint4 dv = __ldg(dr + c), ov = __ldg(orow + c);
+        const uint32_t dd[4] = {dv.x, dv.y, dv.z, dv.w}, oo[4] = {ov.x, ov.y, ov.z, ov.w};
 #pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        acc = fmaf(to_f32<kDT>(uint16_t(dd[e] & 0xFFFFu)), to_f32<kDT>(uint16_t(oo[e] & 0xFFFFu)), acc);
-        acc = fmaf(to_f32<kDT>(uint16_t(dd[e] >> 16)), to_f32<kDT>(uint16_t(oo[e] >> 16)), acc);
+        for (int e = 0; e < 4; ++e) {
+          acc = fmaf(to_f32<kDT>(uint16_t(dd[e] & 0xFFFFu)), to_f32<kDT>(uint16_t(oo[e] & 0xFFFFu)), acc);
+          acc = fmaf(to_f32<kDT>(uint16_t(dd[e] >> 16)), to_f32<kDT>(uint16_t(oo[e] >> 16)), acc);
+        }
       }
       acc += __shfl_xor_sync(0xffffffffu, acc, 1);
       acc += __shfl_xor_sync(0xffffffffu, acc, 2);
       acc += __shfl_xor_sync(0xffffffffu, acc, 4);
-      if ((lane & 7) == 0) dsum[(int64_t(b) * heads + (c >> 3)) * T + t] = acc;
+      if (active && (lane & 7) == 0) dsum[(int64_t(b) * heads + (c >> 3)) * T + t] = acc;
     }
   }
 }
